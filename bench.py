@@ -2,6 +2,7 @@
 """Headline benchmark: top-10 cosine queries/s on a 10M x 768 bf16 gallery (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--rows R --queries Q --k K]
+                    [--dump-outputs DIR]
 
 A step = one pass of the hot path over one batch of synthetic queries: rbod_search (query prep,
 K3 tcgen05 cosine top-k, merge + fp64 rescoring + certification in the finish kernel) on a gallery
@@ -10,7 +11,8 @@ that is already resident in HBM.  ``value`` times the step with device-resident 
 inside the timed region.  ``roofline`` describes the dominant kernel (K3), timed live with CUDA
 events on its launch stream.  ``cpu_baseline`` is the numpy float64 oracle port on a bounded sample
 of the same workload (the one place besides tests/smoke where oracle/ is executed; it is never the
-thing shipped).
+thing shipped).  Gallery and queries come from fixed seeds, so ``--dump-outputs`` of two builds run
+with the same arguments can be compared array for array.
 
 N > 1 (torchrun, one rank per GPU): the 10M rows are block-partitioned over the ranks, every rank
 searches its shard for the same query batch into one packed buffer, ONE NCCL all-gather of the
@@ -62,12 +64,42 @@ def parse_args():
     ap.add_argument("--opt", action="append", default=[], help="library tunable key=value (debug), repeatable")
     ap.add_argument("--sweep", default="", help="comma list of batch sizes: per-size p50 latency and q/s on the "
                     "resident gallery (config C5's query sweep), printed as one JSON line instead of the headline")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="", help="after the timed steps, write what the last "
+                    "timed step returned as DIR/<name>.npy, so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.sweep):
+        ap.error("--dump-outputs writes the headline search's result: not with --impl reference or --sweep")
+    return a
 
 
 def workload_name(a) -> str:
     return (f"{a.rows / 1e6:g}M x {a.dim} {a.dtype} gallery (synthetic unit-norm rows), "
             f"{a.queries}-query batch, exact top-{a.k} cosine")
+
+
+DUMP_LIMIT = 64 << 20        # bytes --dump-outputs writes at most
+
+
+def dump_outputs(path, scores, rows, scores64, limit=DUMP_LIMIT):
+    """Writes one search result as path/scores.npy (float32), rows.npy (global row ids, exact in float64) and
+    scores64.npy (float64).  A result larger than ``limit`` bytes is cut to a fixed, seeded sample of its queries,
+    whose indices go to path/query_index.npy."""
+    import numpy as np
+
+    arrays = {"scores": np.asarray(scores, np.float32), "rows": np.asarray(rows, np.float64),
+              "scores64": np.asarray(scores64, np.float64)}
+    Q = arrays["scores"].shape[0]
+    bytes_per_query = sum(x.itemsize * x.shape[1] for x in arrays.values()) + 8        # + its index when sampled
+    keep = (limit - 4096) // bytes_per_query                                           # 4096: the .npy headers
+    if Q > keep:
+        idx = np.sort(np.random.default_rng(0).choice(Q, keep, replace=False))
+        arrays = {name: x[idx] for name, x in arrays.items()}
+        arrays["query_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, x in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), x)
 
 
 # --------------------------------------------------------------------------------------------
@@ -581,10 +613,11 @@ def run_b200(a):
     S = Searcher(E, g, a.queries, a.k, offsets_all)
     k3_ms, fallback = [], []
     diag = {"search_s": 0.0, "steps": 0, "sweep": 0, "retries": 0}
+    last = {}
 
     def step_device():
         t_s = time.perf_counter()
-        out = S.device_step(q_dev)
+        out = last["out"] = S.device_step(q_dev)
         diag["search_s"] += time.perf_counter() - t_s
         diag["steps"] += 1
         diag["sweep"] += S.stats["sweep_queries"]
@@ -604,6 +637,8 @@ def run_b200(a):
     fallback.clear()
     diag.update(search_s=0.0, steps=0, sweep=0, retries=0)
     ms_dev = E.timed(step_device, a.steps)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, *(t.cpu().numpy() for t in last["out"]))
     per_rank = {"rank": rank, "search_ms_per_step": round(diag["search_s"] / max(diag["steps"], 1) * 1e3, 3),
                 "k3_ms": round(statistics.mean(k3_ms), 3) if k3_ms else 0.0,
                 "uncertified_per_step": statistics.mean(fallback) if fallback else 0,
