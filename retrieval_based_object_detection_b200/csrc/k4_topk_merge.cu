@@ -12,9 +12,10 @@
 //                        kernels -- bitonic merge, rescore, select -- with the candidates round-tripping
 //                        through global memory; the bitonic sort of up to 8192 keys per query was the
 //                        largest fixed cost of a sharded search.)
-//   exact_collect /  exact fp64 sweep over the whole gallery for flagged queries only: collect
-//   select_collected every row whose exact score >= the query's provisional k-th score, then
-//                    select among those.  This is the guarantee behind "identical ids".
+//   select_collected answer of the collecting second pass for flagged queries: the rows the collecting K3
+//                    launch recorded, rescored exactly.  A query whose list overflows goes on to the exact
+//                    fp64 sweep (K5), seeded with its provisional k-th score.  This is the guarantee behind
+//                    "identical ids".
 //   merge_topk       (K4 proper) G sorted per-GPU lists -> global top k, after the NCCL
 //                    all-gather in the row-sharded multi-GPU search.
 //
@@ -616,124 +617,17 @@ __global__ void __launch_bounds__(128) global_cut_kernel(const float* __restrict
   if (lane == 0) out[q] = make_float2(n >= k ? ordered_to_f32(prefix) : -INFINITY, eps);
 }
 
-// ---------------------------------------------------------------------------------------------
-// exact fallback
-// ---------------------------------------------------------------------------------------------
-constexpr int EX_NMAX = 64;  // dim <= 2048 (K3_MAX_DP_WIDE)
-
-__global__ void __launch_bounds__(256)
-exact_collect_kernel(const float* __restrict__ q, const double* __restrict__ q_qq,
-                     const float* __restrict__ master32, const uint16_t* __restrict__ rows16, int kind16, int dim,
-                     int64_t ld32, int64_t ld16, int metric, int64_t n_rows, const uint32_t* __restrict__ row_mask,
-                     const int* __restrict__ flag_q, const double* __restrict__ flag_thr,
-                     const uint32_t* __restrict__ flag_row, const int* __restrict__ active, int f0, int nf, int cap,
-                     double* __restrict__ coll_score, uint32_t* __restrict__ coll_idx, int* __restrict__ coll_cnt) {
-  const int lane = threadIdx.x & 31;
-  const int64_t w0 = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
-  const int64_t nw = (int64_t)gridDim.x * 8;
-  for (int64_t r = w0; r < n_rows; r += nw) {
-    if (row_mask && !((row_mask[r >> 5] >> (r & 31)) & 1u)) continue;
-    double g[EX_NMAX];
-    double gg = 0.0;
-#pragma unroll
-    for (int i = 0; i < EX_NMAX; ++i) {
-      const int c = lane + 32 * i;
-      double x = 0.0;
-      if (c < dim) x = master32 ? (double)master32[r * ld32 + c] : (double)h16_to_f32(rows16[r * ld16 + c], kind16);
-      g[i] = x;
-      gg = fma(x, x, gg);
-    }
-    gg = warp_sum_f64(gg);
-    const double gn = sqrt(gg);
-    for (int f = 0; f < nf; ++f) {
-      if (active != nullptr && !active[f]) continue;   // this query's list is complete: later sweeps leave it alone
-      const int qi = flag_q[f0 + f];
-      const float* qv = q + (int64_t)qi * dim;
-      double acc = 0.0;
-#pragma unroll
-      for (int i = 0; i < EX_NMAX; ++i) {
-        const int c = lane + 32 * i;
-        if (c < dim) {
-          if (metric == RBOD_EUCLID) {
-            const double d = (double)qv[c] - g[i];
-            acc = fma(d, d, acc);
-          } else {
-            acc = fma((double)qv[c], g[i], acc);
-          }
-        }
-      }
-      acc = warp_sum_f64(acc);
-      if (lane == 0) {
-        const double den = sqrt(q_qq[qi]) * gn;
-        const double s = metric == RBOD_EUCLID ? -acc : (metric == RBOD_DOT ? acc : (den > 0.0 ? acc / den : 0.0));
-        // the threshold is the provisional k-th exact score as the finish kernel summed it; this sweep adds the same
-        // products in another order, so the very row that set the threshold may come out an ulp lower here: collect
-        // with a margin far above fp64 summation noise (select_collected ranks by this sweep's own scores)
-        // A list that overflowed was tightened to the k-th best (score, row) PAIR it had recorded -- scores of this very
-        // kernel, so they compare exactly -- and a row bound: more rows than fit tie with the k-th score (duplicates),
-        // and of those only the smallest row slots can be in the answer.
-        const double thr = flag_thr[f0 + f];
-        const uint32_t rb = flag_row != nullptr ? flag_row[f0 + f] : 0xffffffffu;
-        const bool take = rb == 0xffffffffu ? (s >= thr - 1e-12 * fmax(1.0, fabs(thr)))
-                                            : (s > thr || (s == thr && (uint32_t)r <= rb));
-        if (take) {
-          const int slot = atomicAdd(coll_cnt + f, 1);
-          if (slot < cap) {
-            coll_score[(size_t)f * cap + slot] = s;
-            coll_idx[(size_t)f * cap + slot] = (uint32_t)r;
-          }
-        }
-      }
-    }
-  }
-}
-
-// A swept list that overflowed (more than `cap` rows at or above the threshold -- a cluster of duplicates around the
-// k-th score): the k-th best (score desc, row asc) pair among the `cap` rows that WERE recorded is a bound every member
-// of the true top k meets, and a much tighter one (about cap / k times fewer rows pass it).  One CTA per list.
-__global__ void __launch_bounds__(256)
-tighten_kernel(const double* __restrict__ coll_score, const uint32_t* __restrict__ coll_idx, int* __restrict__ coll_cnt,
-               int f0, int cap, int k, double* __restrict__ flag_thr, uint32_t* __restrict__ flag_row,
-               int* __restrict__ active, int* __restrict__ n_active) {
-  const int f = blockIdx.x;
-  if (coll_cnt[f] <= cap) {
-    if (threadIdx.x == 0) active[f] = 0;
-    return;
-  }
-  const double* sc = coll_score + (size_t)f * cap;
-  const uint32_t* ix = coll_idx + (size_t)f * cap;
-  for (int j = threadIdx.x; j < cap; j += blockDim.x) {
-    const double s = sc[j];
-    const uint32_t id = ix[j];
-    int rank = 0;
-    for (int i = 0; i < cap; ++i)
-      if (beats(sc[i], ix[i], s, id)) ++rank;
-    if (rank == k - 1) {
-      flag_thr[f0 + f] = s;
-      flag_row[f0 + f] = id;
-    }
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    active[f] = 1;
-    coll_cnt[f] = 0;
-    atomicAdd(n_active, 1);
-  }
-}
-
+// The answer of a collecting second pass from its rescored list (one CTA per flagged query).  A list that overflowed
+// is left alone: the host sends that query on to the exact sweep (K5).
 __global__ void __launch_bounds__(256)
 select_collected_kernel(const double* __restrict__ coll_score, const uint32_t* __restrict__ coll_idx,
                         const int* __restrict__ coll_cnt, const int* __restrict__ flag_q, int f0, int cap, int k,
                         int metric, float* __restrict__ out_scores, int64_t* __restrict__ out_rows,
-                        double* __restrict__ out_scores64, int* __restrict__ overflow) {
+                        double* __restrict__ out_scores64) {
   const int f = blockIdx.x;
   const int q = flag_q[f0 + f];
-  int cnt = coll_cnt[f];
-  if (cnt > cap) {
-    if (overflow == nullptr) return;   // caller re-runs this query through the exact sweep
-    if (threadIdx.x == 0) atomicExch(overflow, 1);
-    cnt = cap;
-  }
+  const int cnt = coll_cnt[f];
+  if (cnt > cap) return;
   const double* sc = coll_score + (size_t)f * cap;
   const uint32_t* ix = coll_idx + (size_t)f * cap;
   for (int j = threadIdx.x; j < k; j += blockDim.x) {
@@ -893,36 +787,12 @@ int launch_finish(const FinishArgs& A, int64_t Q, cudaStream_t st) {
   return RBOD_OK;
 }
 
-int launch_exact_collect(const float* q, const double* q_qq, const float* master32, const uint16_t* rows16,
-                         int kind16, int dim, int64_t ld32, int64_t ld16, int metric, int64_t n_rows,
-                         const uint32_t* row_mask, const int* flag_q, const double* flag_thr, const uint32_t* flag_row,
-                         const int* active, int f0, int nf, int cap, double* coll_score, uint32_t* coll_idx,
-                         int* coll_cnt, int num_sms, cudaStream_t st) {
-  if (nf <= 0 || n_rows <= 0) return RBOD_OK;
-  if (dim > 32 * EX_NMAX) return set_error(RBOD_E_UNSUPPORTED, "exact fallback supports dim <= %d", 32 * EX_NMAX);
-  const int64_t want = (n_rows + 7) / 8;
-  const int grid = (int)(want < (int64_t)num_sms * 6 ? want : (int64_t)num_sms * 6);
-  exact_collect_kernel<<<grid, 256, 0, st>>>(q, q_qq, master32, rows16, kind16, dim, ld32, ld16, metric, n_rows, row_mask,
-                                             flag_q, flag_thr, flag_row, active, f0, nf, cap, coll_score, coll_idx,
-                                             coll_cnt);
-  RBOD_CUDA(cudaGetLastError());
-  return RBOD_OK;
-}
-
-int launch_tighten(const double* coll_score, const uint32_t* coll_idx, int* coll_cnt, int f0, int nf, int cap, int k,
-                   double* flag_thr, uint32_t* flag_row, int* active, int* n_active, cudaStream_t st) {
-  if (nf <= 0) return RBOD_OK;
-  tighten_kernel<<<nf, 256, 0, st>>>(coll_score, coll_idx, coll_cnt, f0, cap, k, flag_thr, flag_row, active, n_active);
-  RBOD_CUDA(cudaGetLastError());
-  return RBOD_OK;
-}
-
 int launch_select_collected(const double* coll_score, const uint32_t* coll_idx, const int* coll_cnt,
                             const int* flag_q, int f0, int nf, int cap, int k, int metric, float* out_scores,
-                            int64_t* out_rows, double* out_scores64, int* overflow, cudaStream_t st) {
+                            int64_t* out_rows, double* out_scores64, cudaStream_t st) {
   if (nf <= 0) return RBOD_OK;
   select_collected_kernel<<<nf, 256, 0, st>>>(coll_score, coll_idx, coll_cnt, flag_q, f0, cap, k, metric, out_scores,
-                                              out_rows, out_scores64, overflow);
+                                              out_rows, out_scores64);
   RBOD_CUDA(cudaGetLastError());
   return RBOD_OK;
 }

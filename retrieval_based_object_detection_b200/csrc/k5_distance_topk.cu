@@ -1,15 +1,16 @@
-// K5  distance_topk -- exact top-k for the two distances of the collection menu that are not inner
-// products: Distance.EUCLID and Distance.MANHATTAN (util/qdrant_manager.py:61-66, chosen at :68-79 and
-// passed to recreate_collection at :82-85).  Neither is served by the tcgen05 pass: L1 distance is not a
-// contraction at all, and the reference only ever creates such collections at script scale, so both take
-// one exact route on the CUDA cores in fp64 (B200 issues 64 DFMA per clock per SM):
+// K5  distance_topk -- exact top-k by a sweep of the whole gallery on the CUDA cores in fp64 (B200 issues 64 DFMA
+// per clock per SM), for every metric.  It answers what the tcgen05 pass does not cover: Distance.MANHATTAN
+// (util/qdrant_manager.py:61-66, chosen at :68-79 and passed to recreate_collection at :82-85; L1 distance is not a
+// contraction at all, and the reference only ever creates such collections at script scale), k beyond the K3
+// candidate lists, rows wider than K3 takes -- and the finish path's queries the certification left open.  Keys:
 //
-//   key(q, g) = -sum_i (q_i - g_i)^2   (EUCLID)      key(q, g) = -sum_i |q_i - g_i|   (MANHATTAN)
+//   key(q, g) = dot / (|q| |g|)  (COSINE)     = dot  (DOT)
+//             = -sum_i (q_i - g_i)^2   (EUCLID)      = -sum_i |q_i - g_i|   (MANHATTAN)
 //
 // computed in fp64 from the fp32 query and the stored row, so larger key = closer and the ordering
 // (key desc, row asc) needs no certification.  Selection without a Q x N matrix:
 //   1. sample pass: keys of a strided sample of <= cap rows; the k-th best sample key is a threshold no
-//      member of the true top-k can fall below;
+//      member of the true top-k can fall below (a caller that already holds such a bound passes it instead);
 //   2. sweep: one pass over the gallery records every row whose key >= threshold (expected k * stride
 //      rows); a list that overflows `cap` tightens its threshold to the k-th best key it did record --
 //      still a lower bound of the true k-th key -- and only those queries are swept again;

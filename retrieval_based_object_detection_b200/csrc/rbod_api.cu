@@ -291,7 +291,7 @@ int rbod_destroy(rbod_gallery* g) {
   if (g->stats) cudaFree(g->stats);
   DevBuf* bufs[] = {&g->stage_rows, &g->stage_slots, &g->stage_norms, &g->q32, &g->q16, &g->q_dq, &g->q_qq, &g->tau_shared,
                     &g->lists, &g->list_cnt, &g->out_scores,
-                    &g->out_rows, &g->out_scores64, &g->flags, &g->flag_q, &g->flag_thr, &g->flag_lo, &g->flag_row, &g->sweep_ctl, &g->fq16, &g->groupmax, &g->tau_init, &g->coll_score,
+                    &g->out_rows, &g->out_scores64, &g->flags, &g->flag_q, &g->flag_thr, &g->flag_lo, &g->fq16, &g->groupmax, &g->tau_init, &g->coll_score,
                     &g->coll_idx, &g->coll_cnt, &g->mask_dev, &g->dump, &g->sync_counters, &g->prof, &g->seg_idx, &g->seg_off, &g->seg_out,
                     &g->seg_partials, &g->seg_prefix, &g->seg_arrive, &g->seg_scratch, &g->seg_member, &g->gather_idx,
                     &g->gather_out, &g->dist_q64, &g->dist_thr, &g->dist_ctl};
@@ -834,19 +834,19 @@ static int prepare_queries(rbod_gallery* g, const float* queries, int64_t Q, con
                              g->q_dq.as<float>(), g->q_qq.as<double>(), g->tau_shared.as<uint32_t>(), st);
 }
 
-// EUCLID / MANHATTAN: exact fp64 sweep (kernel K5), 32 queries per pass over the gallery.
-static int search_distance(rbod_gallery* g, const float* queries, int64_t Q, int k, const uint32_t* mask_dev,
-                           float* d_scores, int64_t* d_rows, double* d_keys, int64_t* launches, int64_t* resweeps,
-                           cudaStream_t st) {
+// Exact fp64 sweep (kernel K5), 32 queries per pass over the gallery: answers the n queries of q_dev (device, [*, dim]
+// fp32) listed in the host array qsel -- queries 0..n-1 if it is null -- in their rows q * k of the outputs.  kth (host,
+// one per listed query, or null) is each query's provisional k-th key, -inf if it had fewer than k candidates: a
+// lower bound of the true k-th key that replaces the sample pass as the starting threshold.
+static int sweep_exact(rbod_gallery* g, const float* q_dev, int64_t n, const int* qsel, const double* kth, int k,
+                       const uint32_t* mask_dev, float* d_scores, int64_t* d_rows, double* d_keys, int64_t* launches,
+                       int64_t* resweeps, cudaStream_t st) {
   // lists hold 8192 rows and so does the sample: ~k * stride rows pass the threshold it yields (1M rows, k = 10:
   // ~1200), so one sweep is enough unless k * rows / 8192 exceeds a list (then a second sweep with the tightened
   // threshold finishes it)
   const int cap = 8192, sample_cap = 8192, batch = 32, max_iter = 12;
   if (k > 1024)
     return set_error(RBOD_E_UNSUPPORTED, "rbod_search: k=%d > 1024", k);
-  const void* qd = nullptr;
-  RBOD_TRY(to_device(queries, (size_t)Q * g->dim * 4, g->q32, st, &qd));
-  const float* q_dev = static_cast<const float*>(qd);
   RBOD_TRY(g->dist_q64.ensure((size_t)batch * g->dim * 8));
   RBOD_TRY(g->dist_thr.ensure((size_t)2 * batch * 8 + (size_t)batch * 4));   // thresholds, query norms, row bounds
   RBOD_TRY(g->dist_ctl.ensure((size_t)(2 * batch + 1) * 4));
@@ -862,11 +862,15 @@ static int search_distance(rbod_gallery* g, const float* queries, int64_t Q, int
   std::vector<double> h_thr(batch, -INFINITY);
   std::vector<int> h_ctl(2 * batch + 1);
   const int64_t sample_stride = (g->rows + sample_cap - 1) / sample_cap;   // > 1 iff more than `sample_cap` rows
-  for (int64_t q0 = 0; q0 < Q; q0 += batch) {
-    const int nf = (int)std::min<int64_t>(batch, Q - q0);
+  for (int64_t q0 = 0; q0 < n; q0 += batch) {
+    const int nf = (int)std::min<int64_t>(batch, n - q0);
     for (int f = 0; f < batch; ++f) {
-      h_ctl[f] = (int)(q0 + std::min(f, nf - 1));
+      const int64_t i = q0 + std::min(f, nf - 1);
+      h_ctl[f] = qsel ? qsel[i] : (int)i;
       h_ctl[batch + f] = f < nf ? 1 : 0;
+      // kth was summed in another order than this sweep sums, so the very row that set it may come out an ulp lower
+      // here: seed a margin far above fp64 summation noise below it (-inf stays -inf)
+      if (kth) h_thr[f] = kth[i] - 1e-12 * std::max(1.0, std::fabs(kth[i]));
     }
     h_ctl[2 * batch] = 0;
     RBOD_CUDA(cudaMemcpyAsync(d_qsel, h_ctl.data(), h_ctl.size() * 4, cudaMemcpyHostToDevice, st));
@@ -876,7 +880,7 @@ static int search_distance(rbod_gallery* g, const float* queries, int64_t Q, int
     if (nf < batch) RBOD_CUDA(cudaMemsetAsync(g->dist_q64.p, 0, (size_t)batch * g->dim * 8, st));   // zero rows pad the batch
     RBOD_TRY(launch_dist_widen_queries(q_dev, d_qsel, nf, g->dim, g->dist_q64.as<double>(), d_qnorm, st));
     ++*launches;
-    if (sample_stride > 1) {
+    if (!kth && sample_stride > 1) {
       RBOD_TRY(launch_dist_collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim,
                                    g->dim, g->dp, g->rows, 0, sample_stride, mask_dev, d_thr, d_thr_row, d_active, d_qnorm, nf, cap,
                                    g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
@@ -902,7 +906,7 @@ static int search_distance(rbod_gallery* g, const float* queries, int64_t Q, int
       if (iter > 0) ++*resweeps;
     }
     if (left > 0)
-      return set_error(RBOD_E_OVERFLOW, "rbod_search: more than %d rows tie around the k-th distance of a query", cap);
+      return set_error(RBOD_E_OVERFLOW, "rbod_search: more than %d rows tie around the k-th key of a query", cap);
   }
   return RBOD_OK;
 }
@@ -1062,8 +1066,11 @@ int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, con
     }
     const void* md = nullptr;
     if (row_mask) RBOD_TRY(to_device(row_mask, (size_t)((g->rows + 31) / 32) * 4, g->mask_dev, st, &md));
+    const void* qd = nullptr;
+    RBOD_TRY(to_device(queries, (size_t)Q * g->dim * 4, g->q32, st, &qd));
     int64_t n_launch = 0, resweeps = 0;
-    RBOD_TRY(search_distance(g, queries, Q, k, static_cast<const uint32_t*>(md), ds, dr, dk, &n_launch, &resweeps, st));
+    RBOD_TRY(sweep_exact(g, static_cast<const float*>(qd), Q, nullptr, nullptr, k, static_cast<const uint32_t*>(md), ds,
+                         dr, dk, &n_launch, &resweeps, st));
     RBOD_TRY(copy_out(out_scores, ds, n_out * 4, st));
     RBOD_TRY(copy_out(out_rows, dr, n_out * 8, st));
     if (out_scores64) RBOD_TRY(copy_out(out_scores64, dk, n_out * 8, st));
@@ -1162,10 +1169,12 @@ int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, con
 
   int n_sweep = n_flag;   // queries that still need the exact fp64 sweep
   int64_t k3_launches = 1;
+  const int cap = K3_COLLECT_CAP;
+  std::vector<int> cnt_h(n_flag), fq_h(n_flag);
+  std::vector<double> thr_h(n_flag);
   if (n_flag > 0 && g->collect_pass) {
     // Second tensor-core pass over the uncertified queries only: record every row whose approximate
     // score can still reach the query's provisional k-th exact score, rescore those exactly, select.
-    const int cap = K3_COLLECT_CAP;
     SearchPlan P2;
     RBOD_TRY(plan_search(g, n_flag, k, search_variant(g, n_flag), smem_optin, &P2));
     RBOD_TRY(g->fq16.ensure((size_t)P2.q_pad * g->dp * 2));
@@ -1185,80 +1194,36 @@ int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, con
                                       g->coll_cnt.as<int>(), g->coll_score.as<double>(), st));
     RBOD_TRY(launch_select_collected(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
                                      g->flag_q.as<int>(), 0, n_flag, cap, k, g->metric, d_scores, d_rows, d_scores64,
-                                     nullptr, st));
+                                     st));
     launches += 4;
     ++k3_launches;
-    // queries whose list overflowed (a tie cluster wider than `cap`) keep going to the exact sweep
-    std::vector<int> cnt_h(n_flag), fq_h(n_flag);
-    std::vector<double> thr_h(n_flag);
     RBOD_CUDA(cudaMemcpyAsync(cnt_h.data(), g->coll_cnt.p, (size_t)n_flag * 4, cudaMemcpyDeviceToHost, st));
+  }
+  if (n_flag > 0) {
     RBOD_CUDA(cudaMemcpyAsync(fq_h.data(), g->flag_q.p, (size_t)n_flag * 4, cudaMemcpyDeviceToHost, st));
     RBOD_CUDA(cudaMemcpyAsync(thr_h.data(), g->flag_thr.p, (size_t)n_flag * 8, cudaMemcpyDeviceToHost, st));
     RBOD_CUDA(cudaStreamSynchronize(st));
-    n_sweep = 0;
-    for (int f = 0; f < n_flag; ++f)
-      if (cnt_h[f] > cap) {
-        fq_h[n_sweep] = fq_h[f];
-        thr_h[n_sweep] = thr_h[f];
-        ++n_sweep;
-      }
+    if (g->collect_pass) {
+      // queries whose list overflowed (a tie cluster wider than `cap`) keep going to the exact sweep
+      n_sweep = 0;
+      for (int f = 0; f < n_flag; ++f)
+        if (cnt_h[f] > cap) {
+          fq_h[n_sweep] = fq_h[f];
+          thr_h[n_sweep] = thr_h[f];
+          ++n_sweep;
+        }
+    }
     if (n_sweep > 0) {
-      RBOD_CUDA(cudaMemcpyAsync(g->flag_q.p, fq_h.data(), (size_t)n_sweep * 4, cudaMemcpyHostToDevice, st));
-      RBOD_CUDA(cudaMemcpyAsync(g->flag_thr.p, thr_h.data(), (size_t)n_sweep * 8, cudaMemcpyHostToDevice, st));
-      RBOD_CUDA(cudaStreamSynchronize(st));   // the host vectors go out of scope below
+      int64_t resweeps = 0;   // not reported: fallback_queries counts the uncertified queries here
+      RBOD_TRY(sweep_exact(g, q_dev, n_sweep, fq_h.data(), thr_h.data(), k, static_cast<const uint32_t*>(mask_dev),
+                           d_scores, d_rows, d_scores64, &launches, &resweeps, st));
     }
-  }
-  if (n_sweep > 0) {
-    const int cap = 4096, batch = 32, max_tighten = 12;
-    RBOD_TRY(g->coll_score.ensure((size_t)batch * cap * 8));
-    RBOD_TRY(g->coll_idx.ensure((size_t)batch * cap * 4));
-    RBOD_TRY(g->coll_cnt.ensure((size_t)batch * 4));
-    RBOD_TRY(g->flag_row.ensure((size_t)n_sweep * 4));
-    RBOD_TRY(g->sweep_ctl.ensure((size_t)(batch + 1) * 4));
-    RBOD_CUDA(cudaMemsetAsync(g->flag_row.p, 0xff, (size_t)n_sweep * 4, st));   // no row bound yet
-    int* d_active = g->sweep_ctl.as<int>();
-    int* d_nactive = d_active + batch;
-    for (int f0 = 0; f0 < n_sweep; f0 += batch) {
-      const int nf = std::min(batch, n_sweep - f0);
-      RBOD_CUDA(cudaMemsetAsync(g->coll_cnt.p, 0, (size_t)batch * 4, st));
-      const int* active = nullptr;   // first sweep: every query of the batch
-      for (int it = 0;; ++it) {
-        RBOD_TRY(launch_exact_collect(q_dev, g->q_qq.as<double>(), g->master32, g->rows16, g->kind16, g->dim, g->dim,
-                                      g->dp, g->metric, g->rows, static_cast<const uint32_t*>(mask_dev),
-                                      g->flag_q.as<int>(), g->flag_thr.as<double>(), g->flag_row.as<uint32_t>(), active, f0,
-                                      nf, cap, g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(),
-                                      g->coll_cnt.as<int>(), g->num_sms, st));
-        // lists that overflowed (a wide cluster of ties around the k-th score) are tightened to the k-th best
-        // (score, row) pair they did record and swept again, the others are left as they are
-        RBOD_CUDA(cudaMemsetAsync(d_nactive, 0, 4, st));
-        RBOD_TRY(launch_tighten(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(), f0, nf,
-                                cap, k, g->flag_thr.as<double>(), g->flag_row.as<uint32_t>(), d_active, d_nactive, st));
-        launches += 2;
-        int n_active = 0;
-        RBOD_CUDA(cudaMemcpyAsync(&n_active, d_nactive, 4, cudaMemcpyDeviceToHost, st));
-        RBOD_CUDA(cudaStreamSynchronize(st));
-        if (n_active == 0) break;
-        if (it >= max_tighten)
-          return set_error(RBOD_E_OVERFLOW, "rbod_search: a tie cluster around the k-th score did not resolve in %d sweeps",
-                           max_tighten);
-        active = d_active;
-      }
-      RBOD_TRY(launch_select_collected(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(),
-                                       g->coll_cnt.as<int>(), g->flag_q.as<int>(), f0, nf, cap, k, g->metric, d_scores,
-                                       d_rows, d_scores64, d_flags + 1, st));
-      ++launches;
-    }
-    RBOD_CUDA(cudaMemcpyAsync(hflags, d_flags, sizeof(hflags), cudaMemcpyDeviceToHost, st));
-  }
-  if (n_flag > 0) {
     // the second pass rewrote the flagged queries' rows of the answer
     RBOD_TRY(copy_out(out_scores, d_scores, nout * 4, st));
     RBOD_TRY(copy_out(out_rows, d_rows, nout * 8, st));
     if (out_scores64) RBOD_TRY(copy_out(out_scores64, d_scores64, nout * 8, st));
     RBOD_CUDA(cudaStreamSynchronize(st));
   }
-  if (hflags[1])
-    return set_error(RBOD_E_OVERFLOW, "rbod_search: more than 4096 rows tie around the k-th score of a query");
 
   if (stats) {
     stats->fallback_queries = n_flag;

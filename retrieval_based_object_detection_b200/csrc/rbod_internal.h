@@ -170,17 +170,10 @@ int launch_rescore_collected(const float* q, const double* q_qq, const float* ma
                              int kind16, int dim, int64_t ld32, int64_t ld16, int metric, const int* flag_q, int f0,
                              int nf, int cap, const uint32_t* coll_idx, const int* coll_cnt, double* coll_score,
                              cudaStream_t st);
-int launch_exact_collect(const float* q, const double* q_qq, const float* master32, const uint16_t* rows16,
-                         int kind16, int dim, int64_t ld32, int64_t ld16, int metric, int64_t n_rows,
-                         const uint32_t* row_mask, const int* flag_q, const double* flag_thr, const uint32_t* flag_row,
-                         const int* active, int f0, int nf, int cap, double* coll_score, uint32_t* coll_idx,
-                         int* coll_cnt, int num_sms, cudaStream_t st);
-int launch_tighten(const double* coll_score, const uint32_t* coll_idx, int* coll_cnt, int f0, int nf, int cap, int k,
-                   double* flag_thr, uint32_t* flag_row, int* active, int* n_active, cudaStream_t st);
 int launch_select_collected(const double* coll_score, const uint32_t* coll_idx, const int* coll_cnt,
                             const int* flag_q, int f0, int nf, int cap, int k, int metric, float* out_scores,
-                            int64_t* out_rows, double* out_scores64, int* overflow, cudaStream_t st);
-// K5 (EUCLID / MANHATTAN)
+                            int64_t* out_rows, double* out_scores64, cudaStream_t st);
+// K5: exact fp64 sweep (every metric)
 int launch_dist_widen_queries(const float* q, const int* qsel, int nf, int dim, double* q64, double* qnorm,
                               cudaStream_t st);
 int launch_dist_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
@@ -233,8 +226,8 @@ struct rbod_gallery {
   rbod::DevBuf q32, q16, q_dq, q_qq, tau_shared;              // query prep
   rbod::DevBuf lists, list_cnt;                                // K3 candidate lists
   rbod::DevBuf out_scores, out_rows, out_scores64;
-  rbod::DevBuf flags;      // ints: [0]=n_flag [1]=overflow [2]=err; float max_eps at [3]
-  rbod::DevBuf flag_q, flag_thr, flag_lo, flag_row, sweep_ctl, fq16, groupmax, tau_init;
+  rbod::DevBuf flags;      // ints: [0]=n_flag [2]=err; float max_eps at [3]; [4]=queries the pre-pass cut short
+  rbod::DevBuf flag_q, flag_thr, flag_lo, fq16, groupmax, tau_init;
   rbod::DevBuf coll_score, coll_idx, coll_cnt;
   rbod::DevBuf mask_dev, dump, sync_counters, prof;
   rbod::DevBuf sel_keys, sel_n, sel_tau;       // split search: the selection rbod_search_begin leaves for rbod_search_end

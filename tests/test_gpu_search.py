@@ -118,24 +118,29 @@ def test_duplicates_ties_and_fallback(G):
 
 
 def test_wide_tie_cluster_goes_to_exact_sweep(G):
-    """More identical rows than the collecting second pass records (1024): the fp64 sweep answers."""
+    """More identical rows than the collecting second pass records (1024): the fp64 sweep answers, its threshold
+    seeded with the k-th exact score of the first pass -- in the key domain of each metric that can reach it."""
     n, dim, k = 9000, 512, 10
-    g, stored, x = _mk(G, n, dim, "bf16", seed=5)
-    x2 = x.copy()
-    x2[3000:4200] = x2[17]                   # 1201 copies of row 17
-    g.upsert(x2, slots=np.arange(n))
-    stored = g.get_rows(np.arange(n))
-    q = np.stack([x2[17], x2[5000]]).astype(np.float32)
-    res = g.search(q, k, want_scores64=True)
-    ws, wi = OC.cosine_topk(q, stored, k)
-    assert np.array_equal(res.rows, wi)
-    assert list(res.rows[0]) == [17] + list(range(3000, 3009))
-    assert res.stats["fallback_queries"] >= 1 and res.stats["sweep_queries"] >= 1
-    assert res.stats["k3_launches"] == 2
-    g.set_option("collect_pass", 0)          # the sweep alone gives the same answer
-    res2 = g.search(q, k, want_scores64=True)
-    assert np.array_equal(res2.rows, wi) and res2.stats["k3_launches"] == 1
-    g.close()
+    x = O.synthetic_unit_rows(n, dim, seed=5)
+    x[3000:4200] = x[17]                     # 1201 copies of row 17
+    q = np.stack([x[17], x[5000]]).astype(np.float32)
+    for metric in ("cosine", "dot", "euclid"):
+        g = G(dim, dtype="bf16", metric=metric, capacity=n)
+        g.upsert(x)
+        stored = g.get_rows(np.arange(n))
+        res = g.search(q, k, want_scores64=True)
+        # sequential C oracle: identical rows -> identical scores
+        ws, wi = OC.cosine_topk(q, stored, k) if metric == "cosine" else OC.distance_topk(q, stored, k, metric)
+        assert np.array_equal(res.rows, wi), metric
+        assert list(res.rows[0]) == [17] + list(range(3000, 3009)), metric
+        assert np.allclose(res.scores64, ws, rtol=1e-5, atol=1e-9), metric
+        assert res.stats["fallback_queries"] >= 1 and res.stats["sweep_queries"] >= 1, metric
+        assert res.stats["k3_launches"] == 2, metric
+        g.set_option("collect_pass", 0)      # the sweep alone gives the same answer
+        res2 = g.search(q, k, want_scores64=True)
+        assert np.array_equal(res2.rows, wi) and res2.stats["k3_launches"] == 1, metric
+        assert res2.stats["sweep_queries"] >= 1, metric
+        g.close()
 
 
 def test_bf16_gallery_with_fp16_shadow_operand(G):
@@ -654,17 +659,17 @@ def test_upsert_accepts_device_resident_slots(G):
 
 @pytest.mark.parametrize("dtype", ["bf16", "f32"])
 def test_tie_cluster_wider_than_the_sweep_list_still_answers(G, dtype):
-    """More identical rows than even the exact sweep records per query (4096) -- the same image upserted under many
+    """More identical rows than even the exact sweep records per query (8192) -- the same image upserted under many
     ids, or a block of all-equal vectors: the search used to fail with RBOD_E_OVERFLOW.  The sweep now tightens an
     overflowing list to the k-th best (score, row) pair it did record and sweeps again, so the answer is the k
     smallest row slots of the tie, exactly as the (score desc, id asc) order says."""
-    n, dim = 14_000, 256
+    n, dim = 20_000, 256
     x = O.synthetic_unit_rows(n, dim, seed=77)
-    x[3000:9500] = x[17]                                   # 6501 copies of row 17
+    x[3000:13500] = x[17]                                  # 10501 copies of row 17
     g = G(dim, dtype=dtype, capacity=n)
     g.upsert(x)
     stored = g.get_rows(np.arange(n))
-    q = np.stack([x[17], x[12000], x[17] + 0.01 * x[12000]]).astype(np.float32)
+    q = np.stack([x[17], x[15000], x[17] + 0.01 * x[15000]]).astype(np.float32)
     for k in (10, 100):
         res = g.search(q, k, want_scores64=True)
         ws, wi = OC.cosine_topk(q, stored, k)              # sequential C oracle: identical rows -> identical scores

@@ -39,7 +39,7 @@ def launches(tag):
         a[0] += 1
         a[1] += v
     mine = ("k3_cosine", "rescore", "merge_partials", "prep_queries", "select_", "tau_init", "l2norm", "seg_", "gather_",
-            "merge_topk", "dist_", "exact_collect")
+            "merge_topk", "dist_")
     ours = {k: v for k, v in tot.items() if any(m in k for m in mine)}
     total, total_search = sum(v for _, v in tot.values()), sum(v for k, (_, v) in ours.items() if "l2norm" not in k)
     with open(os.path.join(PROF, f"{tag}_launches_bench_summary.txt"), "w") as f:
