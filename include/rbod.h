@@ -28,6 +28,9 @@
  *       from one pair to Q x N with top-k selection (client.search / query_points semantics).
  *       Distance.MANHATTAN collections (util/qdrant_manager.py:61-66), vectors wider than 768 columns and
  *       k > 128 are answered by kernel K5 distance_topk (exact fp64 sweep) behind the same entry point.
+ *   rbod_search_masks                              (the same kernels, one row mask per query)
+ *       client.search_batch(requests=[SearchRequest(vector, filter, limit, ...)]), one payload filter per
+ *       request (filters as at 32_create_delegate_vector.py:125-129, 33_run_all_experiments.py:98-103,117-137).
  *   rbod_merge_topk                                (kernel K4 topk_merge)
  *       no reference call site; merges per-GPU top-k lists after the NCCL all-gather.
  *
@@ -207,6 +210,22 @@ int rbod_segment_delegates(rbod_gallery* g, int32_t kind, const int64_t* row_idx
 int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, const uint32_t* row_mask,
                 float* out_scores, int64_t* out_rows, double* out_scores64, rbod_search_stats* stats,
                 void* stream);
+
+/* Like rbod_search, but each query has its own row mask (one filtered request per query, in one pass).
+ * row_masks:     [n_masks][ceil(rows/32)] uint32, the same bit layout as rbod_search's row_mask. Host or device.
+ *                NULL only when n_masks == 0.
+ * mask_of_query: [Q] int32, the mask each query uses. -1 means no filter. Host or device (a device array is read
+ *                back, Q * 4 bytes, to be checked before anything is launched).
+ *                NULL means every query uses mask 0 (or no mask when n_masks == 0).
+ * Every other argument and output is as for rbod_search.  An id outside [-1, n_masks), n_masks < 0, or n_masks > 0
+ * with row_masks == NULL is RBOD_E_INVAL.
+ * Result: row q is identical, bit for bit in out_scores / out_rows / out_scores64, to
+ * rbod_search(queries + q*dim, 1, k, row_masks + mask_of_query[q]*words, ...).
+ * rbod_search(..., row_mask, ...) is rbod_search_masks(..., row_mask, row_mask ? 1 : 0, NULL, ...).           */
+int rbod_search_masks(rbod_gallery* g, const float* queries, int64_t Q, int32_t k,
+                      const uint32_t* row_masks, int32_t n_masks, const int32_t* mask_of_query,
+                      float* out_scores, int64_t* out_rows, double* out_scores64,
+                      rbod_search_stats* stats, void* stream);
 
 /* --- K4: merge of per-shard top-k lists -------------------------------------------------
  * scores64 / ids: [G, Q, k] as produced by an all-gather of each rank's rbod_search output

@@ -238,16 +238,39 @@ class QdrantClient:
                                                 with_vectors, score_threshold))
 
     def search_batch(self, collection_name: str, requests=None, queries=None, k: Optional[int] = None,
-                     row_filter=None, **_ignored: Any):
-        """Two forms: ``requests=[SearchRequest]`` -> list of ScoredPoint lists (upstream API), or the
-        tensor form ``queries=[Q, dim], k=`` -> (scores [Q,k] float32, ids: list of Q lists)."""
+                     row_filter=None, query_filters=None, **_ignored: Any):
+        """Two forms: ``requests=[SearchRequest]`` -> list of ScoredPoint lists (upstream API), the same as one
+        ``search`` per request; or the tensor form ``queries=[Q, dim], k=`` -> (scores [Q,k] float32, ids: list of Q
+        lists), filtered by ``row_filter`` (every query) or ``query_filters`` (one filter or None per query)."""
         col = self._root.get(collection_name)
         if requests is not None:
-            return [self.search(collection_name, r.vector, r.filter, r.limit, r.offset or 0,
-                                bool(r.with_payload), bool(r.with_vector), r.score_threshold) for r in requests]
+            requests = list(requests)
+            vecs = []
+            for r in requests:
+                q = np.asarray(r.vector, dtype=np.float32).reshape(1, -1)
+                if q.shape[1] != col.dim:
+                    raise ValueError(f"Wrong input: Vector dimension error: expected dim: {col.dim}, got {q.shape[1]}")
+                vecs.append(q[0])
+            # one device search per distinct limit + offset: a large limit does not drag the others to a larger k
+            by_k: Dict[int, List[int]] = {}
+            for i, r in enumerate(requests):
+                by_k.setdefault(int(r.limit) + int(r.offset or 0), []).append(i)
+            out: List[List[ScoredPoint]] = [[] for _ in requests]
+            for kk, members in by_k.items():
+                if kk < 1:
+                    continue
+                scores, slots = col.search(np.stack([vecs[i] for i in members]), kk,
+                                           filters=[requests[i].filter for i in members])
+                for j, i in enumerate(members):
+                    r = requests[i]
+                    out[i] = self._scored(col, scores[j], slots[j], bool(r.with_payload), bool(r.with_vector),
+                                          r.score_threshold)[int(r.offset or 0):]
+            return out
         if queries is None or k is None:
             raise ValueError("search_batch needs either requests= or queries= and k=")
-        scores, slots = col.search(np.asarray(queries, dtype=np.float32), int(k), row_filter)
+        if row_filter is not None and query_filters is not None:
+            raise ValueError("search_batch: pass row_filter (every query) or query_filters (one per query), not both")
+        scores, slots = col.search(np.asarray(queries, dtype=np.float32), int(k), row_filter, filters=query_filters)
         id_of = np.asarray(col.ids + [None], dtype=object)          # slot -1 -> None through the last entry
         ids = id_of[np.asarray(slots)].tolist()
         return scores, ids

@@ -58,7 +58,9 @@ struct alignas(64) K3Params {
   int list_cap;           // a list is pruned back to ~kc entries once it holds this many (64, 128 or 256)
   int list_stride;        // list_cap + 128: a tile can append 128 entries before the capacity check
   int final_cap;          // lists longer than this get a last exact prune to kc entries (keeps the merge within 8192)
-  const uint32_t* row_mask;
+  const uint32_t* row_mask;   // [n_masks][mask_words] row bitmasks, or nullptr = every row allowed
+  const int* mask_of_query;   // [q_pad] mask each query row reads (-1 = none), or nullptr = every row reads mask 0
+  int64_t mask_words;
   const float* row_bias;  // BIAS kernels (EUCLID collections): score = q . g + row_bias[row], row_bias = -|g|^2 / 2
   uint32_t* tau_shared;   // [q_pad] per-query lower bound on the kc-th best score, as ordered keys (nullptr = off)
   const float* collect_thr;   // collect mode: [q_pad] fixed per-query thresholds; every row scoring above is recorded
@@ -637,6 +639,9 @@ __global__ void __launch_bounds__(K3_THREADS, 1) k3_cosine_topk_kernel(const __g
         }
 
         if (col0 + K3_TILE_N > P.n_rows || P.row_mask != nullptr) {
+          // the mask this row's query reads (index into P.row_mask), -1 = none; pad rows of the tile read none.  Looked
+          // up per tile (an L1 hit) rather than held in a register across the tile loop, which is at its register limit.
+          const int mask_id = P.mask_of_query == nullptr ? 0 : (qg < P.q_valid ? __ldg(P.mask_of_query + qg) : -1);
 #pragma unroll
           for (int half = 0; half < 2; ++half) {
             const int64_t c0 = col0 + 64 * half;
@@ -645,11 +650,13 @@ __global__ void __launch_bounds__(K3_THREADS, 1) k3_cosine_topk_kernel(const __g
               const int64_t valid = P.n_rows - c0;
               allow = valid <= 0 ? 0ull : (valid >= 64 ? ~0ull : ((1ull << valid) - 1ull));
             }
-            if (P.row_mask != nullptr) {
+            if (P.row_mask != nullptr && mask_id >= 0) {
+              // one broadcast address per warp with a shared mask; per-query masks read the row's own words (L1 / L2)
+              const uint32_t* mask = P.row_mask + (int64_t)mask_id * P.mask_words;
               const int64_t w0 = c0 >> 5;
               const int64_t nwords = (P.n_rows + 31) >> 5;
-              const uint64_t lo = w0 < nwords ? P.row_mask[w0] : 0u;
-              const uint64_t hi = (w0 + 1) < nwords ? P.row_mask[w0 + 1] : 0u;
+              const uint64_t lo = w0 < nwords ? mask[w0] : 0u;
+              const uint64_t hi = (w0 + 1) < nwords ? mask[w0 + 1] : 0u;
               allow &= (lo | (hi << 32));
             }
 #pragma unroll
@@ -945,6 +952,8 @@ int launch_k3(const K3Launch& L, cudaStream_t st) {
   P.list_stride = L.list_stride;
   P.final_cap = L.final_cap;
   P.row_mask = L.row_mask;
+  P.mask_of_query = L.mask_of_query;
+  P.mask_words = L.mask_words;
   P.row_bias = L.row_bias;
   P.tau_shared = L.tau_shared;
   P.collect_thr = L.collect_thr;

@@ -656,7 +656,8 @@ select_collected_kernel(const double* __restrict__ coll_score, const uint32_t* _
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 gather_flagged_kernel(const uint16_t* __restrict__ q16, int dp, const int* __restrict__ flag_q, int f0, int nf,
-                      int64_t nf_pad, uint16_t* __restrict__ fq16, int* __restrict__ coll_cnt) {
+                      int64_t nf_pad, uint16_t* __restrict__ fq16, int* __restrict__ coll_cnt,
+                      const int* __restrict__ mask_of_query, int* __restrict__ fmask) {
   const int lane = threadIdx.x & 31;
   const int64_t w0 = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
   const int64_t nw = (int64_t)gridDim.x * 8;
@@ -668,7 +669,11 @@ gather_flagged_kernel(const uint16_t* __restrict__ q16, int dp, const int* __res
     } else {
       for (int c = lane; c < dp / 8; c += 32) dst[c] = make_uint4(0u, 0u, 0u, 0u);
     }
-    if (lane == 0) coll_cnt[f] = 0;
+    if (lane == 0) {
+      coll_cnt[f] = 0;
+      // per-query masks: the gathered row keeps its query's mask (pad rows read none)
+      if (mask_of_query != nullptr) fmask[f] = f < nf ? mask_of_query[flag_q[f0 + f]] : -1;
+    }
   }
 }
 
@@ -798,11 +803,12 @@ int launch_select_collected(const double* coll_score, const uint32_t* coll_idx, 
 }
 
 int launch_gather_flagged(const uint16_t* q16, int dp, const int* flag_q, int f0, int nf, int64_t nf_pad,
-                          uint16_t* fq16, int* coll_cnt, cudaStream_t st) {
+                          uint16_t* fq16, int* coll_cnt, const int* mask_of_query, int* fmask, cudaStream_t st) {
   if (nf_pad <= 0) return RBOD_OK;
   const int64_t want = (nf_pad + 7) / 8;
   gather_flagged_kernel<<<(unsigned)(want < 148 * 8 ? want : 148 * 8), 256, 0, st>>>(q16, dp, flag_q, f0, nf, nf_pad,
-                                                                                    fq16, coll_cnt);
+                                                                                    fq16, coll_cnt, mask_of_query,
+                                                                                    fmask);
   RBOD_CUDA(cudaGetLastError());
   return RBOD_OK;
 }

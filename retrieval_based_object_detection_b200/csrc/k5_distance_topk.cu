@@ -69,7 +69,7 @@ __global__ void __launch_bounds__(256, 1)
 dist_collect_kernel(const double* __restrict__ q64, const float* __restrict__ master32,
                     const uint16_t* __restrict__ rows16, int kind16, int dim, int64_t ld32, int64_t ld16,
                     int64_t n_rows, int64_t row0, int64_t stride, const uint32_t* __restrict__ row_mask,
-                    const double* __restrict__ thr, const uint32_t* __restrict__ thr_row, const int* __restrict__ active,
+                    int64_t mask_words, const int* __restrict__ slot_mask, const double* __restrict__ thr, const uint32_t* __restrict__ thr_row, const int* __restrict__ active,
                     const double* __restrict__ qnorm, int nf, int cap, double* __restrict__ coll_key,
                     uint32_t* __restrict__ coll_idx, int* __restrict__ coll_cnt) {
   extern __shared__ __align__(16) uint8_t k5_smem[];
@@ -80,10 +80,12 @@ dist_collect_kernel(const double* __restrict__ q64, const float* __restrict__ ma
   uint32_t* xs = reinterpret_cast<uint32_t*>(k5_smem + (size_t)2 * NQ * K5_CH * 8);  // [2][8][32][pitch]
   __shared__ double thr_s[32], qn_s[32];
   __shared__ uint32_t thr_row_s[32];   // with thr_s a (key, row) pair bound: rows tying with the key count up to this row
+  __shared__ int mask_s[32];            // per-query masks: the mask slot f reads, -1 = none
   if (threadIdx.x < 32) {
     thr_s[threadIdx.x] = (threadIdx.x < nf && active[threadIdx.x]) ? thr[threadIdx.x] : INFINITY;
     thr_row_s[threadIdx.x] = (threadIdx.x < nf && thr_row != nullptr) ? thr_row[threadIdx.x] : 0xffffffffu;
     qn_s[threadIdx.x] = threadIdx.x < nf ? qnorm[threadIdx.x] : 0.0;
+    mask_s[threadIdx.x] = (threadIdx.x < nf && slot_mask != nullptr) ? slot_mask[threadIdx.x] : -1;
   }
   __syncthreads();
   constexpr bool kInner = METRIC == RBOD_COSINE || METRIC == RBOD_DOT;   // keys built from q . g
@@ -99,7 +101,8 @@ dist_collect_kernel(const double* __restrict__ q64, const float* __restrict__ ma
     const int64_t v = (blockIdx.x + g * gridDim.x) * K5_ROWS + warp * 32 + l;
     if (v >= n_visit) return -1;
     const int64_t r = row0 + v * stride;
-    if (row_mask != nullptr && !((row_mask[r >> 5] >> (r & 31)) & 1u)) return -1;
+    // one mask for the whole batch: masked rows are not even loaded
+    if (row_mask != nullptr && slot_mask == nullptr && !((row_mask[r >> 5] >> (r & 31)) & 1u)) return -1;
     return r;
   };
   auto issue = [&](int64_t step, int b) {
@@ -197,7 +200,9 @@ dist_collect_kernel(const double* __restrict__ q64, const float* __restrict__ ma
           // thr_s is +inf for slots beyond the batch and for finished queries; a list that overflowed was tightened to
           // the k-th best (key, row) pair it had recorded, so a cluster of duplicates wider than the list resolves to
           // its smallest row slots instead of overflowing for ever
-          if (key > thr_s[f] || (key == thr_s[f] && (uint32_t)r <= thr_row_s[f])) {
+          // per-query masks (slot_mask != nullptr): a row slot f's mask excludes is never recorded for it
+          if ((key > thr_s[f] || (key == thr_s[f] && (uint32_t)r <= thr_row_s[f])) &&
+              (mask_s[f] < 0 || ((row_mask[(int64_t)mask_s[f] * mask_words + (r >> 5)] >> (r & 31)) & 1u))) {
             const int slot = atomicAdd(coll_cnt + f, 1);
             if (slot < cap) {
               coll_key[(size_t)f * cap + slot] = key;
@@ -304,9 +309,9 @@ int launch_dist_widen_queries(const float* q, const int* qsel, int nf, int dim, 
 
 int launch_dist_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
                         int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride,
-                        const uint32_t* row_mask, const double* thr, const uint32_t* thr_row, const int* active,
-                        const double* qnorm, int nf, int cap, double* coll_key, uint32_t* coll_idx, int* coll_cnt,
-                        int num_sms, cudaStream_t st) {
+                        const uint32_t* row_mask, int64_t mask_words, const int* slot_mask, const double* thr,
+                        const uint32_t* thr_row, const int* active, const double* qnorm, int nf, int cap,
+                        double* coll_key, uint32_t* coll_idx, int* coll_cnt, int num_sms, cudaStream_t st) {
   if (nf <= 0 || n_rows <= 0) return RBOD_OK;
   if (nf > 32) return set_error(RBOD_E_INVAL, "dist_collect: at most 32 queries per pass");
   const int64_t rows_visited = (n_rows - row0 + stride - 1) / stride;
@@ -319,7 +324,8 @@ int launch_dist_collect(int metric, const double* q64, const float* master32, co
     RBOD_CUDA(cudaFuncSetAttribute(dist_collect_kernel<METRIC, NQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                    (int)smem));                                                                \
     dist_collect_kernel<METRIC, NQ><<<grid, 256, smem, st>>>(q64, master32, rows16, kind16, dim, ld32, ld16,    \
-                                                             n_rows, row0, stride, row_mask, thr, thr_row, active, \
+                                                             n_rows, row0, stride, row_mask, mask_words,       \
+                                                             slot_mask, thr, thr_row, active,                  \
                                                              qnorm, nf, cap, coll_key, coll_idx, coll_cnt);    \
   } while (0)
   // 8 accumulators per lane for batches of up to 8 queries (single-query searches of the scripts), 32 otherwise

@@ -292,7 +292,7 @@ int rbod_destroy(rbod_gallery* g) {
   DevBuf* bufs[] = {&g->stage_rows, &g->stage_slots, &g->stage_norms, &g->q32, &g->q16, &g->q_dq, &g->q_qq, &g->tau_shared,
                     &g->lists, &g->list_cnt, &g->out_scores,
                     &g->out_rows, &g->out_scores64, &g->flags, &g->flag_q, &g->flag_thr, &g->flag_lo, &g->fq16, &g->groupmax, &g->tau_init, &g->coll_score,
-                    &g->coll_idx, &g->coll_cnt, &g->mask_dev, &g->dump, &g->sync_counters, &g->prof, &g->seg_idx, &g->seg_off, &g->seg_out,
+                    &g->coll_idx, &g->coll_cnt, &g->mask_dev, &g->mask_ids, &g->fmask_ids, &g->dump, &g->sync_counters, &g->prof, &g->seg_idx, &g->seg_off, &g->seg_out,
                     &g->seg_partials, &g->seg_prefix, &g->seg_arrive, &g->seg_scratch, &g->seg_member, &g->gather_idx,
                     &g->gather_out, &g->dist_q64, &g->dist_thr, &g->dist_ctl};
   for (DevBuf* b : bufs) b->release();
@@ -319,7 +319,7 @@ int rbod_info(const rbod_gallery* g, rbod_gallery_info* out) {
   out->coop_refusals = g->coop_refusals;
   size_t ws = 0;
   const DevBuf* bufs[] = {&g->stage_rows, &g->q32, &g->q16, &g->lists, &g->list_cnt, &g->out_scores, &g->out_rows, &g->out_scores64, &g->coll_score,
-                          &g->coll_idx, &g->mask_dev, &g->dump, &g->seg_idx, &g->seg_out, &g->seg_partials,
+                          &g->coll_idx, &g->mask_dev, &g->mask_ids, &g->fmask_ids, &g->dump, &g->seg_idx, &g->seg_out, &g->seg_partials,
                           &g->gather_out};
   for (const DevBuf* b : bufs) ws += b->cap;
   out->bytes_device = (int64_t)(gallery_bytes(g) + ws);
@@ -713,7 +713,17 @@ struct K3Sample {
   int stride, tiles, splits;
 };
 
-static int run_k3(rbod_gallery* g, const SearchPlan& P, int64_t Q, const uint16_t* q16, const uint32_t* mask_dev,
+// Row masks of one search.  `dev`: [n_masks][words] bitmasks on the device, nullptr = no filter.  `of_query`: the mask
+// each query row of the K3 launch reads ([q_pad] on the device, -1 = none) and `of_query_host` the same ids by original
+// query index ([Q] on the host, read by the sweep's batch control); both nullptr = every query reads mask 0.
+struct SearchMasks {
+  const uint32_t* dev;
+  int64_t words;
+  const int* of_query;
+  const int* of_query_host;
+};
+
+static int run_k3(rbod_gallery* g, const SearchPlan& P, int64_t Q, const uint16_t* q16, const SearchMasks& M,
                   const K3Collect* collect, float* dump, int64_t dump_ld, cudaStream_t st,
                   const K3Sample* sample = nullptr) {
   K3Launch L;
@@ -754,7 +764,9 @@ static int run_k3(rbod_gallery* g, const SearchPlan& P, int64_t Q, const uint16_
   L.list_cap = P.list_cap;
   L.list_stride = P.list_stride;
   L.final_cap = P.final_cap;
-  L.row_mask = mask_dev;
+  L.row_mask = M.dev;
+  L.mask_of_query = M.dev != nullptr ? M.of_query : nullptr;
+  L.mask_words = M.words;
   L.row_bias = g->metric == RBOD_EUCLID ? g->row_bias : nullptr;
   L.tau_shared = (g->tau_share && dump == nullptr && collect == nullptr && sample == nullptr)
                      ? g->tau_shared.as<uint32_t>() : nullptr;
@@ -839,7 +851,7 @@ static int prepare_queries(rbod_gallery* g, const float* queries, int64_t Q, con
 // one per listed query, or null) is each query's provisional k-th key, -inf if it had fewer than k candidates: a
 // lower bound of the true k-th key that replaces the sample pass as the starting threshold.
 static int sweep_exact(rbod_gallery* g, const float* q_dev, int64_t n, const int* qsel, const double* kth, int k,
-                       const uint32_t* mask_dev, float* d_scores, int64_t* d_rows, double* d_keys, int64_t* launches,
+                       const SearchMasks& M, float* d_scores, int64_t* d_rows, double* d_keys, int64_t* launches,
                        int64_t* resweeps, cudaStream_t st) {
   // lists hold 8192 rows and so does the sample: ~k * stride rows pass the threshold it yields (1M rows, k = 10:
   // ~1200), so one sweep is enough unless k * rows / 8192 exceeds a list (then a second sweep with the tightened
@@ -849,18 +861,20 @@ static int sweep_exact(rbod_gallery* g, const float* q_dev, int64_t n, const int
     return set_error(RBOD_E_UNSUPPORTED, "rbod_search: k=%d > 1024", k);
   RBOD_TRY(g->dist_q64.ensure((size_t)batch * g->dim * 8));
   RBOD_TRY(g->dist_thr.ensure((size_t)2 * batch * 8 + (size_t)batch * 4));   // thresholds, query norms, row bounds
-  RBOD_TRY(g->dist_ctl.ensure((size_t)(2 * batch + 1) * 4));
+  RBOD_TRY(g->dist_ctl.ensure((size_t)(3 * batch + 1) * 4));
   RBOD_TRY(g->coll_score.ensure((size_t)batch * cap * 8));
   RBOD_TRY(g->coll_idx.ensure((size_t)batch * cap * 4));
   RBOD_TRY(g->coll_cnt.ensure((size_t)batch * 4));
   int* d_qsel = g->dist_ctl.as<int>();
   int* d_active = d_qsel + batch;
   int* d_nactive = d_qsel + 2 * batch;
+  const bool per_query = M.dev != nullptr && M.of_query_host != nullptr;
+  const int* d_slot_mask = per_query ? d_qsel + 2 * batch + 1 : nullptr;   // the mask each slot of the batch reads
   double* d_thr = g->dist_thr.as<double>();
   double* d_qnorm = d_thr + batch;
   uint32_t* d_thr_row = reinterpret_cast<uint32_t*>(d_qnorm + batch);
   std::vector<double> h_thr(batch, -INFINITY);
-  std::vector<int> h_ctl(2 * batch + 1);
+  std::vector<int> h_ctl(3 * batch + 1, -1);
   const int64_t sample_stride = (g->rows + sample_cap - 1) / sample_cap;   // > 1 iff more than `sample_cap` rows
   for (int64_t q0 = 0; q0 < n; q0 += batch) {
     const int nf = (int)std::min<int64_t>(batch, n - q0);
@@ -868,6 +882,7 @@ static int sweep_exact(rbod_gallery* g, const float* q_dev, int64_t n, const int
       const int64_t i = q0 + std::min(f, nf - 1);
       h_ctl[f] = qsel ? qsel[i] : (int)i;
       h_ctl[batch + f] = f < nf ? 1 : 0;
+      if (per_query) h_ctl[2 * batch + 1 + f] = f < nf ? M.of_query_host[h_ctl[f]] : -1;
       // kth was summed in another order than this sweep sums, so the very row that set it may come out an ulp lower
       // here: seed a margin far above fp64 summation noise below it (-inf stays -inf)
       if (kth) h_thr[f] = kth[i] - 1e-12 * std::max(1.0, std::fabs(kth[i]));
@@ -882,7 +897,8 @@ static int sweep_exact(rbod_gallery* g, const float* q_dev, int64_t n, const int
     ++*launches;
     if (!kth && sample_stride > 1) {
       RBOD_TRY(launch_dist_collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim,
-                                   g->dim, g->dp, g->rows, 0, sample_stride, mask_dev, d_thr, d_thr_row, d_active, d_qnorm, nf, cap,
+                                   g->dim, g->dp, g->rows, 0, sample_stride, M.dev, M.words, d_slot_mask, d_thr, d_thr_row,
+                                   d_active, d_qnorm, nf, cap,
                                    g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
                                    g->num_sms, st));
       RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
@@ -894,7 +910,8 @@ static int sweep_exact(rbod_gallery* g, const float* q_dev, int64_t n, const int
     for (; iter < max_iter && left > 0; ++iter) {
       RBOD_CUDA(cudaMemsetAsync(d_nactive, 0, 4, st));
       RBOD_TRY(launch_dist_collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim,
-                                   g->dim, g->dp, g->rows, 0, 1, mask_dev, d_thr, d_thr_row, d_active, d_qnorm, nf, cap,
+                                   g->dim, g->dp, g->rows, 0, 1, M.dev, M.words, d_slot_mask, d_thr, d_thr_row, d_active,
+                                   d_qnorm, nf, cap,
                                    g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
                                    g->num_sms, st));
       RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
@@ -948,7 +965,7 @@ static bool presample_pays(const rbod_gallery* g, const SearchPlan& P, int64_t Q
 
 // Everything of a search up to and including the main K3 launch: flags cleared, queries prepared, the optional
 // threshold pre-pass, the candidate lists filled.
-static int launch_front(rbod_gallery* g, const float* queries, int64_t Q, const SearchPlan& P, const uint32_t* mask_dev,
+static int launch_front(rbod_gallery* g, const float* queries, int64_t Q, const SearchPlan& P, const SearchMasks& M,
                         bool use_sample, int sample_tiles, cudaStream_t st, const float** q_dev_out,
                         const float** tau_init_out, int64_t* launches_io, Trace& tr) {
   int64_t launches = *launches_io;
@@ -973,14 +990,13 @@ static int launch_front(rbod_gallery* g, const float* queries, int64_t Q, const 
     S.tiles = sample_tiles;
     S.stride = P.tiles_total / sample_tiles;
     S.splits = splits;
-    RBOD_TRY(run_k3(g, PA, Q, g->q16.as<uint16_t>(), mask_dev, nullptr, nullptr, 0, st,
-                    &S));
+    RBOD_TRY(run_k3(g, PA, Q, g->q16.as<uint16_t>(), M, nullptr, nullptr, 0, st, &S));
     RBOD_TRY(launch_tau_init(g->groupmax.as<float>(), K3_SAMPLE_GROUPS, splits, P.q_pad,
                              g->tau_shared.as<uint32_t>(), g->tau_init.as<float>(), st));
     tau_init = g->tau_init.as<float>();
     launches += 2;
   }
-  RBOD_TRY(run_k3(g, P, Q, g->q16.as<uint16_t>(), mask_dev, nullptr, nullptr, 0, st));
+  RBOD_TRY(run_k3(g, P, Q, g->q16.as<uint16_t>(), M, nullptr, nullptr, 0, st));
   if (g->time_k3) RBOD_CUDA(cudaEventRecord(g->ev1, st));
   ++launches;
   tr.mark("k3_launches");
@@ -1028,12 +1044,15 @@ static void fill_finish(rbod_gallery* g, const SearchPlan& P, int k, const float
   F.max_eps = reinterpret_cast<float*>(d_flags + 3);
 }
 
-int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, const uint32_t* row_mask,
-                float* out_scores, int64_t* out_rows, double* out_scores64, rbod_search_stats* stats,
-                void* stream) {
+// rbod_search and rbod_search_masks: a search with one shared mask is the case "every query reads mask 0".
+static int search_impl(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, const uint32_t* row_masks,
+                       int32_t n_masks, const int32_t* mask_of_query, float* out_scores, int64_t* out_rows,
+                       double* out_scores64, rbod_search_stats* stats, void* stream) {
   if (!g) return set_error(RBOD_E_INVAL, "rbod_search: NULL handle");
   if (Q < 0 || k < 1 || (Q > 0 && (!queries || !out_scores || !out_rows)))
     return set_error(RBOD_E_INVAL, "rbod_search: bad arguments");
+  if (n_masks < 0 || (n_masks > 0 && !row_masks))
+    return set_error(RBOD_E_INVAL, "rbod_search_masks: %d masks, row_masks %s", n_masks, row_masks ? "set" : "NULL");
   if (stats) memset(stats, 0, sizeof(*stats));
   g->pending.valid = 0;   // a full search reuses the query buffers a pending rbod_search_begin left behind
   if (Q == 0) return RBOD_OK;
@@ -1045,6 +1064,25 @@ int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, con
   if (g->rows >= 0xffffffffll) return set_error(RBOD_E_UNSUPPORTED, "rbod_search: more than 2^32-2 rows per shard");
   RBOD_CUDA(cudaSetDevice(g->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+
+  // Per-query mask ids are checked on the host before anything is launched; the sweep's batch control reads them there
+  // too.  Without masks every id is -1: a plain search.
+  std::vector<int> ids_host;
+  if (mask_of_query != nullptr) {
+    ids_host.resize((size_t)Q);
+    if (is_device_ptr(mask_of_query)) {
+      RBOD_CUDA(cudaMemcpyAsync(ids_host.data(), mask_of_query, (size_t)Q * 4, cudaMemcpyDeviceToHost, st));
+      RBOD_CUDA(cudaStreamSynchronize(st));
+    } else {
+      memcpy(ids_host.data(), mask_of_query, (size_t)Q * 4);
+    }
+    for (int64_t q = 0; q < Q; ++q)
+      if (ids_host[q] < -1 || ids_host[q] >= n_masks)
+        return set_error(RBOD_E_INVAL, "rbod_search_masks: mask_of_query[%lld] = %d is outside [-1, %d)", (long long)q,
+                         ids_host[q], n_masks);
+    if (n_masks == 0) ids_host.clear();
+  }
+  SearchMasks M = {nullptr, (g->rows + 31) / 32, nullptr, ids_host.empty() ? nullptr : ids_host.data()};
 
   if (distance_metric) {
     const size_t n_out = (size_t)Q * k;
@@ -1065,12 +1103,13 @@ int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, con
       return RBOD_OK;
     }
     const void* md = nullptr;
-    if (row_mask) RBOD_TRY(to_device(row_mask, (size_t)((g->rows + 31) / 32) * 4, g->mask_dev, st, &md));
+    if (n_masks > 0) RBOD_TRY(to_device(row_masks, (size_t)n_masks * M.words * 4, g->mask_dev, st, &md));
+    M.dev = static_cast<const uint32_t*>(md);
     const void* qd = nullptr;
     RBOD_TRY(to_device(queries, (size_t)Q * g->dim * 4, g->q32, st, &qd));
     int64_t n_launch = 0, resweeps = 0;
-    RBOD_TRY(sweep_exact(g, static_cast<const float*>(qd), Q, nullptr, nullptr, k, static_cast<const uint32_t*>(md), ds,
-                         dr, dk, &n_launch, &resweeps, st));
+    RBOD_TRY(sweep_exact(g, static_cast<const float*>(qd), Q, nullptr, nullptr, k, M, ds, dr, dk, &n_launch, &resweeps,
+                         st));
     RBOD_TRY(copy_out(out_scores, ds, n_out * 4, st));
     RBOD_TRY(copy_out(out_rows, dr, n_out * 8, st));
     if (out_scores64) RBOD_TRY(copy_out(out_scores64, dk, n_out * 8, st));
@@ -1124,7 +1163,16 @@ int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, con
   }
 
   const void* mask_dev = nullptr;
-  if (row_mask) RBOD_TRY(to_device(row_mask, (size_t)((g->rows + 31) / 32) * 4, g->mask_dev, st, &mask_dev));
+  if (n_masks > 0) RBOD_TRY(to_device(row_masks, (size_t)n_masks * M.words * 4, g->mask_dev, st, &mask_dev));
+  M.dev = static_cast<const uint32_t*>(mask_dev);
+  if (M.of_query_host != nullptr) {
+    // the K3 launches read one id per query row of the padded tile: pad rows read no mask
+    ids_host.resize((size_t)P.q_pad, -1);
+    M.of_query_host = ids_host.data();
+    RBOD_TRY(g->mask_ids.ensure((size_t)P.q_pad * 4));
+    RBOD_CUDA(cudaMemcpyAsync(g->mask_ids.p, ids_host.data(), (size_t)P.q_pad * 4, cudaMemcpyHostToDevice, st));
+    M.of_query = g->mask_ids.as<int>();
+  }
 
   RBOD_TRY(ensure_lists(g, P));
   RBOD_TRY(g->flag_q.ensure((size_t)Q * 4));
@@ -1138,8 +1186,7 @@ int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, con
   int64_t retries = 0;
   for (int attempt = 0;; ++attempt) {
     const float* tau_init = nullptr;
-    RBOD_TRY(launch_front(g, queries, Q, P, static_cast<const uint32_t*>(mask_dev), use_sample, sample_tiles, st, &q_dev,
-                          &tau_init, &launches, tr));
+    RBOD_TRY(launch_front(g, queries, Q, P, M, use_sample, sample_tiles, st, &q_dev, &tau_init, &launches, tr));
     FinishArgs F;
     fill_finish(g, P, k, tau_init, q_dev, d_scores, d_rows, d_scores64, &F);
     RBOD_TRY(launch_finish(F, Q, st));
@@ -1181,14 +1228,20 @@ int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, con
     RBOD_TRY(g->coll_cnt.ensure((size_t)P2.q_pad * 4));
     RBOD_TRY(g->coll_idx.ensure((size_t)P2.q_pad * cap * 4));
     RBOD_TRY(g->coll_score.ensure((size_t)n_flag * cap * 8));
+    SearchMasks M2 = M;   // the gathered query rows keep their queries' masks
+    if (M.of_query != nullptr) {
+      RBOD_TRY(g->fmask_ids.ensure((size_t)P2.q_pad * 4));
+      M2.of_query = g->fmask_ids.as<int>();
+    }
     RBOD_TRY(launch_gather_flagged(g->q16.as<uint16_t>(), g->dp, g->flag_q.as<int>(), 0, n_flag, P2.q_pad,
-                                   g->fq16.as<uint16_t>(), g->coll_cnt.as<int>(), st));
+                                   g->fq16.as<uint16_t>(), g->coll_cnt.as<int>(), M.of_query, g->fmask_ids.as<int>(),
+                                   st));
     K3Collect C;
     C.thr = g->flag_lo.as<float>();
     C.idx = g->coll_idx.as<uint32_t>();
     C.cnt = g->coll_cnt.as<int>();
     C.cap = cap;
-    RBOD_TRY(run_k3(g, P2, n_flag, g->fq16.as<uint16_t>(), static_cast<const uint32_t*>(mask_dev), &C, nullptr, 0, st));
+    RBOD_TRY(run_k3(g, P2, n_flag, g->fq16.as<uint16_t>(), M2, &C, nullptr, 0, st));
     RBOD_TRY(launch_rescore_collected(q_dev, g->q_qq.as<double>(), g->master32, g->rows16, g->kind16, g->dim, g->dim,
                                       g->dp, g->metric, g->flag_q.as<int>(), 0, n_flag, cap, g->coll_idx.as<uint32_t>(),
                                       g->coll_cnt.as<int>(), g->coll_score.as<double>(), st));
@@ -1215,8 +1268,8 @@ int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, con
     }
     if (n_sweep > 0) {
       int64_t resweeps = 0;   // not reported: fallback_queries counts the uncertified queries here
-      RBOD_TRY(sweep_exact(g, q_dev, n_sweep, fq_h.data(), thr_h.data(), k, static_cast<const uint32_t*>(mask_dev),
-                           d_scores, d_rows, d_scores64, &launches, &resweeps, st));
+      RBOD_TRY(sweep_exact(g, q_dev, n_sweep, fq_h.data(), thr_h.data(), k, M, d_scores, d_rows, d_scores64, &launches,
+                           &resweeps, st));
     }
     // the second pass rewrote the flagged queries' rows of the answer
     RBOD_TRY(copy_out(out_scores, d_scores, nout * 4, st));
@@ -1239,6 +1292,20 @@ int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, con
     }
   }
   return RBOD_OK;
+}
+
+int rbod_search(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, const uint32_t* row_mask,
+                float* out_scores, int64_t* out_rows, double* out_scores64, rbod_search_stats* stats,
+                void* stream) {
+  return search_impl(g, queries, Q, k, row_mask, row_mask ? 1 : 0, nullptr, out_scores, out_rows, out_scores64, stats,
+                     stream);
+}
+
+int rbod_search_masks(rbod_gallery* g, const float* queries, int64_t Q, int32_t k, const uint32_t* row_masks,
+                      int32_t n_masks, const int32_t* mask_of_query, float* out_scores, int64_t* out_rows,
+                      double* out_scores64, rbod_search_stats* stats, void* stream) {
+  return search_impl(g, queries, Q, k, row_masks, n_masks, mask_of_query, out_scores, out_rows, out_scores64, stats,
+                     stream);
 }
 
 // ---- split search: the two halves of rbod_search around an exchange between shards ---------------------------
@@ -1294,8 +1361,8 @@ int rbod_search_begin(rbod_gallery* g, const float* queries, int64_t Q, int32_t 
   const float* q_dev = nullptr;
   const float* tau_init = nullptr;
   int64_t launches = 0;
-  RBOD_TRY(launch_front(g, queries, Q, P, static_cast<const uint32_t*>(mask_dev), use_sample, sample_tiles, st, &q_dev,
-                        &tau_init, &launches, tr));
+  const SearchMasks M = {static_cast<const uint32_t*>(mask_dev), (g->rows + 31) / 32, nullptr, nullptr};
+  RBOD_TRY(launch_front(g, queries, Q, P, M, use_sample, sample_tiles, st, &q_dev, &tau_init, &launches, tr));
   FinishArgs F;
   fill_finish(g, P, k, tau_init, q_dev, nullptr, nullptr, nullptr, &F);
   F.mode = FIN_SELECT;
@@ -1435,7 +1502,8 @@ int rbod_debug_scores(rbod_gallery* g, const float* queries, int64_t Q, float* o
     dst = g->dump.as<float>();
   }
   RBOD_CUDA(cudaMemsetAsync(dst, 0xff, (size_t)Q * ld * 4, st));  // NaN pattern: unwritten cells show up
-  RBOD_TRY(run_k3(g, P, Q, g->q16.as<uint16_t>(), nullptr, nullptr, dst, ld, st));
+  const SearchMasks none = {nullptr, 0, nullptr, nullptr};
+  RBOD_TRY(run_k3(g, P, Q, g->q16.as<uint16_t>(), none, nullptr, dst, ld, st));
   if (!out_dev) RBOD_CUDA(cudaMemcpyAsync(out, dst, (size_t)Q * ld * 4, cudaMemcpyDeviceToHost, st));
   RBOD_CUDA(cudaStreamSynchronize(st));
   return RBOD_OK;

@@ -73,7 +73,9 @@ struct K3Launch {
   int list_cap;           // prune trigger: 64 (kc <= 32), 128 (kc <= 64) or 256
   int list_stride;        // list_cap + K3_TILE_N
   int final_cap;          // lists longer than this get a last exact prune to kc entries
-  const uint32_t* row_mask;
+  const uint32_t* row_mask;       // [n_masks][mask_words] row bitmasks, or nullptr
+  const int* mask_of_query;       // [q_pad] mask id per query row (-1 = no mask), or nullptr = all rows read mask 0
+  int64_t mask_words;
   const float* row_bias;  // EUCLID collections: [capacity rounded up to whole tiles] -|g|^2 / 2 per stored row
   uint32_t* tau_shared;   // [q_pad] ordered-key thresholds shared across slices, preset to key(-inf); or nullptr
   const float* collect_thr;   // collect mode (second pass for uncertified queries), see k3_cosine_topk.cu
@@ -165,7 +167,7 @@ enum { FIN_FULL = 0, FIN_SELECT = 1, FIN_RESUME = 2 };
 int launch_finish(const FinishArgs& A, int64_t Q, cudaStream_t st);
 int launch_global_cut(const float* gathered, int G, int64_t Q, int m, int k, float* out_cut2, cudaStream_t st);
 int launch_gather_flagged(const uint16_t* q16, int dp, const int* flag_q, int f0, int nf, int64_t nf_pad,
-                          uint16_t* fq16, int* coll_cnt, cudaStream_t st);
+                          uint16_t* fq16, int* coll_cnt, const int* mask_of_query, int* fmask, cudaStream_t st);
 int launch_rescore_collected(const float* q, const double* q_qq, const float* master32, const uint16_t* rows16,
                              int kind16, int dim, int64_t ld32, int64_t ld16, int metric, const int* flag_q, int f0,
                              int nf, int cap, const uint32_t* coll_idx, const int* coll_cnt, double* coll_score,
@@ -178,9 +180,9 @@ int launch_dist_widen_queries(const float* q, const int* qsel, int nf, int dim, 
                               cudaStream_t st);
 int launch_dist_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
                         int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride,
-                        const uint32_t* row_mask, const double* thr, const uint32_t* thr_row, const int* active,
-                        const double* qnorm, int nf, int cap, double* coll_key, uint32_t* coll_idx, int* coll_cnt,
-                        int num_sms, cudaStream_t st);
+                        const uint32_t* row_mask, int64_t mask_words, const int* slot_mask, const double* thr,
+                        const uint32_t* thr_row, const int* active, const double* qnorm, int nf, int cap,
+                        double* coll_key, uint32_t* coll_idx, int* coll_cnt, int num_sms, cudaStream_t st);
 int launch_dist_select(const double* coll_key, const uint32_t* coll_idx, int* coll_cnt, const int* qsel, int nf,
                        int cap, int k, int sample, int metric, double* thr, uint32_t* thr_row, int* active,
                        int* n_active, float* out_scores, int64_t* out_rows, double* out_keys, cudaStream_t st);
@@ -230,6 +232,7 @@ struct rbod_gallery {
   rbod::DevBuf flag_q, flag_thr, flag_lo, fq16, groupmax, tau_init;
   rbod::DevBuf coll_score, coll_idx, coll_cnt;
   rbod::DevBuf mask_dev, dump, sync_counters, prof;
+  rbod::DevBuf mask_ids, fmask_ids;   // per-query mask ids: [q_pad] of the main pass, [q_pad] of the collecting pass
   rbod::DevBuf sel_keys, sel_n, sel_tau;       // split search: the selection rbod_search_begin leaves for rbod_search_end
   struct {                                     // what rbod_search_end needs to know about the pending rbod_search_begin
     int64_t Q = 0;
@@ -240,6 +243,6 @@ struct rbod_gallery {
   } pending;
   rbod::DevBuf seg_idx, seg_off, seg_out, seg_partials, seg_prefix, seg_arrive, seg_scratch, seg_member;
   rbod::DevBuf gather_idx, gather_out;
-  rbod::DevBuf dist_q64, dist_thr, dist_ctl;   // K5: widened query batch, thresholds, {qsel, active, n_active}
+  rbod::DevBuf dist_q64, dist_thr, dist_ctl;   // K5: widened query batch, thresholds, {qsel, active, n_active, slot mask}
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };

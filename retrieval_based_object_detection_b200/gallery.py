@@ -181,9 +181,14 @@ class Gallery:
         return out, mem
 
     # -- K3 ---------------------------------------------------------------------------------
-    def search(self, queries, k: int, row_mask=None, want_scores64: bool = False, out=None, stream=None) -> SearchResult:
+    def search(self, queries, k: int, row_mask=None, want_scores64: bool = False, out=None, stream=None,
+               mask_of_query=None) -> SearchResult:
         """Exact top-k of ``queries`` [Q, dim] against the stored rows under the collection's distance (cosine by
-        default; ``scores64`` carries the ordering key -d^2 / -d for euclid / manhattan collections)."""
+        default; ``scores64`` carries the ordering key -d^2 / -d for euclid / manhattan collections).
+
+        ``row_mask``: uint32 row bitmask (bit r % 32 of word r // 32 = row r allowed) shared by every query.  With
+        ``mask_of_query`` [Q] int32 (the mask each query uses, -1 = no filter), ``row_mask`` is [M, words] instead:
+        one mask per distinct filter, all answered in one pass (rbod_search_masks)."""
         keep, p_q = self._in(queries, np.float32, "float32")
         if keep.ndim == 1:
             keep = keep.reshape(1, -1)
@@ -191,6 +196,17 @@ class Gallery:
             raise ValueError(f"search: expected [Q, {self.dim}] queries, got {tuple(keep.shape)}")
         Q = int(keep.shape[0])
         k_mask, p_mask = self._in(row_mask, np.uint32, "int32")
+        k_ids, p_ids = self._in(mask_of_query, np.int32, "int32")
+        n_masks = 0
+        if k_ids is not None:
+            if tuple(k_ids.shape) != (Q,):
+                raise ValueError(f"search: mask_of_query must hold one mask id per query ({Q}), got {tuple(k_ids.shape)}")
+            if k_mask is not None:
+                words = (len(self) + 31) // 32
+                if k_mask.ndim != 2 or k_mask.shape[1] != words:
+                    raise ValueError(f"search: with mask_of_query, row_mask must be [M, {words}] words, "
+                                     f"got {tuple(k_mask.shape)}")
+                n_masks = int(k_mask.shape[0])
         if out is not None:
             scores, rows = out[0], out[1]
             s64 = out[2] if len(out) > 2 else None
@@ -202,8 +218,12 @@ class Gallery:
             rows, p_r = self._alloc_like(keep, (Q, k), np.int64, "int64")
             s64, p_64 = (self._alloc_like(keep, (Q, k), np.float64, "float64") if want_scores64 else (None, None))
         st = N.SearchStats()
-        N.check(self._lib.rbod_search(self._h, p_q, Q, int(k), p_mask, p_s, p_r, p_64, ctypes.byref(st),
-                                      stream if stream is not None else _current_stream()))
+        stream = stream if stream is not None else _current_stream()
+        if k_ids is not None:
+            N.check(self._lib.rbod_search_masks(self._h, p_q, Q, int(k), p_mask, n_masks, p_ids, p_s, p_r, p_64,
+                                                ctypes.byref(st), stream))
+        else:
+            N.check(self._lib.rbod_search(self._h, p_q, Q, int(k), p_mask, p_s, p_r, p_64, ctypes.byref(st), stream))
         stats = {f: getattr(st, f) for f, _ in st._fields_}
         return SearchResult(scores, rows, s64, stats)
 

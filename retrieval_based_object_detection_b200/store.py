@@ -649,11 +649,31 @@ class Collection:
         bits[:n] = allowed
         return np.packbits(bits, bitorder="little").view(np.uint32).copy()
 
-    def search(self, queries: np.ndarray, k: int, flt=None):
-        """-> (scores [Q,k] float32, slots [Q,k] int64) via the device (K3 + exact rescoring)."""
+    def search(self, queries: np.ndarray, k: int, flt=None, filters=None):
+        """-> (scores [Q,k] float32, slots [Q,k] int64) via the device (K3 + exact rescoring).  ``flt`` filters every
+        query; ``filters`` is one filter (or None) per query instead, all answered in one device search."""
         self.flush()
-        mask = self.filter_mask(flt)
-        res = self.gallery.search(np.ascontiguousarray(queries, dtype=np.float32), k, row_mask=mask)
+        q = np.ascontiguousarray(queries, dtype=np.float32)
+        if filters is not None:
+            if flt is not None:
+                raise ValueError("search: pass one filter for all queries or one per query, not both")
+            filters = list(filters)
+            if len(filters) != len(q):
+                raise ValueError(f"search: {len(filters)} filters for {len(q)} queries")
+            # equal filters compile to one mask; models are not hashable, their repr is deterministic
+            masks, mask_id = [], {}
+            ids = np.full(len(filters), -1, dtype=np.int32)
+            for i, f in enumerate(filters):
+                if f is not None:
+                    key = repr(f)
+                    if key not in mask_id:
+                        mask_id[key] = len(masks)
+                        masks.append(self.filter_mask(f))
+                    ids[i] = mask_id[key]
+            if masks:
+                res = self.gallery.search(q, k, row_mask=np.stack(masks), mask_of_query=ids)
+                return res.scores, res.rows
+        res = self.gallery.search(q, k, row_mask=self.filter_mask(flt))
         return res.scores, res.rows
 
 
