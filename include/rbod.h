@@ -145,7 +145,9 @@ int rbod_set_option(rbod_gallery* g, const char* key, int64_t value);
  * row_slots: [n] int64 destination slots (host or device; a device array is read back for validation), or NULL to
  *            append.
  *            A slot equal to the current count appends; smaller overwrites (upsert-by-id
- *            is resolved to a slot by the caller).
+ *            is resolved to a slot by the caller).  Slots must be distinct (a repeated slot is
+ *            RBOD_E_INVAL) and the new slots must fill [count, max slot] without holes
+ *            (RBOD_E_RANGE); a call refused for its slots changes nothing.
  * out_norms: optional [n] fp32 L2 norms of the incoming rows (host or device), or NULL.   */
 int rbod_upsert(rbod_gallery* g, const float* rows, int64_t n, const int64_t* row_slots, float* out_norms,
                 int32_t flags, void* stream);

@@ -422,11 +422,25 @@ int rbod_upsert(rbod_gallery* g, const float* rows, int64_t n, const int64_t* ro
 
   int64_t new_rows = g->rows + n;
   if (row_slots) {
-    int64_t mx = -1, fresh = 0;
+    int64_t mn = INT64_MAX, mx = -1, fresh = 0;
     for (int64_t i = 0; i < n; ++i) {
       if (row_slots[i] < 0) return set_error(RBOD_E_RANGE, "rbod_upsert: negative slot at %lld", (long long)i);
-      if (row_slots[i] >= g->rows) ++fresh;
+      mn = std::min(mn, row_slots[i]);
       mx = std::max(mx, row_slots[i]);
+    }
+    if (mx - g->rows >= n)   // a hole whatever the slots are; also bounds the bitmap below
+      return set_error(RBOD_E_RANGE, "rbod_upsert: slots would leave holes (max slot %lld, rows %lld)",
+                       (long long)mx, (long long)g->rows);
+    // Slots must be distinct: two K1 warps would write a repeated slot in no defined order (master, 16-bit row and
+    // bias each from either input, stats from both), and counted twice below it would hide a hole.  One bit per slot
+    // of [mn, mx], no sort: a bulk overwrite may carry millions of slots, a delete's move carries one.
+    std::vector<uint64_t> seen((size_t)((mx - mn) / 64 + 1), 0);
+    for (int64_t i = 0; i < n; ++i) {
+      const uint64_t off = (uint64_t)(row_slots[i] - mn), bit = 1ull << (off % 64);
+      if (seen[off / 64] & bit)
+        return set_error(RBOD_E_INVAL, "rbod_upsert: slot %lld appears more than once", (long long)row_slots[i]);
+      seen[off / 64] |= bit;
+      if (row_slots[i] >= g->rows) ++fresh;
     }
     new_rows = std::max(g->rows, mx + 1);
     if (mx + 1 > g->rows + fresh)

@@ -45,6 +45,13 @@ class FakeGallery:
         if slots is None:
             slots = np.arange(len(self._rows), len(self._rows) + len(rows))
         slots = np.asarray(slots, dtype=np.int64)
+        # refused like rbod_upsert does: repeated slots, negative slots, slots that leave holes
+        if len(np.unique(slots)) != len(slots):
+            raise RuntimeError("rbod_upsert: slot appears more than once")
+        if len(slots) and slots.min() < 0:
+            raise RuntimeError("rbod_upsert: negative slot")
+        if len(slots) and slots.max() + 1 > len(self._rows) + int((slots >= len(self._rows)).sum()):
+            raise RuntimeError("rbod_upsert: slots would leave holes")
         new_n = max(len(self._rows), int(slots.max()) + 1 if len(slots) else 0)
         if new_n > len(self._rows):
             grown = np.zeros((new_n, self.dim), dtype=np.float32)

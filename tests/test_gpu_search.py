@@ -25,21 +25,34 @@ def _mk(G, n, dim, dtype, seed, clustered=False):
     return g, g.get_rows(np.arange(n)), x
 
 
+RAW_SHAPES = [("bf16", 1000, 768, 130), ("f16", 200, 512, 5), ("f32", 513, 512, 128), ("bf16", 300, 64, 7),
+              ("bf16", 4097, 320, 260)]
+# the COSINE cases keep the ids they had before the metric became a parameter
+RAW_CASES = [pytest.param(metric, *shape, id="-".join(map(str, shape)) + ("" if metric == "cosine" else "-" + metric))
+             for metric in ("cosine", "dot", "euclid") for shape in RAW_SHAPES]
+
+
 @pytest.mark.parametrize("variant", [0, 1, 2])
-@pytest.mark.parametrize("dtype,n,dim,Q", [("bf16", 1000, 768, 130), ("f16", 200, 512, 5), ("f32", 513, 512, 128),
-                                           ("bf16", 300, 64, 7), ("bf16", 4097, 320, 260)])
-def test_raw_tensor_core_scores(G, variant, dtype, n, dim, Q):
-    """The tcgen05 pass itself: q16 . g16 with fp32 accumulation, every (query, row) cell."""
-    g, stored, _ = _mk(G, n, dim, dtype, seed=n)
-    g.set_option("k3_variant", variant)
+@pytest.mark.parametrize("metric,dtype,n,dim,Q", RAW_CASES)
+def test_raw_tensor_core_scores(G, metric, variant, dtype, n, dim, Q):
+    """The tcgen05 pass itself: q16 . g16 with fp32 accumulation, every (query, row) cell.  COSINE multiplies the unit
+    query, DOT and EUCLID the query as given (rows and queries of different norms here), and EUCLID adds the row bias
+    fp32(-|g|^2 / 2); fp32 galleries search an fp16 operand (COSINE) or a bf16 one (DOT, EUCLID)."""
+    from test_gpu_gallery_lifecycle import raw_scores_reference
+
+    x = O.synthetic_unit_rows(n, dim, seed=n)
     q = O.synthetic_unit_rows(Q, dim, seed=99)
+    if metric != "cosine":
+        x = x * np.linspace(0.25, 2.0, n, dtype=np.float32)[:, None]
+        q = q * np.linspace(0.5, 1.5, Q, dtype=np.float32)[:, None]
+    g = G(dim, dtype=dtype, metric=metric, capacity=n)
+    g.upsert(x)
+    stored = g.get_rows(np.arange(n))
+    g.set_option("k3_variant", variant)
     got = g.debug_scores(q)
-    kind = "bf16" if dtype == "bf16" else "f16"        # fp32 galleries search an fp16 shadow
-    qn = O.l2_normalize_store(q, kind)[0].astype(np.float64)
-    g16 = O.round_store(stored, kind).astype(np.float64)
-    want = qn @ g16.T
+    want, tol = raw_scores_reference(metric, dtype, q, stored)
     assert got.shape == (Q, n) and not np.isnan(got).any()
-    assert np.abs(got - want).max() < 2e-5, np.abs(got - want).max()
+    assert (np.abs(got - want) <= tol).all(), np.abs(got - want).max()
     g.close()
 
 
