@@ -31,6 +31,11 @@
  *   rbod_search_masks                              (the same kernels, one row mask per query)
  *       client.search_batch(requests=[SearchRequest(vector, filter, limit, ...)]), one payload filter per
  *       request (filters as at 32_create_delegate_vector.py:125-129, 33_run_all_experiments.py:98-103,117-137).
+ *   rbod_recommend                                 (kernel K6 recommend, exact fp64 sweep)
+ *       client.recommend(positive=[...], negative=[...], strategy=RecommendStrategy.BEST_SCORE), recommend_batch and
+ *       query_points(query=RecommendQuery(...)): "stored objects like these examples and unlike those" (refining a
+ *       class from a few labelled crops, mining hard negatives).  The average_vector strategy needs no entry point of
+ *       its own: it is one rbod_search of the composed vector.
  *   rbod_merge_topk                                (kernel K4 topk_merge)
  *       no reference call site; merges per-GPU top-k lists after the NCCL all-gather.
  *
@@ -228,6 +233,38 @@ int rbod_search_masks(rbod_gallery* g, const float* queries, int64_t Q, int32_t 
                       const uint32_t* row_masks, int32_t n_masks, const int32_t* mask_of_query,
                       float* out_scores, int64_t* out_rows, double* out_scores64,
                       rbod_search_stats* stats, void* stream);
+
+/* --- K6: recommendation, best_score strategy ---------------------------------------------
+ * A request is a set of 1 to 32 examples, each positive ("like this") or negative ("unlike this").  For an example e and
+ * a stored row g the key is rbod_search's exact fp64 ordering key, computed from the fp32 example and the stored row:
+ *   COSINE dot / (|e| |g|),  DOT dot,  EUCLID -sum (e - g)^2,  MANHATTAN -sum |e - g|.
+ * bp = the largest key over the request's positives, bn = over its negatives (-inf where there are none), and
+ *   sim(x) = x (COSINE, DOT, MANHATTAN) or -sqrt(-x) (EUCLID),   s(y) = 0.5 * (y / (1 + |y|) + 1),
+ *   score  = s(sim(bp)) if bp > bn, else -s(sim(bn))
+ * (the best_score rule of Qdrant >= 1.7, merge_similarities / scaled_fast_sigmoid; not checked against a live Qdrant).
+ * The score is larger-is-better for every metric: rows come ordered by (score desc, row slot asc).
+ * examples:        [n_examples, dim] fp32, host or device.  Example points given by id are passed as their stored rows
+ *                  (rbod_get_rows); leaving those rows out of a request's answer is the caller's business.
+ * example_sign:    [n_examples] int8, +1 (positive) or -1 (negative), host.
+ * request_offsets: [R + 1] int64, host: request r owns examples [request_offsets[r], request_offsets[r + 1]); they run
+ *                  from 0 to n_examples and every request has 1 to 32 examples.
+ * row_masks / n_masks / mask_of_request: as rbod_search_masks's row_masks / n_masks / mask_of_query, one id per request
+ *                  (-1 = no filter; NULL = every request reads mask 0, or no mask when n_masks == 0).
+ * out_scores:      [R, k] fp32 (float)score; -inf where fewer than k rows are allowed.
+ * out_rows:        [R, k] int64 row slots; -1 where fewer than k rows are allowed.
+ * out_keys:        optional [R, k] fp64 score (-inf padded), or NULL.  Outputs host or device.
+ * stats:           optional: queries = sweep_queries = R, total_launches, fallback_queries = re-sweeps of requests
+ *                  whose list of rows at or above the threshold overflowed.
+ * RBOD_E_INVAL (checked on the host before anything is launched, a device mask_of_request after reading it back): a
+ * request without examples or with more than 32, a sign other than +1 / -1, offsets that are not monotone or do not
+ * run from 0 to n_examples, a mask id outside [-1, n_masks), n_masks < 0, n_masks > 0 with row_masks == NULL, k < 1.
+ * k > 1024 is RBOD_E_UNSUPPORTED.  R = 0 and an empty collection return RBOD_OK (the latter with padding).  More than
+ * 8192 rows tied with a request's k-th score is RBOD_E_OVERFLOW, as for rbod_search.
+ * Result: row r is identical, bit for bit, whether request r is sent alone or with others.                  */
+int rbod_recommend(rbod_gallery* g, const float* examples, int64_t n_examples, const int8_t* example_sign,
+                   const int64_t* request_offsets, int64_t R, int32_t k, const uint32_t* row_masks, int32_t n_masks,
+                   const int32_t* mask_of_request, float* out_scores, int64_t* out_rows, double* out_keys,
+                   rbod_search_stats* stats, void* stream);
 
 /* --- K4: merge of per-shard top-k lists -------------------------------------------------
  * scores64 / ids: [G, Q, k] as produced by an all-gather of each rank's rbod_search output

@@ -9,7 +9,7 @@ is a call through the C ABI in include/rbod.h.  There is no CPU implementation o
 operations: without the built extension and a B200 they raise.
 
 Method subset = what the four scripts call (SURVEY.md §8(b)) + ``search`` / ``query_points`` /
-``search_batch`` as BASELINE.json's north star specifies.  Configuration is by environment only,
+``search_batch`` as BASELINE.json's north star specifies, + ``recommend`` / ``recommend_batch``.  Configuration is by environment only,
 because the scripts take no flags: ``RBOD_STORE_DIR``, ``RBOD_GALLERY_DTYPE`` (f32 | bf16 | f16),
 ``RBOD_DEVICE`` (CUDA ordinal).
 """
@@ -25,8 +25,9 @@ from retrieval_based_object_detection_b200.store import Collection, CollectionNo
 
 from . import models
 from .models import (Batch, CollectionConfig, CollectionDescription, CollectionInfo, CollectionParams,
-                     CollectionsResponse, CountResult, Distance, PointStruct, QueryResponse, Record, ScoredPoint,
-                     UpdateResult, UpdateStatus, VectorParams)
+                     CollectionsResponse, CountResult, Distance, PointStruct, QueryResponse, RecommendQuery,
+                     RecommendRequest, RecommendStrategy, Record, ScoredPoint, UpdateResult, UpdateStatus,
+                     VectorParams)
 
 __all__ = ["QdrantClient", "models", "CollectionNotFound"]
 __version__ = "1.9.0+rbod"
@@ -206,9 +207,11 @@ class QdrantClient:
         return self._records(col, slots, bool(with_payload), bool(with_vectors))
 
     # ------------------------------------------------------------------ search
-    def _scored(self, col: Collection, scores, slots, with_payload, with_vectors, score_threshold) -> List[ScoredPoint]:
+    def _scored(self, col: Collection, scores, slots, with_payload, with_vectors, score_threshold,
+                is_distance: Optional[bool] = None) -> List[ScoredPoint]:
         # EUCLID / MANHATTAN scores are distances (ascending, smaller = closer): the threshold is an upper bound
-        is_distance = col.distance in ("Euclid", "Manhattan")
+        if is_distance is None:
+            is_distance = col.distance in ("Euclid", "Manhattan")
         keep = [(float(sc), int(s)) for sc, s in zip(scores, slots)
                 if s >= 0 and (score_threshold is None
                                or (sc <= score_threshold if is_distance else sc >= score_threshold))]
@@ -234,6 +237,11 @@ class QdrantClient:
     def query_points(self, collection_name: str, query=None, query_filter=None, limit: int = 10, offset: int = 0,
                      with_payload=True, with_vectors=False, score_threshold: Optional[float] = None,
                      **_ignored: Any) -> QueryResponse:
+        if isinstance(query, RecommendQuery):
+            rec = query.recommend
+            return QueryResponse(points=self.recommend(
+                collection_name, rec.positive, rec.negative, query_filter, limit, offset, with_payload, with_vectors,
+                score_threshold, _ignored.get("using"), _ignored.get("lookup_from"), rec.strategy))
         return QueryResponse(points=self.search(collection_name, query, query_filter, limit, offset, with_payload,
                                                 with_vectors, score_threshold))
 
@@ -274,6 +282,55 @@ class QdrantClient:
         id_of = np.asarray(col.ids + [None], dtype=object)          # slot -1 -> None through the last entry
         ids = id_of[np.asarray(slots)].tolist()
         return scores, ids
+
+    # ------------------------------------------------------------------ recommendation (K6)
+    def recommend(self, collection_name: str, positive=None, negative=None, query_filter=None, limit: int = 10,
+                  offset: int = 0, with_payload=True, with_vectors=False, score_threshold: Optional[float] = None,
+                  using=None, lookup_from=None, strategy=None, **_ignored: Any) -> List[ScoredPoint]:
+        """Stored points like the ``positive`` examples and unlike the ``negative`` ones; each example is a point id
+        (its stored vector) or a raw vector, 1 to 32 per request, and example points never appear in the answer.
+
+        ``strategy`` (``RecommendStrategy`` or its string):
+        * "average_vector" (default): a search of mean(positive), or 2 mean(positive) - mean(negative) when there are
+          negatives, composed in float64 and rounded to float32 once.  Scores are the collection's search scores
+          (distances for Euclid / Manhattan, where ``score_threshold`` is an upper bound).
+        * "best_score": per stored row, bp / bn = its best search key against a positive / negative example, and the
+          score is s(sim(bp)) if bp > bn, else -s(sim(bn)), with sim = identity (minus the L2 distance for Euclid) and
+          s(y) = 0.5 (y / (1 + |y|) + 1).  This is the rule of Qdrant >= 1.7 as read from its source; it has not been
+          checked against a live Qdrant.  Scores are larger-is-better for every distance: ``score_threshold`` keeps
+          scores >= it.  Answered exactly by an fp64 sweep of the collection on the GPU.
+
+        ``using`` (named vectors) and ``lookup_from`` (another collection) are not supported: ValueError."""
+        req = RecommendRequest(positive=positive, negative=negative, filter=query_filter, limit=limit, offset=offset,
+                               with_payload=with_payload, with_vector=with_vectors, score_threshold=score_threshold,
+                               using=using, lookup_from=lookup_from, strategy=strategy)
+        return self.recommend_batch(collection_name, [req])[0]
+
+    def recommend_batch(self, collection_name: str, requests, **_ignored: Any) -> List[List[ScoredPoint]]:
+        """One ``recommend`` per ``RecommendRequest``, answered with one device call per strategy and distinct
+        limit + offset + example ids; the output equals the per-request loop."""
+        col = self._root.get(collection_name)
+        requests = list(requests)
+        by_strategy: Dict[str, List[int]] = {}
+        for i, r in enumerate(requests):
+            if r.using is not None:
+                raise ValueError("recommend: named vectors (using=) are not supported by this drop-in")
+            if r.lookup_from is not None:
+                raise ValueError("recommend: lookup_from (examples from another collection) is not supported")
+            s = r.strategy.value if isinstance(r.strategy, RecommendStrategy) else (r.strategy or "average_vector")
+            if s not in ("average_vector", "best_score"):
+                raise ValueError(f"unknown recommend strategy {r.strategy!r}")
+            by_strategy.setdefault(s, []).append(i)
+        out: List[List[ScoredPoint]] = [[] for _ in requests]
+        for s, members in by_strategy.items():
+            res = col.recommend([(requests[i].positive, requests[i].negative, requests[i].filter,
+                                  int(requests[i].limit) + int(requests[i].offset or 0)) for i in members], s)
+            is_distance = s == "average_vector" and col.distance in ("Euclid", "Manhattan")
+            for (scores, slots), i in zip(res, members):
+                r = requests[i]
+                out[i] = self._scored(col, scores, slots, bool(r.with_payload), bool(r.with_vector), r.score_threshold,
+                                      is_distance)[int(r.offset or 0):]
+        return out
 
     # ------------------------------------------------------------------ delegates (K2)
     def build_delegates(self, collection_name: str, group_key: str = "class_name", scroll_filter=None,

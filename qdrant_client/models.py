@@ -127,6 +127,30 @@ class SearchRequest(_Model):
     _defaults = {"filter": None, "with_payload": None, "with_vector": None, "score_threshold": None, "offset": 0}
 
 
+class RecommendStrategy(str, enum.Enum):
+    """average_vector (the default): one search of the composed vector; best_score: per row, the best positive against
+    the best negative example (exact fp64 sweep on the device)."""
+    AVERAGE_VECTOR = "average_vector"
+    BEST_SCORE = "best_score"
+
+
+class RecommendRequest(_Model):
+    _fields = ("positive", "negative", "filter", "params", "limit", "offset", "with_payload", "with_vector",
+               "score_threshold", "using", "lookup_from", "strategy", "shard_key")
+    _defaults = {"positive": None, "negative": None, "filter": None, "params": None, "offset": 0, "with_payload": None,
+                 "with_vector": None, "score_threshold": None, "using": None, "lookup_from": None, "strategy": None,
+                 "shard_key": None}
+
+
+class RecommendInput(_Model):
+    _fields = ("positive", "negative", "strategy")
+    _defaults = {"positive": None, "negative": None, "strategy": None}
+
+
+class RecommendQuery(_Model):
+    _fields = ("recommend",)
+
+
 class PointIdsList(_Model):
     _fields = ("points",)
 

@@ -942,6 +942,91 @@ static int sweep_exact(rbod_gallery* g, const float* q_dev, int64_t n, const int
   return RBOD_OK;
 }
 
+// Exact best_score recommendation (kernel K6), the same loop as sweep_exact over requests instead of queries: requests
+// are packed whole, in order, into passes of at most 32 example slots and 32 requests.  Per pass a strided sample pass
+// gives every request its starting threshold, then the gallery is swept, and the requests whose list overflowed are
+// tightened and swept again.  Request r's answer goes to rows r * k of the outputs.  Nothing a request's answer depends
+// on (its slots' accumulators, its threshold, its list, its mask) is shared with another request of the pass, so the
+// packing does not change any answer.  ex_dev: [E, dim] fp32 examples on the device; sign / off / mask_of_req: host.
+static int reco_sweep(rbod_gallery* g, const float* ex_dev, const int8_t* sign, const int64_t* off, int64_t R, int k,
+                      const SearchMasks& M, const int* mask_of_req, float* d_scores, int64_t* d_rows, double* d_keys,
+                      int64_t* launches, int64_t* resweeps, cudaStream_t st) {
+  const int cap = 8192, sample_cap = 8192, batch = 32, max_iter = 12;
+  RBOD_TRY(g->dist_q64.ensure((size_t)batch * g->dim * 8));
+  RBOD_TRY(g->dist_thr.ensure((size_t)2 * batch * 8 + (size_t)batch * 4));   // thresholds, example norms, row bounds
+  RBOD_TRY(g->dist_ctl.ensure((size_t)(5 * batch + 1) * 4));
+  RBOD_TRY(g->coll_score.ensure((size_t)batch * cap * 8));
+  RBOD_TRY(g->coll_idx.ensure((size_t)batch * cap * 4));
+  RBOD_TRY(g->coll_cnt.ensure((size_t)batch * 4));
+  int* d_wsel = g->dist_ctl.as<int>();   // slot -> example (what the widening reads)
+  int* d_slot = d_wsel + batch;           // slot table of the pass (k6_recommend.cu)
+  int* d_req = d_wsel + 2 * batch;        // request of the pass -> request of the call (the output row)
+  int* d_active = d_wsel + 3 * batch;
+  int* d_rmask = d_wsel + 4 * batch;      // the mask each request of the pass reads, -1 = none
+  int* d_nactive = d_wsel + 5 * batch;
+  double* d_thr = g->dist_thr.as<double>();
+  double* d_qnorm = d_thr + batch;
+  uint32_t* d_thr_row = reinterpret_cast<uint32_t*>(d_qnorm + batch);
+  const std::vector<double> h_thr(batch, -INFINITY);
+  std::vector<int> h_ctl(5 * batch + 1);
+  const int64_t sample_stride = (g->rows + sample_cap - 1) / sample_cap;   // > 1 iff more than `sample_cap` rows
+  for (int64_t r0 = 0; r0 < R;) {
+    int nreq = 0, ns = 0;
+    while (r0 + nreq < R && nreq < batch && ns + (off[r0 + nreq + 1] - off[r0 + nreq]) <= batch) {
+      ns += (int)(off[r0 + nreq + 1] - off[r0 + nreq]);
+      ++nreq;
+    }
+    std::fill(h_ctl.begin(), h_ctl.end(), 0);
+    for (int s = 0; s < batch; ++s) h_ctl[s] = (int)(off[r0] + std::min(s, ns - 1));
+    for (int q = 0; q < nreq; ++q) {
+      const int64_t e0 = off[r0 + q], e1 = off[r0 + q + 1];
+      for (int64_t e = e0; e < e1; ++e)
+        h_ctl[batch + (int)(e - off[r0])] = q | (e == e1 - 1 ? 32 : 0) | (sign[e] < 0 ? 64 : 0);
+      h_ctl[2 * batch + q] = (int)(r0 + q);
+      h_ctl[3 * batch + q] = 1;
+      h_ctl[4 * batch + q] = (M.dev != nullptr && mask_of_req != nullptr) ? mask_of_req[r0 + q] : -1;
+    }
+    RBOD_CUDA(cudaMemcpyAsync(d_wsel, h_ctl.data(), h_ctl.size() * 4, cudaMemcpyHostToDevice, st));
+    RBOD_CUDA(cudaMemcpyAsync(d_thr, h_thr.data(), (size_t)batch * 8, cudaMemcpyHostToDevice, st));
+    RBOD_CUDA(cudaMemsetAsync(d_thr_row, 0xff, (size_t)batch * 4, st));
+    RBOD_CUDA(cudaMemsetAsync(g->coll_cnt.p, 0, (size_t)batch * 4, st));
+    if (ns < batch) RBOD_CUDA(cudaMemsetAsync(g->dist_q64.p, 0, (size_t)batch * g->dim * 8, st));
+    RBOD_TRY(launch_dist_widen_queries(ex_dev, d_wsel, ns, g->dim, g->dist_q64.as<double>(), d_qnorm, st));
+    ++*launches;
+    // the K5 selection ranks by the key it is given; metric COSINE emits that key as the score and pads with -inf,
+    // which is what K (larger is better for every metric) needs
+    if (sample_stride > 1) {
+      RBOD_TRY(launch_reco_collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim,
+                                   g->dim, g->dp, g->rows, 0, sample_stride, M.dev, M.words, d_slot, d_rmask, d_thr,
+                                   d_thr_row, d_active, d_qnorm, ns, nreq, cap, g->coll_score.as<double>(),
+                                   g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(), g->num_sms, st));
+      RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
+                                  d_req, nreq, cap, k, 1, RBOD_COSINE, d_thr, d_thr_row, d_active, d_nactive, d_scores,
+                                  d_rows, d_keys, st));
+      *launches += 2;
+    }
+    int iter = 0, left = nreq;
+    for (; iter < max_iter && left > 0; ++iter) {
+      RBOD_CUDA(cudaMemsetAsync(d_nactive, 0, 4, st));
+      RBOD_TRY(launch_reco_collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim,
+                                   g->dim, g->dp, g->rows, 0, 1, M.dev, M.words, d_slot, d_rmask, d_thr, d_thr_row,
+                                   d_active, d_qnorm, ns, nreq, cap, g->coll_score.as<double>(),
+                                   g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(), g->num_sms, st));
+      RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
+                                  d_req, nreq, cap, k, 0, RBOD_COSINE, d_thr, d_thr_row, d_active, d_nactive, d_scores,
+                                  d_rows, d_keys, st));
+      *launches += 2;
+      RBOD_CUDA(cudaMemcpyAsync(&left, d_nactive, 4, cudaMemcpyDeviceToHost, st));
+      RBOD_CUDA(cudaStreamSynchronize(st));
+      if (iter > 0) ++*resweeps;
+    }
+    if (left > 0)
+      return set_error(RBOD_E_OVERFLOW, "rbod_recommend: more than %d rows tie around the k-th score of a request", cap);
+    r0 += nreq;
+  }
+  return RBOD_OK;
+}
+
 // bf16 COSINE collections: a bf16 query sits up to 2e-3 from the exact unit query, more than the gap between the
 // k-th and the (k + slack)-th score once k reaches the high tens (10M rows, k = 100: 17-37 % of the queries were
 // not certified and took the collecting second pass).  An fp16 copy of the stored rows as the search operand brings
@@ -1320,6 +1405,102 @@ int rbod_search_masks(rbod_gallery* g, const float* queries, int64_t Q, int32_t 
                       double* out_scores64, rbod_search_stats* stats, void* stream) {
   return search_impl(g, queries, Q, k, row_masks, n_masks, mask_of_query, out_scores, out_rows, out_scores64, stats,
                      stream);
+}
+
+int rbod_recommend(rbod_gallery* g, const float* examples, int64_t n_examples, const int8_t* example_sign,
+                   const int64_t* request_offsets, int64_t R, int32_t k, const uint32_t* row_masks, int32_t n_masks,
+                   const int32_t* mask_of_request, float* out_scores, int64_t* out_rows, double* out_keys,
+                   rbod_search_stats* stats, void* stream) {
+  // the host-side arguments are checked first, so a malformed call is refused before anything touches a device
+  if (R < 0 || R > (1ll << 24)) return set_error(RBOD_E_INVAL, "rbod_recommend: R = %lld out of range", (long long)R);
+  if (k < 1) return set_error(RBOD_E_INVAL, "rbod_recommend: k = %d < 1", k);
+  if (n_examples < 0) return set_error(RBOD_E_INVAL, "rbod_recommend: n_examples = %lld", (long long)n_examples);
+  if (n_masks < 0 || (n_masks > 0 && !row_masks))
+    return set_error(RBOD_E_INVAL, "rbod_recommend: %d masks, row_masks %s", n_masks, row_masks ? "set" : "NULL");
+  if (R > 0 && (!examples || !example_sign || !request_offsets || !out_scores || !out_rows))
+    return set_error(RBOD_E_INVAL, "rbod_recommend: NULL examples, signs, offsets or outputs");
+  if (request_offsets) {
+    if (request_offsets[0] != 0 || request_offsets[R] != n_examples)
+      return set_error(RBOD_E_INVAL, "rbod_recommend: request_offsets must run from 0 to n_examples = %lld",
+                       (long long)n_examples);
+    for (int64_t r = 0; r < R; ++r) {
+      const int64_t n = request_offsets[r + 1] - request_offsets[r];
+      if (n < 1 || n > 32)
+        return set_error(RBOD_E_INVAL, "rbod_recommend: request %lld has %lld examples, not 1 to 32 (offsets monotone)",
+                         (long long)r, (long long)n);
+    }
+  }
+  for (int64_t e = 0; e < (R > 0 ? n_examples : 0); ++e)
+    if (example_sign[e] != 1 && example_sign[e] != -1)
+      return set_error(RBOD_E_INVAL, "rbod_recommend: example_sign[%lld] = %d is not +1 or -1", (long long)e,
+                       (int)example_sign[e]);
+  const bool ids_dev = is_device_ptr(mask_of_request);
+  if (mask_of_request && !ids_dev)
+    for (int64_t r = 0; r < R; ++r)
+      if (mask_of_request[r] < -1 || mask_of_request[r] >= n_masks)
+        return set_error(RBOD_E_INVAL, "rbod_recommend: mask_of_request[%lld] = %d is outside [-1, %d)", (long long)r,
+                         mask_of_request[r], n_masks);
+  if (k > 1024) return set_error(RBOD_E_UNSUPPORTED, "rbod_recommend: k=%d > 1024", k);
+  if (!g) return set_error(RBOD_E_INVAL, "rbod_recommend: NULL handle");
+  if (stats) memset(stats, 0, sizeof(*stats));
+  if (R == 0) return RBOD_OK;
+  if (g->rows >= 0xffffffffll) return set_error(RBOD_E_UNSUPPORTED, "rbod_recommend: more than 2^32-2 rows per shard");
+  RBOD_CUDA(cudaSetDevice(g->device));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+
+  // one mask id per request: -1 without masks, mask 0 for every request when mask_of_request is NULL
+  std::vector<int> ids(n_masks > 0 ? (size_t)R : 0, 0);
+  if (n_masks > 0 && mask_of_request) {
+    if (ids_dev) {
+      RBOD_CUDA(cudaMemcpyAsync(ids.data(), mask_of_request, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
+      RBOD_CUDA(cudaStreamSynchronize(st));
+      for (int64_t r = 0; r < R; ++r)
+        if (ids[r] < -1 || ids[r] >= n_masks)
+          return set_error(RBOD_E_INVAL, "rbod_recommend: mask_of_request[%lld] = %d is outside [-1, %d)",
+                           (long long)r, ids[r], n_masks);
+    } else {
+      memcpy(ids.data(), mask_of_request, (size_t)R * 4);
+    }
+  }
+  SearchMasks M = {nullptr, (g->rows + 31) / 32, nullptr, nullptr};
+
+  const size_t n_out = (size_t)R * k;
+  RBOD_TRY(g->out_scores.ensure(n_out * 4));
+  RBOD_TRY(g->out_rows.ensure(n_out * 8));
+  RBOD_TRY(g->out_scores64.ensure(n_out * 8));
+  if (g->rows == 0) {
+    std::vector<float> hs(n_out, -INFINITY);
+    std::vector<int64_t> hr(n_out, -1);
+    std::vector<double> hd(n_out, -INFINITY);
+    RBOD_CUDA(cudaMemcpyAsync(out_scores, hs.data(), n_out * 4, cudaMemcpyDefault, st));
+    RBOD_CUDA(cudaMemcpyAsync(out_rows, hr.data(), n_out * 8, cudaMemcpyDefault, st));
+    if (out_keys) RBOD_CUDA(cudaMemcpyAsync(out_keys, hd.data(), n_out * 8, cudaMemcpyDefault, st));
+    RBOD_CUDA(cudaStreamSynchronize(st));
+    if (stats) stats->queries = R;
+    return RBOD_OK;
+  }
+  float* ds = is_device_ptr(out_scores) ? out_scores : g->out_scores.as<float>();
+  int64_t* dr = is_device_ptr(out_rows) ? out_rows : g->out_rows.as<int64_t>();
+  double* dk = (out_keys && is_device_ptr(out_keys)) ? out_keys : g->out_scores64.as<double>();
+  const void* md = nullptr;
+  if (n_masks > 0) RBOD_TRY(to_device(row_masks, (size_t)n_masks * M.words * 4, g->mask_dev, st, &md));
+  M.dev = static_cast<const uint32_t*>(md);
+  const void* xd = nullptr;
+  RBOD_TRY(to_device(examples, (size_t)n_examples * g->dim * 4, g->q32, st, &xd));
+  int64_t n_launch = 0, resweeps = 0;
+  RBOD_TRY(reco_sweep(g, static_cast<const float*>(xd), example_sign, request_offsets, R, k, M,
+                      ids.empty() ? nullptr : ids.data(), ds, dr, dk, &n_launch, &resweeps, st));
+  RBOD_TRY(copy_out(out_scores, ds, n_out * 4, st));
+  RBOD_TRY(copy_out(out_rows, dr, n_out * 8, st));
+  if (out_keys) RBOD_TRY(copy_out(out_keys, dk, n_out * 8, st));
+  RBOD_CUDA(cudaStreamSynchronize(st));
+  if (stats) {
+    stats->queries = R;
+    stats->sweep_queries = R;          // every request is answered by the fp64 sweep
+    stats->total_launches = n_launch;
+    stats->fallback_queries = resweeps;
+  }
+  return RBOD_OK;
 }
 
 // ---- split search: the two halves of rbod_search around an exchange between shards ---------------------------

@@ -186,6 +186,13 @@ int launch_dist_collect(int metric, const double* q64, const float* master32, co
 int launch_dist_select(const double* coll_key, const uint32_t* coll_idx, int* coll_cnt, const int* qsel, int nf,
                        int cap, int k, int sample, int metric, double* thr, uint32_t* thr_row, int* active,
                        int* n_active, float* out_scores, int64_t* out_rows, double* out_keys, cudaStream_t st);
+// K6: exact best_score recommendation sweep (selection through K5's widen / select launchers)
+int launch_reco_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
+                        int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride,
+                        const uint32_t* row_mask, int64_t mask_words, const int* slot_tab, const int* req_mask,
+                        const double* thr, const uint32_t* thr_row, const int* active, const double* qnorm,
+                        int n_slots, int n_req, int cap, double* coll_key, uint32_t* coll_idx, int* coll_cnt,
+                        int num_sms, cudaStream_t st);
 int launch_merge_topk(const double* scores64, const int64_t* ids, int64_t shard_stride, const int64_t* row0_host,
                       int G, int64_t Q, int k, float* out_scores, int64_t* out_ids, double* out_scores64,
                       cudaStream_t st, const double* ubound = nullptr, int* flag_q = nullptr, int* n_flag = nullptr);

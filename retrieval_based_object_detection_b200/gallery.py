@@ -227,6 +227,47 @@ class Gallery:
         stats = {f: getattr(st, f) for f, _ in st._fields_}
         return SearchResult(scores, rows, s64, stats)
 
+    # -- K6 ---------------------------------------------------------------------------------
+    def recommend(self, examples, signs, offsets, k: int, row_mask=None, mask_of_request=None,
+                  want_keys: bool = False) -> SearchResult:
+        """Exact best_score recommendation (rbod_recommend): request r is the examples ``offsets[r]:offsets[r + 1]`` of
+        ``examples`` [E, dim], each positive (``signs`` +1) or negative (-1), 1 to 32 per request.  A row's score is
+        s(sim(bp)) when its best positive key bp beats its best negative key bn, else -s(sim(bn)), with the search key
+        of the collection's metric, sim = identity (-sqrt(-key) for euclid) and s(y) = 0.5 (y / (1 + |y|) + 1): the
+        best_score rule of Qdrant >= 1.7, not checked against a live Qdrant.  Larger is better for every metric.
+
+        -> ``scores`` [R, k] float32 descending (-inf padded), ``rows`` [R, k] int64 (-1 padded), ``scores64`` the fp64
+        scores when ``want_keys``.  ``row_mask`` / ``mask_of_request`` are as ``search``'s ``row_mask`` /
+        ``mask_of_query``, one mask id per request."""
+        keep, p_x = self._in(examples, np.float32, "float32")
+        if keep.ndim != 2 or keep.shape[1] != self.dim:
+            raise ValueError(f"recommend: expected [E, {self.dim}] examples, got {tuple(keep.shape)}")
+        sg = _as_host(signs, np.int8)
+        off = _as_host(offsets, np.int64)
+        if off.ndim != 1 or len(off) < 1 or sg.shape != (int(keep.shape[0]),):
+            raise ValueError("recommend: offsets must be [R + 1] and signs [E]")
+        R = len(off) - 1
+        k_mask, p_mask = self._in(row_mask, np.uint32, "int32")
+        k_ids, p_ids = self._in(mask_of_request, np.int32, "int32")
+        n_masks = 0 if k_mask is None else 1
+        if k_ids is not None:
+            if tuple(k_ids.shape) != (R,):
+                raise ValueError(f"recommend: mask_of_request must hold one mask id per request ({R})")
+            n_masks = 0
+            if k_mask is not None:
+                words = (len(self) + 31) // 32
+                if k_mask.ndim != 2 or k_mask.shape[1] != words:
+                    raise ValueError(f"recommend: with mask_of_request, row_mask must be [M, {words}] words, "
+                                     f"got {tuple(k_mask.shape)}")
+                n_masks = int(k_mask.shape[0])
+        scores, p_s = self._alloc_like(keep, (R, k), np.float32, "float32")
+        rows, p_r = self._alloc_like(keep, (R, k), np.int64, "int64")
+        keys, p_k = (self._alloc_like(keep, (R, k), np.float64, "float64") if want_keys else (None, None))
+        st = N.SearchStats()
+        N.check(self._lib.rbod_recommend(self._h, p_x, int(keep.shape[0]), sg.ctypes.data, off.ctypes.data, R, int(k),
+                                         p_mask, n_masks, p_ids, p_s, p_r, p_k, ctypes.byref(st), _current_stream()))
+        return SearchResult(scores, rows, keys, {f: getattr(st, f) for f, _ in st._fields_})
+
     # -- split search (row-sharded collections): see include/rbod.h "Split search" ------------------------------
     def search_begin(self, queries, k: int, approx_m: int, out_approx, row_mask=None, stream=None) -> dict:
         """First half: K3 + selection; fills ``out_approx`` [Q, approx_m + 1] float32 (torch CUDA tensor) with this

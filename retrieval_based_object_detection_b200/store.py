@@ -32,6 +32,8 @@ import numpy as np
 
 FORMAT_VERSION = 1
 _FLUSH_THRESHOLD = 65536  # staged rows that force a device flush
+MAX_RECOMMEND_EXAMPLES = 32   # examples per recommendation request (rbod_recommend)
+MAX_RECOMMEND_FETCH = 1024    # rows a recommendation request fetches: limit + offset + its example ids
 
 
 class CollectionNotFound(Exception):
@@ -660,21 +662,101 @@ class Collection:
             filters = list(filters)
             if len(filters) != len(q):
                 raise ValueError(f"search: {len(filters)} filters for {len(q)} queries")
-            # equal filters compile to one mask; models are not hashable, their repr is deterministic
-            masks, mask_id = [], {}
-            ids = np.full(len(filters), -1, dtype=np.int32)
-            for i, f in enumerate(filters):
-                if f is not None:
-                    key = repr(f)
-                    if key not in mask_id:
-                        mask_id[key] = len(masks)
-                        masks.append(self.filter_mask(f))
-                    ids[i] = mask_id[key]
-            if masks:
-                res = self.gallery.search(q, k, row_mask=np.stack(masks), mask_of_query=ids)
+            masks, ids = self._filter_masks(filters)
+            if masks is not None:
+                res = self.gallery.search(q, k, row_mask=masks, mask_of_query=ids)
                 return res.scores, res.rows
         res = self.gallery.search(q, k, row_mask=self.filter_mask(flt))
         return res.scores, res.rows
+
+    def _filter_masks(self, filters):
+        """One filter (or None) per request -> (row masks [M, words], or None when every filter is None; mask id per
+        request, int32, -1 = no filter).  Equal filters compile to one mask; models are not hashable, their repr is
+        deterministic."""
+        masks, mask_id = [], {}
+        ids = np.full(len(filters), -1, dtype=np.int32)
+        for i, f in enumerate(filters):
+            if f is not None:
+                key = repr(f)
+                if key not in mask_id:
+                    mask_id[key] = len(masks)
+                    masks.append(self.filter_mask(f))
+                ids[i] = mask_id[key]
+        return (np.stack(masks) if masks else None), ids
+
+    def recommend(self, requests, strategy: str):
+        """Recommendation: ``requests`` = [(positive, negative, filter, k)], where every example is a point id or a raw
+        vector and k = limit + offset.  Examples given by id take their stored vector and never appear in that
+        request's answer.  ``strategy``:
+
+        * "average_vector": one search of mean(P), or 2 mean(P) - mean(N) when there are negatives, composed in float64
+          and rounded to float32 once; scores are the collection's ordinary search scores.  Needs a positive.
+        * "best_score": ``Gallery.recommend`` (exact fp64 sweep, kernel K6); scores are larger-is-better for every
+          metric (see include/rbod.h, rbod_recommend).
+
+        Each request fetches k + (its distinct example ids) rows, at most 1024, and has 1 to 32 examples.  Requests
+        with the same fetch share one device call.  -> [(scores float32, slots int64)] per request, at most k each,
+        example points removed."""
+        if strategy not in ("average_vector", "best_score"):
+            raise ValueError(f"unknown recommend strategy {strategy!r}")
+        self.flush()
+        plans = []
+        for pos, neg, flt, k in requests:
+            items = [(x, 1) for x in (pos or [])] + [(x, -1) for x in (neg or [])]
+            if not 1 <= len(items) <= MAX_RECOMMEND_EXAMPLES:
+                raise ValueError(f"recommend: a request needs 1 to {MAX_RECOMMEND_EXAMPLES} examples, got {len(items)}")
+            if strategy == "average_vector" and not pos:
+                raise ValueError("recommend: the average_vector strategy needs at least one positive example")
+            vecs, signs, ex_slots = [], [], set()
+            for x, sign in items:
+                if isinstance(x, (str, uuid.UUID)) or (isinstance(x, (int, np.integer)) and not isinstance(x, bool)):
+                    pid = canonical_id(x)
+                    slot = self.slot_of.get(pid)
+                    if slot is None:
+                        raise ValueError(f"recommend: point {pid!r} not found in collection {self.name!r}")
+                    ex_slots.add(slot)
+                    vecs.append(slot)
+                else:
+                    v = np.asarray(x, dtype=np.float32).reshape(-1)
+                    if v.shape[0] != self.dim:
+                        raise ValueError(f"Wrong input: Vector dimension error: expected dim: {self.dim}, got {v.shape[0]}")
+                    vecs.append(v)
+                signs.append(sign)
+            fetch = int(k) + len(ex_slots)
+            if fetch > MAX_RECOMMEND_FETCH:
+                raise ValueError(f"recommend: limit + offset + example ids = {fetch} exceeds {MAX_RECOMMEND_FETCH}")
+            plans.append((vecs, signs, ex_slots, flt, int(k), fetch))
+        id_slots = sorted({v for p in plans for v in p[0] if isinstance(v, int)})
+        stored = dict(zip(id_slots, self.stored_vectors(id_slots)))
+        out = [(np.zeros(0, np.float32), np.zeros(0, np.int64))] * len(plans)
+        by_fetch = {}
+        for i, p in enumerate(plans):
+            if p[4] >= 1:
+                by_fetch.setdefault(p[5], []).append(i)
+        for fetch, members in by_fetch.items():
+            flts = [plans[i][3] for i in members]
+            ex = [np.stack([stored[v] if isinstance(v, int) else v for v in plans[i][0]]) for i in members]
+            if strategy == "average_vector":
+                q = []
+                for i, e in zip(members, ex):
+                    sg = np.asarray(plans[i][1])
+                    e64 = e.astype(np.float64)
+                    mp = e64[sg > 0].mean(axis=0)
+                    q.append(2.0 * mp - e64[sg < 0].mean(axis=0) if (sg < 0).any() else mp)
+                scores, rows = self.search(np.stack(q).astype(np.float32), fetch, filters=flts)
+            else:
+                masks, ids = self._filter_masks(flts)
+                offsets = np.zeros(len(members) + 1, dtype=np.int64)
+                np.cumsum([len(e) for e in ex], out=offsets[1:])
+                signs = np.concatenate([np.asarray(plans[i][1], dtype=np.int8) for i in members])
+                res = self.gallery.recommend(np.concatenate(ex), signs, offsets, fetch,
+                                             row_mask=masks, mask_of_request=None if masks is None else ids)
+                scores, rows = res.scores, res.rows
+            scores, rows = np.asarray(scores), np.asarray(rows)
+            for j, i in enumerate(members):
+                keep = ~np.isin(rows[j], list(plans[i][2]))
+                out[i] = (scores[j][keep][:plans[i][4]], rows[j][keep][:plans[i][4]])
+        return out
 
 
 class StoreRoot:
