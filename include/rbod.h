@@ -36,6 +36,10 @@
  *       query_points(query=RecommendQuery(...)): "stored objects like these examples and unlike those" (refining a
  *       class from a few labelled crops, mining hard negatives).  The average_vector strategy needs no entry point of
  *       its own: it is one rbod_search of the composed vector.
+ *   rbod_discover                                  (kernel K7 discover, exact fp64 sweep)
+ *       client.discover(target=..., context=[ContextExamplePair(positive, negative), ...]), discover_batch and
+ *       query_points(query=DiscoverQuery(...) | ContextQuery(...)): "like this target, on the right side of these
+ *       corrections" (pairs such as "this crop is the class, that near-identical one is not").
  *   rbod_merge_topk                                (kernel K4 topk_merge)
  *       no reference call site; merges per-GPU top-k lists after the NCCL all-gather.
  *
@@ -265,6 +269,36 @@ int rbod_recommend(rbod_gallery* g, const float* examples, int64_t n_examples, c
                    const int64_t* request_offsets, int64_t R, int32_t k, const uint32_t* row_masks, int32_t n_masks,
                    const int32_t* mask_of_request, float* out_scores, int64_t* out_rows, double* out_keys,
                    rbod_search_stats* stats, void* stream);
+
+/* --- K7: discovery and context search ---------------------------------------------------
+ * A request is an optional target t followed by pairs (p, n) of examples ("like p, not n"): 1 to 32 examples, 0 to 15
+ * pairs with a target, 1 to 16 without.  Keys and sim are rbod_recommend's: for an example e and a stored row g the
+ * fp64 key of the fp32 example and the stored row (COSINE dot / (|e| |g|), DOT dot, EUCLID -sum (e - g)^2, MANHATTAN
+ * -sum |e - g|), sim(x) = x (-sqrt(-x) for EUCLID).  With
+ *   f(y) = y / (1 + |y|),  s(y) = 0.5 * (f(y) + 1),  MARGIN = 2^-23 (f32 epsilon),  P = key(p, g),  N = key(n, g):
+ *   rank_pair = +1 if P > N else -1 (a tie counts -1),  loss_pair = f(min(sim(P) - sim(N) - MARGIN, 0))
+ *   discovery (with a target):  score = sum of rank_pair + s(sim(key(t, g)))
+ *   context (no target):        score = sum of loss_pair, summed in pair order; 0 for every row on the positive
+ *                               side of every pair, so the top k is often a plateau of rows tied at 0
+ * (the rule of Qdrant >= 1.7, DiscoveryQuery::score_by / ContextPair::loss_by, as read from its source; not checked
+ * against a live Qdrant.  The EUCLID sim is best_score's, a choice of this library.)  The score is larger-is-better for
+ * every metric: rows come ordered by (score desc, row slot asc).  A request of a target alone scores s(sim(key(t, g))),
+ * the order of rbod_search.
+ * examples:        [n_examples, dim] fp32, host or device; example points given by id are passed as their stored rows.
+ * example_role:    [n_examples] int8, host: 0 = target (only as a request's first example), +1 = a pair's positive
+ *                  (always followed by its negative), -1 = a pair's negative (always preceded by its positive).
+ * request_offsets, row_masks, n_masks, mask_of_request, out_scores, out_rows, out_keys, stats: as rbod_recommend.
+ * RBOD_E_INVAL (checked on the host before anything is launched, a device mask_of_request after reading it back): a
+ * request without examples or with more than 32, offsets that are not monotone or do not run from 0 to n_examples, a
+ * role outside {0, +1, -1}, a target that is not its request's first example (or a second target), a +1 not followed
+ * by a -1 or a -1 not preceded by a +1, a mask id outside [-1, n_masks), n_masks < 0, n_masks > 0 with row_masks ==
+ * NULL, k < 1.  k > 1024 is RBOD_E_UNSUPPORTED.  R = 0 and an empty collection return RBOD_OK (the latter with
+ * padding).  More than 8192 rows tied with a request's k-th score after the re-sweeps is RBOD_E_OVERFLOW.
+ * Result: row r is identical, bit for bit, whether request r is sent alone or with others.                  */
+int rbod_discover(rbod_gallery* g, const float* examples, int64_t n_examples, const int8_t* example_role,
+                  const int64_t* request_offsets, int64_t R, int32_t k, const uint32_t* row_masks, int32_t n_masks,
+                  const int32_t* mask_of_request, float* out_scores, int64_t* out_rows, double* out_keys,
+                  rbod_search_stats* stats, void* stream);
 
 /* --- K4: merge of per-shard top-k lists -------------------------------------------------
  * scores64 / ids: [G, Q, k] as produced by an all-gather of each rank's rbod_search output

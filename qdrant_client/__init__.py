@@ -9,7 +9,8 @@ is a call through the C ABI in include/rbod.h.  There is no CPU implementation o
 operations: without the built extension and a B200 they raise.
 
 Method subset = what the four scripts call (SURVEY.md §8(b)) + ``search`` / ``query_points`` /
-``search_batch`` as BASELINE.json's north star specifies, + ``recommend`` / ``recommend_batch``.  Configuration is by environment only,
+``search_batch`` as BASELINE.json's north star specifies, + ``recommend`` / ``recommend_batch``, + ``discover`` /
+``discover_batch`` and ``query_points(query=DiscoverQuery | ContextQuery)``.  Configuration is by environment only,
 because the scripts take no flags: ``RBOD_STORE_DIR``, ``RBOD_GALLERY_DTYPE`` (f32 | bf16 | f16),
 ``RBOD_DEVICE`` (CUDA ordinal).
 """
@@ -25,7 +26,8 @@ from retrieval_based_object_detection_b200.store import Collection, CollectionNo
 
 from . import models
 from .models import (Batch, CollectionConfig, CollectionDescription, CollectionInfo, CollectionParams,
-                     CollectionsResponse, CountResult, Distance, PointStruct, QueryResponse, RecommendQuery,
+                     CollectionsResponse, ContextExamplePair, ContextPair, ContextQuery, CountResult,
+                     DiscoverQuery, DiscoverRequest, Distance, PointStruct, QueryResponse, RecommendQuery,
                      RecommendRequest, RecommendStrategy, Record, ScoredPoint, UpdateResult, UpdateStatus,
                      VectorParams)
 
@@ -54,6 +56,27 @@ def _distance_name(d) -> str:
         if str(d).lower() in (cand.value.lower(), cand.name.lower()):
             return cand.value
     raise ValueError(f"unknown distance {d!r}")
+
+
+def _context_pairs(context) -> list:
+    """A discovery ``context`` -> [(positive, negative)].  ``context`` is None, one pair or a list of pairs; a pair is a
+    ``ContextExamplePair``, a ``ContextPair`` or a (positive, negative) tuple (a 2-tuple whose members are neither
+    pair models nor 2-tuples)."""
+    models_ = (ContextExamplePair, ContextPair)
+
+    def is_pair(p):
+        return isinstance(p, models_) or (isinstance(p, tuple) and len(p) == 2 and not any(
+            isinstance(x, models_) or (isinstance(x, tuple) and len(x) == 2) for x in p))
+
+    if context is None:
+        return []
+    out = []
+    for p in ([context] if is_pair(context) else list(context)):
+        if not is_pair(p):
+            raise ValueError(f"discover: a context pair is a ContextExamplePair, a ContextPair or a (positive, negative) "
+                             f"tuple, got {p!r}")
+        out.append((p.positive, p.negative) if isinstance(p, models_) else p)
+    return out
 
 
 class QdrantClient:
@@ -242,6 +265,13 @@ class QdrantClient:
             return QueryResponse(points=self.recommend(
                 collection_name, rec.positive, rec.negative, query_filter, limit, offset, with_payload, with_vectors,
                 score_threshold, _ignored.get("using"), _ignored.get("lookup_from"), rec.strategy))
+        if isinstance(query, (DiscoverQuery, ContextQuery)):
+            target, context = ((query.discover.target, query.discover.context) if isinstance(query, DiscoverQuery)
+                               else (None, query.context))
+            req = DiscoverRequest(target=target, context=context, filter=query_filter, limit=limit, offset=offset,
+                                  with_payload=with_payload, with_vector=with_vectors, using=_ignored.get("using"),
+                                  lookup_from=_ignored.get("lookup_from"))
+            return QueryResponse(points=self._discover(collection_name, [req], score_threshold)[0])
         return QueryResponse(points=self.search(collection_name, query, query_filter, limit, offset, with_payload,
                                                 with_vectors, score_threshold))
 
@@ -331,6 +361,52 @@ class QdrantClient:
                 out[i] = self._scored(col, scores, slots, bool(r.with_payload), bool(r.with_vector), r.score_threshold,
                                       is_distance)[int(r.offset or 0):]
         return out
+
+    # ------------------------------------------------------------------ discovery and context search (K7)
+    def discover(self, collection_name: str, target=None, context=None, query_filter=None, search_params=None,
+                 limit: int = 10, offset: int = 0, with_payload=True, with_vectors=False, using=None,
+                 lookup_from=None, **_ignored: Any) -> List[ScoredPoint]:
+        """Stored points ranked by ``target`` within the region that ``context`` marks out.  ``context`` is a list of
+        pairs, or one pair; a pair is a ``ContextExamplePair``, a ``ContextPair`` or a (positive, negative) tuple.
+        Every example is a point id (its stored vector) or a raw vector, 1 to 32 per request (the target and two per
+        pair), and example points never appear in the answer.
+
+        With a pair's keys P / N (the collection's search key of a row against the positive / negative example), sim
+        the identity (minus the L2 distance for Euclid), f(y) = y / (1 + |y|), s(y) = 0.5 (f(y) + 1) and MARGIN =
+        2**-23, a row scores
+        * with a target (discovery): the sum over pairs of (+1 if P > N else -1), plus s(sim(key of the target));
+        * without (context search): the sum over pairs of f(min(sim(P) - sim(N) - MARGIN, 0)), which is 0 for every
+          row on the positive side of every pair; ties are ordered by point slot.
+        This is the rule of Qdrant >= 1.7 as read from its source; it has not been checked against a live Qdrant.
+        Scores are larger-is-better for every distance.  Answered exactly by an fp64 sweep of the collection on the
+        GPU.  A request with neither a target nor a context pair is a ValueError; ``using`` (named vectors) and
+        ``lookup_from`` (another collection) are not supported: ValueError."""
+        req = DiscoverRequest(target=target, context=context, filter=query_filter, params=search_params, limit=limit,
+                              offset=offset, with_payload=with_payload, with_vector=with_vectors, using=using,
+                              lookup_from=lookup_from)
+        return self.discover_batch(collection_name, [req])[0]
+
+    def discover_batch(self, collection_name: str, requests, **_ignored: Any) -> List[List[ScoredPoint]]:
+        """One ``discover`` per ``DiscoverRequest``, answered with one device call per distinct limit + offset +
+        example ids; the output equals the per-request loop."""
+        return self._discover(collection_name, list(requests), None)
+
+    def _discover(self, collection_name: str, requests, score_threshold) -> List[List[ScoredPoint]]:
+        col = self._root.get(collection_name)
+        plans = []
+        for r in requests:
+            if r.using is not None:
+                raise ValueError("discover: named vectors (using=) are not supported by this drop-in")
+            if r.lookup_from is not None:
+                raise ValueError("discover: lookup_from (examples from another collection) is not supported")
+            pairs = _context_pairs(r.context)
+            if r.target is None and not pairs:
+                raise ValueError("discover: a request needs a target or at least one context pair")
+            plans.append((r.target, pairs, r.filter, int(r.limit) + int(r.offset or 0)))
+        res = col.discover(plans)
+        return [self._scored(col, scores, slots, bool(r.with_payload), bool(r.with_vector), score_threshold,
+                             False)[int(r.offset or 0):]
+                for (scores, slots), r in zip(res, requests)]
 
     # ------------------------------------------------------------------ delegates (K2)
     def build_delegates(self, collection_name: str, group_key: str = "class_name", scroll_filter=None,

@@ -151,6 +151,37 @@ class RecommendQuery(_Model):
     _fields = ("recommend",)
 
 
+class ContextExamplePair(_Model):
+    """One correction of ``discover``: stored points should be like ``positive`` and unlike ``negative`` (each a point
+    id or a vector)."""
+    _fields = ("positive", "negative")
+
+
+class DiscoverRequest(_Model):
+    _fields = ("target", "context", "filter", "params", "limit", "offset", "with_payload", "with_vector", "using",
+               "lookup_from", "shard_key")
+    _defaults = {"target": None, "context": None, "filter": None, "params": None, "offset": 0, "with_payload": None,
+                 "with_vector": None, "using": None, "lookup_from": None, "shard_key": None}
+
+
+class ContextPair(_Model):
+    """A (positive, negative) pair of the query API (``DiscoverInput.context``, ``ContextQuery.context``)."""
+    _fields = ("positive", "negative")
+
+
+class DiscoverInput(_Model):
+    _fields = ("target", "context")
+
+
+class DiscoverQuery(_Model):
+    _fields = ("discover",)
+
+
+class ContextQuery(_Model):
+    """Context search: ``context`` is one ``ContextPair`` or a list of them."""
+    _fields = ("context",)
+
+
 class PointIdsList(_Model):
     _fields = ("points",)
 

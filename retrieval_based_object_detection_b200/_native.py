@@ -77,6 +77,8 @@ SIGNATURES = {
     "rbod_search_masks": (ctypes.c_int, [_P, _P, _I64, _I32, _P, _I32, _P, _P, _P, _P, ctypes.POINTER(SearchStats), _P]),
     "rbod_recommend": (ctypes.c_int, [_P, _P, _I64, _P, _P, _I64, _I32, _P, _I32, _P, _P, _P, _P,
                                       ctypes.POINTER(SearchStats), _P]),
+    "rbod_discover": (ctypes.c_int, [_P, _P, _I64, _P, _P, _I64, _I32, _P, _I32, _P, _P, _P, _P,
+                                     ctypes.POINTER(SearchStats), _P]),
     "rbod_merge_topk": (ctypes.c_int, [_P, _P, _I32, _I64, _I32, _P, _P, _P, _P]),
     "rbod_merge_topk_packed": (ctypes.c_int, [_P, _P, _I32, _I64, _I32, _P, _P, _P, _P]),
     "rbod_search_begin": (ctypes.c_int, [_P, _P, _I64, _I32, _I32, _P, _P, ctypes.POINTER(SearchStats), _P]),

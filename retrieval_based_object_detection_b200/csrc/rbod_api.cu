@@ -942,15 +942,18 @@ static int sweep_exact(rbod_gallery* g, const float* q_dev, int64_t n, const int
   return RBOD_OK;
 }
 
-// Exact best_score recommendation (kernel K6), the same loop as sweep_exact over requests instead of queries: requests
-// are packed whole, in order, into passes of at most 32 example slots and 32 requests.  Per pass a strided sample pass
-// gives every request its starting threshold, then the gallery is swept, and the requests whose list overflowed are
-// tightened and swept again.  Request r's answer goes to rows r * k of the outputs.  Nothing a request's answer depends
-// on (its slots' accumulators, its threshold, its list, its mask) is shared with another request of the pass, so the
-// packing does not change any answer.  ex_dev: [E, dim] fp32 examples on the device; sign / off / mask_of_req: host.
-static int reco_sweep(rbod_gallery* g, const float* ex_dev, const int8_t* sign, const int64_t* off, int64_t R, int k,
-                      const SearchMasks& M, const int* mask_of_req, float* d_scores, int64_t* d_rows, double* d_keys,
-                      int64_t* launches, int64_t* resweeps, cudaStream_t st) {
+// Exact example-based search (kernels K6 recommend, K7 discover), the same loop as sweep_exact over requests instead of
+// queries: requests are packed whole, in order, into passes of at most 32 example slots and 32 requests.  Per pass a
+// strided sample pass gives every request its starting threshold, then the gallery is swept, and the requests whose
+// list overflowed are tightened and swept again.  Request r's answer goes to rows r * k of the outputs.  Nothing a
+// request's answer depends on (its slots' accumulators, its threshold, its list, its mask) is shared with another
+// request of the pass, so the packing does not change any answer.  ex_dev: [E, dim] fp32 examples on the device;
+// flags: [E] the examples' slot-table flags (rbod_internal.h), off / mask_of_req: host.  collect: the kernel's launcher,
+// who: the entry point named in errors.
+static int example_sweep(rbod_gallery* g, CollectLauncher collect, const char* who, const float* ex_dev,
+                         const int* flags, const int64_t* off, int64_t R, int k, const SearchMasks& M,
+                         const int* mask_of_req, float* d_scores, int64_t* d_rows, double* d_keys, int64_t* launches,
+                         int64_t* resweeps, cudaStream_t st) {
   const int cap = 8192, sample_cap = 8192, batch = 32, max_iter = 12;
   RBOD_TRY(g->dist_q64.ensure((size_t)batch * g->dim * 8));
   RBOD_TRY(g->dist_thr.ensure((size_t)2 * batch * 8 + (size_t)batch * 4));   // thresholds, example norms, row bounds
@@ -959,7 +962,7 @@ static int reco_sweep(rbod_gallery* g, const float* ex_dev, const int8_t* sign, 
   RBOD_TRY(g->coll_idx.ensure((size_t)batch * cap * 4));
   RBOD_TRY(g->coll_cnt.ensure((size_t)batch * 4));
   int* d_wsel = g->dist_ctl.as<int>();   // slot -> example (what the widening reads)
-  int* d_slot = d_wsel + batch;           // slot table of the pass (k6_recommend.cu)
+  int* d_slot = d_wsel + batch;           // slot table of the pass (rbod_internal.h)
   int* d_req = d_wsel + 2 * batch;        // request of the pass -> request of the call (the output row)
   int* d_active = d_wsel + 3 * batch;
   int* d_rmask = d_wsel + 4 * batch;      // the mask each request of the pass reads, -1 = none
@@ -981,7 +984,7 @@ static int reco_sweep(rbod_gallery* g, const float* ex_dev, const int8_t* sign, 
     for (int q = 0; q < nreq; ++q) {
       const int64_t e0 = off[r0 + q], e1 = off[r0 + q + 1];
       for (int64_t e = e0; e < e1; ++e)
-        h_ctl[batch + (int)(e - off[r0])] = q | (e == e1 - 1 ? 32 : 0) | (sign[e] < 0 ? 64 : 0);
+        h_ctl[batch + (int)(e - off[r0])] = q | (e == e1 - 1 ? SLOT_LAST : 0) | flags[e];
       h_ctl[2 * batch + q] = (int)(r0 + q);
       h_ctl[3 * batch + q] = 1;
       h_ctl[4 * batch + q] = (M.dev != nullptr && mask_of_req != nullptr) ? mask_of_req[r0 + q] : -1;
@@ -996,10 +999,10 @@ static int reco_sweep(rbod_gallery* g, const float* ex_dev, const int8_t* sign, 
     // the K5 selection ranks by the key it is given; metric COSINE emits that key as the score and pads with -inf,
     // which is what K (larger is better for every metric) needs
     if (sample_stride > 1) {
-      RBOD_TRY(launch_reco_collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim,
-                                   g->dim, g->dp, g->rows, 0, sample_stride, M.dev, M.words, d_slot, d_rmask, d_thr,
-                                   d_thr_row, d_active, d_qnorm, ns, nreq, cap, g->coll_score.as<double>(),
-                                   g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(), g->num_sms, st));
+      RBOD_TRY(collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim, g->dim, g->dp,
+                       g->rows, 0, sample_stride, M.dev, M.words, d_slot, d_rmask, d_thr, d_thr_row, d_active, d_qnorm,
+                       ns, nreq, cap, g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
+                       g->num_sms, st));
       RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
                                   d_req, nreq, cap, k, 1, RBOD_COSINE, d_thr, d_thr_row, d_active, d_nactive, d_scores,
                                   d_rows, d_keys, st));
@@ -1008,10 +1011,10 @@ static int reco_sweep(rbod_gallery* g, const float* ex_dev, const int8_t* sign, 
     int iter = 0, left = nreq;
     for (; iter < max_iter && left > 0; ++iter) {
       RBOD_CUDA(cudaMemsetAsync(d_nactive, 0, 4, st));
-      RBOD_TRY(launch_reco_collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim,
-                                   g->dim, g->dp, g->rows, 0, 1, M.dev, M.words, d_slot, d_rmask, d_thr, d_thr_row,
-                                   d_active, d_qnorm, ns, nreq, cap, g->coll_score.as<double>(),
-                                   g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(), g->num_sms, st));
+      RBOD_TRY(collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim, g->dim, g->dp,
+                       g->rows, 0, 1, M.dev, M.words, d_slot, d_rmask, d_thr, d_thr_row, d_active, d_qnorm, ns, nreq,
+                       cap, g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(), g->num_sms,
+                       st));
       RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
                                   d_req, nreq, cap, k, 0, RBOD_COSINE, d_thr, d_thr_row, d_active, d_nactive, d_scores,
                                   d_rows, d_keys, st));
@@ -1021,7 +1024,7 @@ static int reco_sweep(rbod_gallery* g, const float* ex_dev, const int8_t* sign, 
       if (iter > 0) ++*resweeps;
     }
     if (left > 0)
-      return set_error(RBOD_E_OVERFLOW, "rbod_recommend: more than %d rows tie around the k-th score of a request", cap);
+      return set_error(RBOD_E_OVERFLOW, "%s: more than %d rows tie around the k-th score of a request", who, cap);
     r0 += nreq;
   }
   return RBOD_OK;
@@ -1407,44 +1410,51 @@ int rbod_search_masks(rbod_gallery* g, const float* queries, int64_t Q, int32_t 
                      stream);
 }
 
-int rbod_recommend(rbod_gallery* g, const float* examples, int64_t n_examples, const int8_t* example_sign,
-                   const int64_t* request_offsets, int64_t R, int32_t k, const uint32_t* row_masks, int32_t n_masks,
-                   const int32_t* mask_of_request, float* out_scores, int64_t* out_rows, double* out_keys,
-                   rbod_search_stats* stats, void* stream) {
-  // the host-side arguments are checked first, so a malformed call is refused before anything touches a device
-  if (R < 0 || R > (1ll << 24)) return set_error(RBOD_E_INVAL, "rbod_recommend: R = %lld out of range", (long long)R);
-  if (k < 1) return set_error(RBOD_E_INVAL, "rbod_recommend: k = %d < 1", k);
-  if (n_examples < 0) return set_error(RBOD_E_INVAL, "rbod_recommend: n_examples = %lld", (long long)n_examples);
+// Checks common to rbod_recommend and rbod_discover, made on the host before anything touches a device, in the order
+// they are reported: counts, masks, NULL pointers, offsets (request sizes 1 to 32).  `what` names the per-example array.
+static int check_example_args(const char* who, const char* what, const float* examples, int64_t n_examples,
+                              const void* per_example, const int64_t* off, int64_t R, int k,
+                              const uint32_t* row_masks, int32_t n_masks, const float* out_scores,
+                              const int64_t* out_rows) {
+  if (R < 0 || R > (1ll << 24)) return set_error(RBOD_E_INVAL, "%s: R = %lld out of range", who, (long long)R);
+  if (k < 1) return set_error(RBOD_E_INVAL, "%s: k = %d < 1", who, k);
+  if (n_examples < 0) return set_error(RBOD_E_INVAL, "%s: n_examples = %lld", who, (long long)n_examples);
   if (n_masks < 0 || (n_masks > 0 && !row_masks))
-    return set_error(RBOD_E_INVAL, "rbod_recommend: %d masks, row_masks %s", n_masks, row_masks ? "set" : "NULL");
-  if (R > 0 && (!examples || !example_sign || !request_offsets || !out_scores || !out_rows))
-    return set_error(RBOD_E_INVAL, "rbod_recommend: NULL examples, signs, offsets or outputs");
-  if (request_offsets) {
-    if (request_offsets[0] != 0 || request_offsets[R] != n_examples)
-      return set_error(RBOD_E_INVAL, "rbod_recommend: request_offsets must run from 0 to n_examples = %lld",
+    return set_error(RBOD_E_INVAL, "%s: %d masks, row_masks %s", who, n_masks, row_masks ? "set" : "NULL");
+  if (R > 0 && (!examples || !per_example || !off || !out_scores || !out_rows))
+    return set_error(RBOD_E_INVAL, "%s: NULL examples, %s, offsets or outputs", who, what);
+  if (off) {
+    if (off[0] != 0 || off[R] != n_examples)
+      return set_error(RBOD_E_INVAL, "%s: request_offsets must run from 0 to n_examples = %lld", who,
                        (long long)n_examples);
     for (int64_t r = 0; r < R; ++r) {
-      const int64_t n = request_offsets[r + 1] - request_offsets[r];
+      const int64_t n = off[r + 1] - off[r];
       if (n < 1 || n > 32)
-        return set_error(RBOD_E_INVAL, "rbod_recommend: request %lld has %lld examples, not 1 to 32 (offsets monotone)",
+        return set_error(RBOD_E_INVAL, "%s: request %lld has %lld examples, not 1 to 32 (offsets monotone)", who,
                          (long long)r, (long long)n);
     }
   }
-  for (int64_t e = 0; e < (R > 0 ? n_examples : 0); ++e)
-    if (example_sign[e] != 1 && example_sign[e] != -1)
-      return set_error(RBOD_E_INVAL, "rbod_recommend: example_sign[%lld] = %d is not +1 or -1", (long long)e,
-                       (int)example_sign[e]);
+  return RBOD_OK;
+}
+
+// The rest of rbod_recommend / rbod_discover once the requests themselves are checked: the host mask ids, k, the
+// handle, then example_sweep with `collect` over the examples whose slot-table flags are `flags` [n_examples].
+static int example_search(const char* who, CollectLauncher collect, rbod_gallery* g, const float* examples,
+                          int64_t n_examples, const int* flags, const int64_t* request_offsets, int64_t R, int32_t k,
+                          const uint32_t* row_masks, int32_t n_masks, const int32_t* mask_of_request,
+                          float* out_scores, int64_t* out_rows, double* out_keys, rbod_search_stats* stats,
+                          void* stream) {
   const bool ids_dev = is_device_ptr(mask_of_request);
   if (mask_of_request && !ids_dev)
     for (int64_t r = 0; r < R; ++r)
       if (mask_of_request[r] < -1 || mask_of_request[r] >= n_masks)
-        return set_error(RBOD_E_INVAL, "rbod_recommend: mask_of_request[%lld] = %d is outside [-1, %d)", (long long)r,
+        return set_error(RBOD_E_INVAL, "%s: mask_of_request[%lld] = %d is outside [-1, %d)", who, (long long)r,
                          mask_of_request[r], n_masks);
-  if (k > 1024) return set_error(RBOD_E_UNSUPPORTED, "rbod_recommend: k=%d > 1024", k);
-  if (!g) return set_error(RBOD_E_INVAL, "rbod_recommend: NULL handle");
+  if (k > 1024) return set_error(RBOD_E_UNSUPPORTED, "%s: k=%d > 1024", who, k);
+  if (!g) return set_error(RBOD_E_INVAL, "%s: NULL handle", who);
   if (stats) memset(stats, 0, sizeof(*stats));
   if (R == 0) return RBOD_OK;
-  if (g->rows >= 0xffffffffll) return set_error(RBOD_E_UNSUPPORTED, "rbod_recommend: more than 2^32-2 rows per shard");
+  if (g->rows >= 0xffffffffll) return set_error(RBOD_E_UNSUPPORTED, "%s: more than 2^32-2 rows per shard", who);
   RBOD_CUDA(cudaSetDevice(g->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
 
@@ -1456,8 +1466,8 @@ int rbod_recommend(rbod_gallery* g, const float* examples, int64_t n_examples, c
       RBOD_CUDA(cudaStreamSynchronize(st));
       for (int64_t r = 0; r < R; ++r)
         if (ids[r] < -1 || ids[r] >= n_masks)
-          return set_error(RBOD_E_INVAL, "rbod_recommend: mask_of_request[%lld] = %d is outside [-1, %d)",
-                           (long long)r, ids[r], n_masks);
+          return set_error(RBOD_E_INVAL, "%s: mask_of_request[%lld] = %d is outside [-1, %d)", who, (long long)r,
+                           ids[r], n_masks);
     } else {
       memcpy(ids.data(), mask_of_request, (size_t)R * 4);
     }
@@ -1488,8 +1498,8 @@ int rbod_recommend(rbod_gallery* g, const float* examples, int64_t n_examples, c
   const void* xd = nullptr;
   RBOD_TRY(to_device(examples, (size_t)n_examples * g->dim * 4, g->q32, st, &xd));
   int64_t n_launch = 0, resweeps = 0;
-  RBOD_TRY(reco_sweep(g, static_cast<const float*>(xd), example_sign, request_offsets, R, k, M,
-                      ids.empty() ? nullptr : ids.data(), ds, dr, dk, &n_launch, &resweeps, st));
+  RBOD_TRY(example_sweep(g, collect, who, static_cast<const float*>(xd), flags, request_offsets, R, k, M,
+                         ids.empty() ? nullptr : ids.data(), ds, dr, dk, &n_launch, &resweeps, st));
   RBOD_TRY(copy_out(out_scores, ds, n_out * 4, st));
   RBOD_TRY(copy_out(out_rows, dr, n_out * 8, st));
   if (out_keys) RBOD_TRY(copy_out(out_keys, dk, n_out * 8, st));
@@ -1501,6 +1511,58 @@ int rbod_recommend(rbod_gallery* g, const float* examples, int64_t n_examples, c
     stats->fallback_queries = resweeps;
   }
   return RBOD_OK;
+}
+
+int rbod_recommend(rbod_gallery* g, const float* examples, int64_t n_examples, const int8_t* example_sign,
+                   const int64_t* request_offsets, int64_t R, int32_t k, const uint32_t* row_masks, int32_t n_masks,
+                   const int32_t* mask_of_request, float* out_scores, int64_t* out_rows, double* out_keys,
+                   rbod_search_stats* stats, void* stream) {
+  RBOD_TRY(check_example_args("rbod_recommend", "signs", examples, n_examples, example_sign, request_offsets, R, k,
+                              row_masks, n_masks, out_scores, out_rows));
+  const int64_t E = R > 0 ? n_examples : 0;
+  std::vector<int> flags(E);
+  for (int64_t e = 0; e < E; ++e) {
+    if (example_sign[e] != 1 && example_sign[e] != -1)
+      return set_error(RBOD_E_INVAL, "rbod_recommend: example_sign[%lld] = %d is not +1 or -1", (long long)e,
+                       (int)example_sign[e]);
+    flags[e] = example_sign[e] < 0 ? SLOT_NEG : 0;
+  }
+  return example_search("rbod_recommend", launch_reco_collect, g, examples, n_examples, flags.data(), request_offsets,
+                        R, k, row_masks, n_masks, mask_of_request, out_scores, out_rows, out_keys, stats, stream);
+}
+
+int rbod_discover(rbod_gallery* g, const float* examples, int64_t n_examples, const int8_t* example_role,
+                  const int64_t* request_offsets, int64_t R, int32_t k, const uint32_t* row_masks, int32_t n_masks,
+                  const int32_t* mask_of_request, float* out_scores, int64_t* out_rows, double* out_keys,
+                  rbod_search_stats* stats, void* stream) {
+  RBOD_TRY(check_example_args("rbod_discover", "roles", examples, n_examples, example_role, request_offsets, R, k,
+                              row_masks, n_masks, out_scores, out_rows));
+  const int64_t E = R > 0 ? n_examples : 0;
+  for (int64_t e = 0; e < E; ++e)
+    if (example_role[e] < -1 || example_role[e] > 1)
+      return set_error(RBOD_E_INVAL, "rbod_discover: example_role[%lld] = %d is not 0, +1 or -1", (long long)e,
+                       (int)example_role[e]);
+  // an optional target first, then (+1, -1) pairs; a request with a target is a discovery, without one a context search
+  std::vector<int> flags(E);
+  for (int64_t r = 0; r < R; ++r) {
+    const int64_t e0 = request_offsets[r], e1 = request_offsets[r + 1];
+    const int disc = example_role[e0] == 0 ? SLOT_DISC : 0;
+    for (int64_t e = e0; e < e1; ++e) {
+      const int role = example_role[e];
+      if (role == 0 && e != e0)
+        return set_error(RBOD_E_INVAL, "rbod_discover: request %lld: %s target at example %lld (a target comes first)",
+                         (long long)r, disc ? "a second" : "a", (long long)e);
+      if (role == 1 && (e + 1 == e1 || example_role[e + 1] != -1))
+        return set_error(RBOD_E_INVAL, "rbod_discover: request %lld: positive example %lld is not followed by a negative",
+                         (long long)r, (long long)e);
+      if (role == -1 && (e == e0 || example_role[e - 1] != 1))
+        return set_error(RBOD_E_INVAL, "rbod_discover: request %lld: negative example %lld is not preceded by a positive",
+                         (long long)r, (long long)e);
+      flags[e] = disc | (role == 0 ? SLOT_TARGET : role < 0 ? SLOT_NEG : 0);
+    }
+  }
+  return example_search("rbod_discover", launch_disc_collect, g, examples, n_examples, flags.data(), request_offsets,
+                        R, k, row_masks, n_masks, mask_of_request, out_scores, out_rows, out_keys, stats, stream);
 }
 
 // ---- split search: the two halves of rbod_search around an exchange between shards ---------------------------

@@ -186,8 +186,24 @@ int launch_dist_collect(int metric, const double* q64, const float* master32, co
 int launch_dist_select(const double* coll_key, const uint32_t* coll_idx, int* coll_cnt, const int* qsel, int nf,
                        int cap, int k, int sample, int metric, double* thr, uint32_t* thr_row, int* active,
                        int* n_active, float* out_scores, int64_t* out_rows, double* out_keys, cudaStream_t st);
-// K6: exact best_score recommendation sweep (selection through K5's widen / select launchers)
+// K6 / K7: exact example sweeps (rbod_slot_sweep.cuh; selection through K5's widen / select launchers).  Slot table of
+// a pass: request of the pass | SLOT_LAST (the request's last slot) | the example's flags: SLOT_NEG (a negative
+// example, K6; a pair's negative, K7), SLOT_TARGET (K7's target) and SLOT_DISC (K7, on every slot of a request with a
+// target: the request is scored as a discovery, not a context search).
+constexpr int SLOT_REQ = 31, SLOT_LAST = 32, SLOT_NEG = 64, SLOT_TARGET = 128, SLOT_DISC = 256;
+using CollectLauncher = int (*)(int metric, const double* q64, const float* master32, const uint16_t* rows16,
+                                int kind16, int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0,
+                                int64_t stride, const uint32_t* row_mask, int64_t mask_words, const int* slot_tab,
+                                const int* req_mask, const double* thr, const uint32_t* thr_row, const int* active,
+                                const double* qnorm, int n_slots, int n_req, int cap, double* coll_key,
+                                uint32_t* coll_idx, int* coll_cnt, int num_sms, cudaStream_t st);
 int launch_reco_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
+                        int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride,
+                        const uint32_t* row_mask, int64_t mask_words, const int* slot_tab, const int* req_mask,
+                        const double* thr, const uint32_t* thr_row, const int* active, const double* qnorm,
+                        int n_slots, int n_req, int cap, double* coll_key, uint32_t* coll_idx, int* coll_cnt,
+                        int num_sms, cudaStream_t st);
+int launch_disc_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
                         int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride,
                         const uint32_t* row_mask, int64_t mask_words, const int* slot_tab, const int* req_mask,
                         const double* thr, const uint32_t* thr_row, const int* active, const double* qnorm,

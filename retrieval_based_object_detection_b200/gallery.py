@@ -239,33 +239,56 @@ class Gallery:
         -> ``scores`` [R, k] float32 descending (-inf padded), ``rows`` [R, k] int64 (-1 padded), ``scores64`` the fp64
         scores when ``want_keys``.  ``row_mask`` / ``mask_of_request`` are as ``search``'s ``row_mask`` /
         ``mask_of_query``, one mask id per request."""
+        return self._example_search("recommend", "signs", examples, signs, offsets, k, row_mask, mask_of_request,
+                                    want_keys)
+
+    # -- K7 ---------------------------------------------------------------------------------
+    def discover(self, examples, roles, offsets, k: int, row_mask=None, mask_of_request=None,
+                 want_keys: bool = False) -> SearchResult:
+        """Exact discovery and context search (rbod_discover): request r is the examples ``offsets[r]:offsets[r + 1]``
+        of ``examples`` [E, dim], 1 to 32 per request: an optional target first (``roles`` 0), then pairs of a positive
+        (+1) directly followed by its negative (-1).  With the search key of the collection's metric, sim = identity
+        (-sqrt(-key) for euclid), f(y) = y / (1 + |y|), s(y) = 0.5 (f(y) + 1) and MARGIN = 2**-23, a row scores
+
+        * with a target t (discovery): sum over pairs of (+1 if key(p) > key(n) else -1) + s(sim(key(t)));
+        * without (context): sum over pairs, in order, of f(min(sim(key(p)) - sim(key(n)) - MARGIN, 0)), which is 0
+          for every row on the positive side of every pair.
+
+        This is the rule of Qdrant >= 1.7 as read from its source, not checked against a live Qdrant.  Larger is better
+        for every metric.  Returns and masks as ``recommend``."""
+        return self._example_search("discover", "roles", examples, roles, offsets, k, row_mask, mask_of_request,
+                                    want_keys)
+
+    def _example_search(self, name, what, examples, per_example, offsets, k, row_mask, mask_of_request, want_keys):
+        """rbod_recommend / rbod_discover (``name``) with ``per_example`` the int8 signs / roles (``what``)."""
         keep, p_x = self._in(examples, np.float32, "float32")
         if keep.ndim != 2 or keep.shape[1] != self.dim:
-            raise ValueError(f"recommend: expected [E, {self.dim}] examples, got {tuple(keep.shape)}")
-        sg = _as_host(signs, np.int8)
+            raise ValueError(f"{name}: expected [E, {self.dim}] examples, got {tuple(keep.shape)}")
+        sg = _as_host(per_example, np.int8)
         off = _as_host(offsets, np.int64)
         if off.ndim != 1 or len(off) < 1 or sg.shape != (int(keep.shape[0]),):
-            raise ValueError("recommend: offsets must be [R + 1] and signs [E]")
+            raise ValueError(f"{name}: offsets must be [R + 1] and {what} [E]")
         R = len(off) - 1
         k_mask, p_mask = self._in(row_mask, np.uint32, "int32")
         k_ids, p_ids = self._in(mask_of_request, np.int32, "int32")
         n_masks = 0 if k_mask is None else 1
         if k_ids is not None:
             if tuple(k_ids.shape) != (R,):
-                raise ValueError(f"recommend: mask_of_request must hold one mask id per request ({R})")
+                raise ValueError(f"{name}: mask_of_request must hold one mask id per request ({R})")
             n_masks = 0
             if k_mask is not None:
                 words = (len(self) + 31) // 32
                 if k_mask.ndim != 2 or k_mask.shape[1] != words:
-                    raise ValueError(f"recommend: with mask_of_request, row_mask must be [M, {words}] words, "
+                    raise ValueError(f"{name}: with mask_of_request, row_mask must be [M, {words}] words, "
                                      f"got {tuple(k_mask.shape)}")
                 n_masks = int(k_mask.shape[0])
         scores, p_s = self._alloc_like(keep, (R, k), np.float32, "float32")
         rows, p_r = self._alloc_like(keep, (R, k), np.int64, "int64")
         keys, p_k = (self._alloc_like(keep, (R, k), np.float64, "float64") if want_keys else (None, None))
         st = N.SearchStats()
-        N.check(self._lib.rbod_recommend(self._h, p_x, int(keep.shape[0]), sg.ctypes.data, off.ctypes.data, R, int(k),
-                                         p_mask, n_masks, p_ids, p_s, p_r, p_k, ctypes.byref(st), _current_stream()))
+        N.check(getattr(self._lib, "rbod_" + name)(self._h, p_x, int(keep.shape[0]), sg.ctypes.data, off.ctypes.data, R,
+                                                 int(k), p_mask, n_masks, p_ids, p_s, p_r, p_k, ctypes.byref(st),
+                                                 _current_stream()))
         return SearchResult(scores, rows, keys, {f: getattr(st, f) for f, _ in st._fields_})
 
     # -- split search (row-sharded collections): see include/rbod.h "Split search" ------------------------------

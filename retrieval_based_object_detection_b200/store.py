@@ -32,8 +32,8 @@ import numpy as np
 
 FORMAT_VERSION = 1
 _FLUSH_THRESHOLD = 65536  # staged rows that force a device flush
-MAX_RECOMMEND_EXAMPLES = 32   # examples per recommendation request (rbod_recommend)
-MAX_RECOMMEND_FETCH = 1024    # rows a recommendation request fetches: limit + offset + its example ids
+MAX_RECOMMEND_EXAMPLES = 32   # examples per recommendation / discovery request (rbod_recommend, rbod_discover)
+MAX_RECOMMEND_FETCH = 1024    # rows such a request fetches: limit + offset + its example ids
 
 
 class CollectionNotFound(Exception):
@@ -707,27 +707,13 @@ class Collection:
                 raise ValueError(f"recommend: a request needs 1 to {MAX_RECOMMEND_EXAMPLES} examples, got {len(items)}")
             if strategy == "average_vector" and not pos:
                 raise ValueError("recommend: the average_vector strategy needs at least one positive example")
-            vecs, signs, ex_slots = [], [], set()
-            for x, sign in items:
-                if isinstance(x, (str, uuid.UUID)) or (isinstance(x, (int, np.integer)) and not isinstance(x, bool)):
-                    pid = canonical_id(x)
-                    slot = self.slot_of.get(pid)
-                    if slot is None:
-                        raise ValueError(f"recommend: point {pid!r} not found in collection {self.name!r}")
-                    ex_slots.add(slot)
-                    vecs.append(slot)
-                else:
-                    v = np.asarray(x, dtype=np.float32).reshape(-1)
-                    if v.shape[0] != self.dim:
-                        raise ValueError(f"Wrong input: Vector dimension error: expected dim: {self.dim}, got {v.shape[0]}")
-                    vecs.append(v)
-                signs.append(sign)
+            vecs, ex_slots = self._resolve_examples([x for x, _ in items], "recommend")
+            signs = [sign for _, sign in items]
             fetch = int(k) + len(ex_slots)
             if fetch > MAX_RECOMMEND_FETCH:
                 raise ValueError(f"recommend: limit + offset + example ids = {fetch} exceeds {MAX_RECOMMEND_FETCH}")
             plans.append((vecs, signs, ex_slots, flt, int(k), fetch))
-        id_slots = sorted({v for p in plans for v in p[0] if isinstance(v, int)})
-        stored = dict(zip(id_slots, self.stored_vectors(id_slots)))
+        stored = self._stored_examples([p[0] for p in plans])
         out = [(np.zeros(0, np.float32), np.zeros(0, np.int64))] * len(plans)
         by_fetch = {}
         for i, p in enumerate(plans):
@@ -753,6 +739,77 @@ class Collection:
                                              row_mask=masks, mask_of_request=None if masks is None else ids)
                 scores, rows = res.scores, res.rows
             scores, rows = np.asarray(scores), np.asarray(rows)
+            for j, i in enumerate(members):
+                keep = ~np.isin(rows[j], list(plans[i][2]))
+                out[i] = (scores[j][keep][:plans[i][4]], rows[j][keep][:plans[i][4]])
+        return out
+
+
+    def _resolve_examples(self, examples, who: str):
+        """Examples of a recommendation or discovery request, each a point id or a raw vector -> (one entry per
+        example: the point's slot (int) or the vector as float32 [dim]; the set of slots given by id).  An unknown id
+        is a ValueError that names it."""
+        vecs, ex_slots = [], set()
+        for x in examples:
+            if isinstance(x, (str, uuid.UUID)) or (isinstance(x, (int, np.integer)) and not isinstance(x, bool)):
+                pid = canonical_id(x)
+                slot = self.slot_of.get(pid)
+                if slot is None:
+                    raise ValueError(f"{who}: point {pid!r} not found in collection {self.name!r}")
+                ex_slots.add(slot)
+                vecs.append(slot)
+            else:
+                v = np.asarray(x, dtype=np.float32).reshape(-1)
+                if v.shape[0] != self.dim:
+                    raise ValueError(f"Wrong input: Vector dimension error: expected dim: {self.dim}, got {v.shape[0]}")
+                vecs.append(v)
+        return vecs, ex_slots
+
+    def _stored_examples(self, vec_lists):
+        """{slot: stored vector} of every slot in the ``_resolve_examples`` lists ``vec_lists``, read in one call."""
+        id_slots = sorted({v for vecs in vec_lists for v in vecs if isinstance(v, int)})
+        return dict(zip(id_slots, self.stored_vectors(id_slots)))
+
+    def discover(self, requests):
+        """Discovery and context search: ``requests`` = [(target, pairs, filter, k)], where ``target`` is None or an
+        example, ``pairs`` a list of (positive, negative) examples, every example a point id or a raw vector, and k =
+        limit + offset.  ``Gallery.discover`` (exact fp64 sweep, kernel K7) answers them; scores are larger-is-better
+        for every metric (see include/rbod.h, rbod_discover).  Examples given by id take their stored vector and never
+        appear in that request's answer.
+
+        Each request has a target or at least one pair, 1 to 32 examples, and fetches k + (its distinct example ids)
+        rows, at most 1024.  Requests with the same fetch share one device call.  -> [(scores float32, slots int64)]
+        per request, at most k each, example points removed."""
+        self.flush()
+        plans = []
+        for target, pairs, flt, k in requests:
+            pairs = list(pairs or [])
+            items = ([] if target is None else [(target, 0)]) + [(x, r) for p, n in pairs for x, r in ((p, 1), (n, -1))]
+            if not items:
+                raise ValueError("discover: a request needs a target or at least one context pair")
+            if len(items) > MAX_RECOMMEND_EXAMPLES:
+                raise ValueError(f"discover: a request has at most {MAX_RECOMMEND_EXAMPLES} examples (a target and "
+                                 f"two per pair), got {len(items)}")
+            vecs, ex_slots = self._resolve_examples([x for x, _ in items], "discover")
+            fetch = int(k) + len(ex_slots)
+            if fetch > MAX_RECOMMEND_FETCH:
+                raise ValueError(f"discover: limit + offset + example ids = {fetch} exceeds {MAX_RECOMMEND_FETCH}")
+            plans.append((vecs, [r for _, r in items], ex_slots, flt, int(k), fetch))
+        stored = self._stored_examples([p[0] for p in plans])
+        out = [(np.zeros(0, np.float32), np.zeros(0, np.int64))] * len(plans)
+        by_fetch = {}
+        for i, p in enumerate(plans):
+            if p[4] >= 1:
+                by_fetch.setdefault(p[5], []).append(i)
+        for fetch, members in by_fetch.items():
+            ex = [np.stack([stored[v] if isinstance(v, int) else v for v in plans[i][0]]) for i in members]
+            masks, ids = self._filter_masks([plans[i][3] for i in members])
+            offsets = np.zeros(len(members) + 1, dtype=np.int64)
+            np.cumsum([len(e) for e in ex], out=offsets[1:])
+            roles = np.concatenate([np.asarray(plans[i][1], dtype=np.int8) for i in members])
+            res = self.gallery.discover(np.concatenate(ex), roles, offsets, fetch,
+                                        row_mask=masks, mask_of_request=None if masks is None else ids)
+            scores, rows = np.asarray(res.scores), np.asarray(res.rows)
             for j, i in enumerate(members):
                 keep = ~np.isin(rows[j], list(plans[i][2]))
                 out[i] = (scores[j][keep][:plans[i][4]], rows[j][keep][:plans[i][4]])
