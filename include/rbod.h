@@ -40,6 +40,10 @@
  *       client.discover(target=..., context=[ContextExamplePair(positive, negative), ...]), discover_batch and
  *       query_points(query=DiscoverQuery(...) | ContextQuery(...)): "like this target, on the right side of these
  *       corrections" (pairs such as "this crop is the class, that near-identical one is not").
+ *   rbod_search_mmr                                (the search's kernels, then kernel K8 mmr_select)
+ *       client.query_points(query=NearestQuery(nearest=v, mmr=Mmr(diversity, candidates_limit))) and
+ *       query_batch_points: a top-k that is not ten near-copies of one object (the gallery holds ~18 augmented variants
+ *       of every crop, 23_augmentation.py / 31_...py).
  *   rbod_merge_topk                                (kernel K4 topk_merge)
  *       no reference call site; merges per-GPU top-k lists after the NCCL all-gather.
  *
@@ -237,6 +241,44 @@ int rbod_search_masks(rbod_gallery* g, const float* queries, int64_t Q, int32_t 
                       const uint32_t* row_masks, int32_t n_masks, const int32_t* mask_of_query,
                       float* out_scores, int64_t* out_rows, double* out_scores64,
                       rbod_search_stats* stats, void* stream);
+
+/* --- K8: maximal marginal relevance (MMR) ------------------------------------------------
+ * For a query q with the exact candidates c_0 .. c_{L-1} of rbod_search_masks(..., k = candidates, ...), ordered as that
+ * search orders them (key desc, row slot asc), and with
+ *   key(x, g)  the search key in fp64 from the stored values (the fp32 master of an f32 collection, the 16-bit rows
+ *              otherwise, never the fp16 shadow): COSINE dot / (|x| |g|), DOT dot, EUCLID -sum (x - g)^2,
+ *              MANHATTAN -sum |x - g|,
+ *   sim(y)     y, or -sqrt(-y) for EUCLID (rbod_recommend's sim: larger is better for every metric),
+ *   rel(c)     sim(key(q, c)), the candidate search's own fp64 key,
+ *   lambda     1 - diversity[q],
+ * the first pick is c_0 and every later pick maximises, over the candidates not yet picked,
+ *   mmr(c) = lambda * rel(c) - diversity * max over picked s of sim(key(s, c))
+ * computed in fp64 in exactly that order (the picked stored row s is the query side of the pairwise key); exact ties go
+ * to the smaller candidate rank.  Results come in SELECTION order, each with its ordinary search score (cosine / dot, or
+ * the distance for EUCLID / MANHATTAN), so they are not sorted by score; diversity 0 returns the search's first `limit`
+ * rows.  (Qdrant >= 1.15 documents the same kind of rule; this one was not checked against a live Qdrant or its source.
+ * The EUCLID sim and the tie rule are choices of this library.)
+ * queries:         [Q, dim] fp32, host or device.
+ * limit:           results per query; candidates: L, limit <= L <= 1024.
+ * diversity:       [Q] fp64 in [0, 1], host.
+ * score_threshold: [Q] fp32, host, or NULL; NaN = none.  A candidate takes part only if its fp32 search score is >= the
+ *                  threshold (<= for EUCLID / MANHATTAN, whose scores are distances), so a request still fills `limit`
+ *                  when enough candidates pass.
+ * row_masks / n_masks / mask_of_query: as rbod_search_masks.
+ * out_scores:      [Q, limit] fp32 search scores in selection order; -inf (COSINE, DOT) or +inf (EUCLID, MANHATTAN) where
+ *                  fewer candidates exist.
+ * out_rows:        [Q, limit] int64 row slots in selection order, -1 padded.
+ * out_keys:        optional [Q, limit] fp64 search keys (-inf padded), or NULL.  Outputs host or device.
+ * stats:           optional: the candidate search's, total_launches counting K8.
+ * RBOD_E_INVAL (checked on the host before anything is launched, a device mask_of_query after reading it back): limit < 1,
+ * candidates < limit, a diversity that is NaN or outside [0, 1], diversity == NULL with Q > 0, a mask id outside
+ * [-1, n_masks), n_masks < 0, n_masks > 0 with row_masks == NULL, NULL queries or outputs with Q > 0.  candidates > 1024
+ * is RBOD_E_UNSUPPORTED.  Q = 0 and an empty collection return RBOD_OK (the latter with padding).
+ * Result: row q is identical, bit for bit, whether query q is sent alone or with others.                    */
+int rbod_search_mmr(rbod_gallery* g, const float* queries, int64_t Q, int32_t limit, int32_t candidates,
+                    const double* diversity, const float* score_threshold, const uint32_t* row_masks, int32_t n_masks,
+                    const int32_t* mask_of_query, float* out_scores, int64_t* out_rows, double* out_keys,
+                    rbod_search_stats* stats, void* stream);
 
 /* --- K6: recommendation, best_score strategy ---------------------------------------------
  * A request is a set of 1 to 32 examples, each positive ("like this") or negative ("unlike this").  For an example e and

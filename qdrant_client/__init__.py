@@ -10,7 +10,8 @@ operations: without the built extension and a B200 they raise.
 
 Method subset = what the four scripts call (SURVEY.md §8(b)) + ``search`` / ``query_points`` /
 ``search_batch`` as BASELINE.json's north star specifies, + ``recommend`` / ``recommend_batch``, + ``discover`` /
-``discover_batch`` and ``query_points(query=DiscoverQuery | ContextQuery)``.  Configuration is by environment only,
+``discover_batch`` and ``query_points(query=DiscoverQuery | ContextQuery)``, + ``query_points(query=NearestQuery(mmr=...))``
+and ``query_batch_points``.  Configuration is by environment only,
 because the scripts take no flags: ``RBOD_STORE_DIR``, ``RBOD_GALLERY_DTYPE`` (f32 | bf16 | f16),
 ``RBOD_DEVICE`` (CUDA ordinal).
 """
@@ -18,6 +19,7 @@ from __future__ import annotations
 
 import atexit
 import os
+import uuid
 from typing import Any, Dict, Iterable, List, Optional, Sequence
 
 import numpy as np
@@ -27,9 +29,9 @@ from retrieval_based_object_detection_b200.store import Collection, CollectionNo
 from . import models
 from .models import (Batch, CollectionConfig, CollectionDescription, CollectionInfo, CollectionParams,
                      CollectionsResponse, ContextExamplePair, ContextPair, ContextQuery, CountResult,
-                     DiscoverQuery, DiscoverRequest, Distance, PointStruct, QueryResponse, RecommendQuery,
-                     RecommendRequest, RecommendStrategy, Record, ScoredPoint, UpdateResult, UpdateStatus,
-                     VectorParams)
+                     DiscoverQuery, DiscoverRequest, Distance, NearestQuery, PointStruct, QueryRequest, QueryResponse,
+                     RecommendQuery, RecommendRequest, RecommendStrategy, Record, ScoredPoint, SearchRequest,
+                     UpdateResult, UpdateStatus, VectorParams)
 
 __all__ = ["QdrantClient", "models", "CollectionNotFound"]
 __version__ = "1.9.0+rbod"
@@ -56,6 +58,9 @@ def _distance_name(d) -> str:
         if str(d).lower() in (cand.value.lower(), cand.name.lower()):
             return cand.value
     raise ValueError(f"unknown distance {d!r}")
+
+
+MAX_MMR_CANDIDATES = 1024   # candidates_limit of an MMR query (rbod_search_mmr)
 
 
 def _context_pairs(context) -> list:
@@ -272,8 +277,118 @@ class QdrantClient:
                                   with_payload=with_payload, with_vector=with_vectors, using=_ignored.get("using"),
                                   lookup_from=_ignored.get("lookup_from"))
             return QueryResponse(points=self._discover(collection_name, [req], score_threshold)[0])
+        if isinstance(query, NearestQuery):
+            req = QueryRequest(query=query, filter=query_filter, limit=limit, offset=offset, with_payload=with_payload,
+                               with_vector=with_vectors, score_threshold=score_threshold, using=_ignored.get("using"),
+                               lookup_from=_ignored.get("lookup_from"), prefetch=_ignored.get("prefetch"))
+            if query.mmr is None:
+                vec = self._nearest_vector(req)
+                return QueryResponse(points=self.search(collection_name, vec, query_filter, limit, offset, with_payload,
+                                                        with_vectors, score_threshold))
+            return QueryResponse(points=self._mmr(collection_name, [req])[0])
         return QueryResponse(points=self.search(collection_name, query, query_filter, limit, offset, with_payload,
                                                 with_vectors, score_threshold))
+
+    @staticmethod
+    def _nearest_vector(r):
+        """The vector of a ``QueryRequest`` whose query is a ``NearestQuery``; what this drop-in does not support is a
+        ValueError."""
+        if r.using is not None:
+            raise ValueError("query_points: named vectors (using=) are not supported by this drop-in")
+        if r.lookup_from is not None:
+            raise ValueError("query_points: lookup_from (vectors from another collection) is not supported")
+        if r.prefetch is not None:
+            raise ValueError("query_points: prefetch (and fusion) is not supported by this drop-in")
+        v = r.query.nearest
+        if isinstance(v, (str, uuid.UUID)) or (isinstance(v, (int, np.integer)) and not isinstance(v, bool)):
+            raise ValueError("query_points: NearestQuery(nearest=<point id>) is not supported; pass the vector")
+        return v
+
+    def _mmr(self, collection_name: str, requests) -> List[List[ScoredPoint]]:
+        """``QueryRequest``s whose query is a ``NearestQuery`` with ``mmr``: one device call (``Collection.search_mmr``)
+        per distinct (limit + offset, candidates_limit)."""
+        col = self._root.get(collection_name)
+        plans = []
+        for r in requests:
+            q = np.asarray(self._nearest_vector(r), dtype=np.float32).reshape(-1)
+            if q.shape[0] != col.dim:
+                raise ValueError(f"Wrong input: Vector dimension error: expected dim: {col.dim}, got {q.shape[0]}")
+            m = r.query.mmr
+            k = int(r.limit) + int(r.offset or 0)
+            div = 0.5 if m.diversity is None else float(m.diversity)
+            if not 0.0 <= div <= 1.0:
+                raise ValueError(f"query_points: mmr diversity must be in [0, 1], got {m.diversity!r}")
+            cand = k if m.candidates_limit is None else int(m.candidates_limit)
+            if cand < k:
+                raise ValueError(f"query_points: mmr candidates_limit = {cand} is smaller than limit + offset = {k}")
+            if cand > MAX_MMR_CANDIDATES:
+                raise ValueError(f"query_points: mmr candidates_limit = {cand} exceeds {MAX_MMR_CANDIDATES}")
+            plans.append((q, k, cand, div))
+        out: List[List[ScoredPoint]] = [[] for _ in requests]
+        groups: Dict[tuple, List[int]] = {}
+        for i, (_, k, cand, _) in enumerate(plans):
+            if k >= 1:
+                groups.setdefault((k, cand), []).append(i)
+        for (k, cand), members in groups.items():
+            scores, slots = col.search_mmr(np.stack([plans[i][0] for i in members]), k, cand,
+                                           np.array([plans[i][3] for i in members]),
+                                           [requests[i].score_threshold for i in members],
+                                           [requests[i].filter for i in members])
+            for j, i in enumerate(members):
+                r = requests[i]
+                out[i] = self._scored(col, scores[j], slots[j], bool(r.with_payload), bool(r.with_vector),
+                                      r.score_threshold)[int(r.offset or 0):]
+        return out
+
+    def query_batch_points(self, collection_name: str, requests, **_ignored: Any) -> List[QueryResponse]:
+        """One ``query_points`` per ``QueryRequest``; each kind of query goes to its batch path: vectors and plain
+        ``NearestQuery`` to ``search_batch``, ``NearestQuery`` with ``mmr`` to one device call per distinct (limit +
+        offset, candidates_limit), ``RecommendQuery`` to ``recommend_batch``, ``DiscoverQuery`` / ``ContextQuery`` to
+        discovery.  The output equals the per-request ``query_points`` loop."""
+        requests = list(requests)
+        out: List[List[ScoredPoint]] = [[] for _ in requests]
+        kinds: Dict[str, List[int]] = {}
+        for i, r in enumerate(requests):
+            q = r.query
+            kind = ("mmr" if isinstance(q, NearestQuery) and q.mmr is not None else "recommend"
+                    if isinstance(q, RecommendQuery) else "discover" if isinstance(q, (DiscoverQuery, ContextQuery))
+                    else "search")
+            kinds.setdefault(kind, []).append(i)
+        for kind, members in kinds.items():
+            reqs = [requests[i] for i in members]
+            if kind == "search":
+                res = self.search_batch(collection_name, [SearchRequest(
+                    vector=self._nearest_vector(r) if isinstance(r.query, NearestQuery) else r.query, filter=r.filter,
+                    limit=r.limit, offset=r.offset, with_payload=r.with_payload, with_vector=r.with_vector,
+                    score_threshold=r.score_threshold) for r in reqs])
+            elif kind == "mmr":
+                res = self._mmr(collection_name, reqs)
+            elif kind == "recommend":
+                res = self.recommend_batch(collection_name, [RecommendRequest(
+                    positive=r.query.recommend.positive, negative=r.query.recommend.negative, filter=r.filter,
+                    limit=r.limit, offset=r.offset, with_payload=r.with_payload, with_vector=r.with_vector,
+                    score_threshold=r.score_threshold, using=r.using, lookup_from=r.lookup_from,
+                    strategy=r.query.recommend.strategy) for r in reqs])
+            else:
+                res = [None] * len(reqs)
+                by_thr: Dict[Any, List[int]] = {}
+                for j, r in enumerate(reqs):
+                    by_thr.setdefault(r.score_threshold, []).append(j)
+                for thr, js in by_thr.items():
+                    dreqs = []
+                    for j in js:
+                        r = reqs[j]
+                        target, context = ((r.query.discover.target, r.query.discover.context)
+                                           if isinstance(r.query, DiscoverQuery) else (None, r.query.context))
+                        dreqs.append(DiscoverRequest(target=target, context=context, filter=r.filter, limit=r.limit,
+                                                     offset=r.offset, with_payload=r.with_payload,
+                                                     with_vector=r.with_vector, using=r.using,
+                                                     lookup_from=r.lookup_from))
+                    for j, pts in zip(js, self._discover(collection_name, dreqs, thr)):
+                        res[j] = pts
+            for i, pts in zip(members, res):
+                out[i] = pts
+        return [QueryResponse(points=p) for p in out]
 
     def search_batch(self, collection_name: str, requests=None, queries=None, k: Optional[int] = None,
                      row_filter=None, query_filters=None, **_ignored: Any):

@@ -182,6 +182,30 @@ class ContextQuery(_Model):
     _fields = ("context",)
 
 
+class Mmr(_Model):
+    """Maximal marginal relevance of a ``NearestQuery``: ``limit`` picks among the exact top-``candidates_limit``, each
+    trading relevance against similarity to the points already picked.  Defaults of this drop-in (not checked against
+    Qdrant): ``diversity`` 0.5, ``candidates_limit`` = limit + offset."""
+    _fields = ("diversity", "candidates_limit")
+    _defaults = {"diversity": None, "candidates_limit": None}
+
+
+class NearestQuery(_Model):
+    """Nearest-neighbour search of the query API: ``nearest`` is a vector; with ``mmr`` the answer is diversified."""
+    _fields = ("nearest", "mmr")
+    _defaults = {"mmr": None}
+
+
+class QueryRequest(_Model):
+    """One request of ``query_batch_points``: ``query`` is a vector, a ``NearestQuery``, a ``RecommendQuery``, a
+    ``DiscoverQuery`` or a ``ContextQuery``."""
+    _fields = ("query", "filter", "limit", "offset", "with_payload", "with_vector", "score_threshold", "using",
+               "lookup_from", "prefetch", "params", "shard_key")
+    _defaults = {"query": None, "filter": None, "limit": 10, "offset": 0, "with_payload": None, "with_vector": None,
+                 "score_threshold": None, "using": None, "lookup_from": None, "prefetch": None, "params": None,
+                 "shard_key": None}
+
+
 class PointIdsList(_Model):
     _fields = ("points",)
 

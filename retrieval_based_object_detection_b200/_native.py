@@ -79,6 +79,8 @@ SIGNATURES = {
                                       ctypes.POINTER(SearchStats), _P]),
     "rbod_discover": (ctypes.c_int, [_P, _P, _I64, _P, _P, _I64, _I32, _P, _I32, _P, _P, _P, _P,
                                      ctypes.POINTER(SearchStats), _P]),
+    "rbod_search_mmr": (ctypes.c_int, [_P, _P, _I64, _I32, _I32, _P, _P, _P, _I32, _P, _P, _P, _P,
+                                       ctypes.POINTER(SearchStats), _P]),
     "rbod_merge_topk": (ctypes.c_int, [_P, _P, _I32, _I64, _I32, _P, _P, _P, _P]),
     "rbod_merge_topk_packed": (ctypes.c_int, [_P, _P, _I32, _I64, _I32, _P, _P, _P, _P]),
     "rbod_search_begin": (ctypes.c_int, [_P, _P, _I64, _I32, _I32, _P, _P, ctypes.POINTER(SearchStats), _P]),

@@ -21,6 +21,7 @@
 //
 // All of it is small, latency/HBM-bound integer and fp64 work on CUDA cores.
 #include "rbod_common.cuh"
+#include "rbod_exact_score.cuh"
 #include "rbod_internal.h"
 
 #include <algorithm>
@@ -200,33 +201,6 @@ __device__ void certify_query(const FinishArgs& P, int64_t q, float tau, const Q
   }
 }
 
-// Exact score of (query, stored row) with the query already widened to fp64 in shared memory: one warp per pair,
-// every lane returns it.  Vector path (dim % 8 == 0, rows 16-byte aligned): the whole row is in flight before the
-// first multiply (up to 4 x 16 bytes per lane for 16-bit rows up to 1024 columns), 8 elements per lane and step.
-template <int METRIC>
-__device__ __forceinline__ void score_step8(const double* __restrict__ q8, const float (&x)[8], double& a, double& b) {
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const double xd = (double)x[i];
-    if (METRIC == RBOD_EUCLID) {
-      const double d = q8[i] - xd;
-      a = fma(d, d, a);
-    } else {
-      a = fma(q8[i], xd, a);
-      if (METRIC == RBOD_COSINE) b = fma(xd, xd, b);
-    }
-  }
-}
-
-__device__ __forceinline__ void unpack8(const uint4& h, int kind16, float (&x)[8]) {
-  const uint32_t w[4] = {h.x, h.y, h.z, h.w};
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    x[2 * i] = h16_to_f32(static_cast<uint16_t>(w[i] & 0xffffu), kind16);
-    x[2 * i + 1] = h16_to_f32(static_cast<uint16_t>(w[i] >> 16), kind16);
-  }
-}
-
 // A stored 16-bit row of up to 1024 columns as this lane's share of it: 8 consecutive elements per 256-column step.
 struct RowRegs { uint4 h[4]; };
 __device__ __forceinline__ void load_row16(RowRegs& R, const uint16_t* __restrict__ g16, int dim, int lane) {
@@ -235,16 +209,6 @@ __device__ __forceinline__ void load_row16(RowRegs& R, const uint16_t* __restric
     const int c0 = lane * 8 + 256 * i;
     R.h[i] = c0 < dim ? __ldg(reinterpret_cast<const uint4*>(g16 + c0)) : make_uint4(0u, 0u, 0u, 0u);
   }
-}
-
-template <int METRIC>
-__device__ __forceinline__ double finish_score(double a, double b, double qq) {
-  a = warp_sum_f64(a);
-  if (METRIC == RBOD_EUCLID) return -a;
-  if (METRIC == RBOD_DOT) return a;
-  b = warp_sum_f64(b);
-  const double den = sqrt(qq) * sqrt(b);
-  return den > 0.0 ? a / den : 0.0;
 }
 
 template <int METRIC>
@@ -258,41 +222,6 @@ __device__ __forceinline__ double exact_score_regs(const double* __restrict__ q6
       float x[8];
       unpack8(R.h[i], kind16, x);
       score_step8<METRIC>(q64 + c0, x, a, b);
-    }
-  }
-  return finish_score<METRIC>(a, b, qq);
-}
-
-template <int METRIC>
-__device__ __forceinline__ double exact_score_q64(const double* __restrict__ q64, double qq,
-                                                  const float* __restrict__ g32, const uint16_t* __restrict__ g16,
-                                                  int kind16, int dim, int lane) {
-  double a = 0.0, b = 0.0;
-  const bool vec = (dim & 7) == 0 &&
-                   (g32 ? (reinterpret_cast<uintptr_t>(g32) & 15) == 0 : (reinterpret_cast<uintptr_t>(g16) & 15) == 0);
-  if (vec) {
-    for (int c0 = lane * 8; c0 < dim; c0 += 256) {
-      float x[8];
-      if (g32) {
-        const float4 g0 = __ldg(reinterpret_cast<const float4*>(g32 + c0));
-        const float4 g1 = __ldg(reinterpret_cast<const float4*>(g32 + c0 + 4));
-        x[0] = g0.x; x[1] = g0.y; x[2] = g0.z; x[3] = g0.w;
-        x[4] = g1.x; x[5] = g1.y; x[6] = g1.z; x[7] = g1.w;
-      } else {
-        unpack8(__ldg(reinterpret_cast<const uint4*>(g16 + c0)), kind16, x);
-      }
-      score_step8<METRIC>(q64 + c0, x, a, b);
-    }
-  } else {
-    for (int c = lane; c < dim; c += 32) {
-      const double xd = g32 ? (double)g32[c] : (double)h16_to_f32(g16[c], kind16);
-      if (METRIC == RBOD_EUCLID) {
-        const double d = q64[c] - xd;
-        a = fma(d, d, a);
-      } else {
-        a = fma(q64[c], xd, a);
-        if (METRIC == RBOD_COSINE) b = fma(xd, xd, b);
-      }
     }
   }
   return finish_score<METRIC>(a, b, qq);

@@ -294,7 +294,8 @@ int rbod_destroy(rbod_gallery* g) {
                     &g->out_rows, &g->out_scores64, &g->flags, &g->flag_q, &g->flag_thr, &g->flag_lo, &g->fq16, &g->groupmax, &g->tau_init, &g->coll_score,
                     &g->coll_idx, &g->coll_cnt, &g->mask_dev, &g->mask_ids, &g->fmask_ids, &g->dump, &g->sync_counters, &g->prof, &g->seg_idx, &g->seg_off, &g->seg_out,
                     &g->seg_partials, &g->seg_prefix, &g->seg_arrive, &g->seg_scratch, &g->seg_member, &g->gather_idx,
-                    &g->gather_out, &g->dist_q64, &g->dist_thr, &g->dist_ctl};
+                    &g->gather_out, &g->dist_q64, &g->dist_thr, &g->dist_ctl, &g->mmr_scores, &g->mmr_rows,
+                    &g->mmr_keys, &g->mmr_ctl, &g->mmr_q64};
   for (DevBuf* b : bufs) b->release();
   if (g->ev0) cudaEventDestroy(g->ev0);
   if (g->ev1) cudaEventDestroy(g->ev1);
@@ -1408,6 +1409,116 @@ int rbod_search_masks(rbod_gallery* g, const float* queries, int64_t Q, int32_t 
                       double* out_scores64, rbod_search_stats* stats, void* stream) {
   return search_impl(g, queries, Q, k, row_masks, n_masks, mask_of_query, out_scores, out_rows, out_scores64, stats,
                      stream);
+}
+
+// Maximal marginal relevance: the exact top-`candidates` of every query (search_impl, unchanged, into the handle's K8
+// workspaces), then K8's greedy selection of `limit` of them, then the copy-out.
+int rbod_search_mmr(rbod_gallery* g, const float* queries, int64_t Q, int32_t limit, int32_t candidates,
+                    const double* diversity, const float* score_threshold, const uint32_t* row_masks, int32_t n_masks,
+                    const int32_t* mask_of_query, float* out_scores, int64_t* out_rows, double* out_keys,
+                    rbod_search_stats* stats, void* stream) {
+  const char* who = "rbod_search_mmr";
+  if (Q < 0 || Q > (1ll << 24)) return set_error(RBOD_E_INVAL, "%s: Q = %lld out of range", who, (long long)Q);
+  if (limit < 1) return set_error(RBOD_E_INVAL, "%s: limit = %d < 1", who, limit);
+  if (candidates < limit)
+    return set_error(RBOD_E_INVAL, "%s: candidates = %d < limit = %d", who, candidates, limit);
+  if (n_masks < 0 || (n_masks > 0 && !row_masks))
+    return set_error(RBOD_E_INVAL, "%s: %d masks, row_masks %s", who, n_masks, row_masks ? "set" : "NULL");
+  if (Q > 0 && !diversity) return set_error(RBOD_E_INVAL, "%s: diversity is NULL", who);
+  if (Q > 0 && (!queries || !out_scores || !out_rows)) return set_error(RBOD_E_INVAL, "%s: NULL queries or outputs", who);
+  for (int64_t q = 0; q < Q; ++q)
+    if (!(diversity[q] >= 0.0 && diversity[q] <= 1.0))
+      return set_error(RBOD_E_INVAL, "%s: query %lld: diversity %g is not in [0, 1]", who, (long long)q, diversity[q]);
+  // mask ids are checked here, on the host, and handed to the search as a host array
+  std::vector<int32_t> ids;
+  if (mask_of_query && Q > 0) {
+    ids.resize((size_t)Q);
+    if (is_device_ptr(mask_of_query)) {
+      if (!g) return set_error(RBOD_E_INVAL, "%s: NULL handle", who);
+      RBOD_CUDA(cudaSetDevice(g->device));
+      RBOD_CUDA(cudaMemcpyAsync(ids.data(), mask_of_query, (size_t)Q * 4, cudaMemcpyDeviceToHost,
+                                static_cast<cudaStream_t>(stream)));
+      RBOD_CUDA(cudaStreamSynchronize(static_cast<cudaStream_t>(stream)));
+    } else {
+      memcpy(ids.data(), mask_of_query, (size_t)Q * 4);
+    }
+    for (int64_t q = 0; q < Q; ++q)
+      if (ids[q] < -1 || ids[q] >= n_masks)
+        return set_error(RBOD_E_INVAL, "%s: query %lld: mask_of_query = %d is outside [-1, %d)", who, (long long)q,
+                         ids[q], n_masks);
+  }
+  if (candidates > MMR_MAX_CANDIDATES)
+    return set_error(RBOD_E_UNSUPPORTED, "%s: candidates = %d > %d", who, candidates, MMR_MAX_CANDIDATES);
+  if (!g) return set_error(RBOD_E_INVAL, "%s: NULL handle", who);
+  if (stats) memset(stats, 0, sizeof(*stats));
+  if (Q == 0) return RBOD_OK;
+  RBOD_CUDA(cudaSetDevice(g->device));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const bool dist = g->metric == RBOD_EUCLID || g->metric == RBOD_MANHATTAN;
+  const size_t n_out = (size_t)Q * limit;
+  if (g->rows == 0) {
+    std::vector<float> hs(n_out, dist ? INFINITY : -INFINITY);
+    std::vector<int64_t> hr(n_out, -1);
+    std::vector<double> hd(n_out, -INFINITY);
+    RBOD_CUDA(cudaMemcpyAsync(out_scores, hs.data(), n_out * 4, cudaMemcpyDefault, st));
+    RBOD_CUDA(cudaMemcpyAsync(out_rows, hr.data(), n_out * 8, cudaMemcpyDefault, st));
+    if (out_keys) RBOD_CUDA(cudaMemcpyAsync(out_keys, hd.data(), n_out * 8, cudaMemcpyDefault, st));
+    RBOD_CUDA(cudaStreamSynchronize(st));
+    if (stats) stats->queries = Q;
+    return RBOD_OK;
+  }
+
+  // 1. the candidates: an ordinary search with k = candidates, written straight into the K8 workspaces
+  const size_t n_cand = (size_t)Q * candidates;
+  RBOD_TRY(g->mmr_scores.ensure(n_cand * 4));
+  RBOD_TRY(g->mmr_rows.ensure(n_cand * 8));
+  RBOD_TRY(g->mmr_keys.ensure(n_cand * 8));
+  RBOD_TRY(search_impl(g, queries, Q, candidates, row_masks, n_masks, ids.empty() ? nullptr : ids.data(),
+                       g->mmr_scores.as<float>(), g->mmr_rows.as<int64_t>(), g->mmr_keys.as<double>(), stats, stream));
+
+  // 2. K8
+  std::vector<double> ctl_d(diversity, diversity + Q);
+  std::vector<float> ctl_t;
+  if (score_threshold) ctl_t.assign(score_threshold, score_threshold + Q);
+  RBOD_TRY(g->mmr_ctl.ensure((size_t)Q * 12));
+  RBOD_CUDA(cudaMemcpyAsync(g->mmr_ctl.p, ctl_d.data(), (size_t)Q * 8, cudaMemcpyHostToDevice, st));
+  if (score_threshold)
+    RBOD_CUDA(cudaMemcpyAsync(g->mmr_ctl.as<double>() + Q, ctl_t.data(), (size_t)Q * 4, cudaMemcpyHostToDevice, st));
+  RBOD_TRY(g->out_scores.ensure(n_out * 4));
+  RBOD_TRY(g->out_rows.ensure(n_out * 8));
+  RBOD_TRY(g->out_scores64.ensure(n_out * 8));
+  MmrArgs A;
+  A.Q = Q;
+  A.L = candidates;
+  A.limit = limit;
+  A.cand_rows = g->mmr_rows.as<int64_t>();
+  A.cand_scores = g->mmr_scores.as<float>();
+  A.cand_keys = g->mmr_keys.as<double>();
+  A.diversity = g->mmr_ctl.as<double>();
+  A.score_threshold = score_threshold ? reinterpret_cast<const float*>(g->mmr_ctl.as<double>() + Q) : nullptr;
+  A.master32 = g->master32;
+  A.rows16 = g->rows16;
+  A.kind16 = g->kind16;
+  A.dim = g->dim;
+  A.ld32 = g->dim;
+  A.ld16 = g->dp;
+  A.q64_scratch = nullptr;
+  if (g->dim > MMR_SMEM_DIM) {
+    RBOD_TRY(g->mmr_q64.ensure((size_t)mmr_grid(Q, g->dim, g->num_sms) * g->dim * 8));
+    A.q64_scratch = g->mmr_q64.as<double>();
+  }
+  A.out_scores = is_device_ptr(out_scores) ? out_scores : g->out_scores.as<float>();
+  A.out_rows = is_device_ptr(out_rows) ? out_rows : g->out_rows.as<int64_t>();
+  A.out_keys = (out_keys && is_device_ptr(out_keys)) ? out_keys : g->out_scores64.as<double>();
+  RBOD_TRY(launch_mmr_select(g->metric, A, g->num_sms, st));
+
+  // 3. copy-out
+  RBOD_TRY(copy_out(out_scores, A.out_scores, n_out * 4, st));
+  RBOD_TRY(copy_out(out_rows, A.out_rows, n_out * 8, st));
+  if (out_keys) RBOD_TRY(copy_out(out_keys, A.out_keys, n_out * 8, st));
+  RBOD_CUDA(cudaStreamSynchronize(st));
+  if (stats) stats->total_launches += 1;
+  return RBOD_OK;
 }
 
 // Checks common to rbod_recommend and rbod_discover, made on the host before anything touches a device, in the order

@@ -7,6 +7,8 @@
 #include <cstdarg>
 #include <cstddef>
 
+#include <algorithm>
+
 #include "../../include/rbod.h"
 
 namespace rbod {
@@ -209,6 +211,31 @@ int launch_disc_collect(int metric, const double* q64, const float* master32, co
                         const double* thr, const uint32_t* thr_row, const int* active, const double* qnorm,
                         int n_slots, int n_req, int cap, double* coll_key, uint32_t* coll_idx, int* coll_cnt,
                         int num_sms, cudaStream_t st);
+// K8: maximal marginal relevance over each query's exact candidate list (k8_mmr.cu).  Device pointers throughout.
+constexpr int MMR_MAX_CANDIDATES = 1024;
+constexpr int MMR_SMEM_DIM = 4096;   // picks up to this many columns are widened into shared memory, wider ones into
+                                     // q64_scratch: one row per CTA of mmr_grid
+struct MmrArgs {
+  int64_t Q;
+  int L, limit;
+  const int64_t* cand_rows;   // [Q][L] the candidate search's answer: row slots (-1 padded), fp32 scores, fp64 keys
+  const float* cand_scores;
+  const double* cand_keys;
+  const double* diversity;    // [Q] in [0, 1]
+  const float* score_threshold;   // [Q] (NaN = none) or nullptr
+  const float* master32;
+  const uint16_t* rows16;
+  int kind16, dim;
+  int64_t ld32, ld16;
+  double* q64_scratch;        // [mmr_grid][dim] when dim > MMR_SMEM_DIM, else unused
+  float* out_scores;          // [Q][limit] in selection order
+  int64_t* out_rows;
+  double* out_keys;
+};
+inline int64_t mmr_grid(int64_t Q, int dim, int num_sms) {
+  return dim > MMR_SMEM_DIM ? std::min<int64_t>(Q, 2 * (int64_t)num_sms) : Q;
+}
+int launch_mmr_select(int metric, const MmrArgs& A, int num_sms, cudaStream_t st);
 int launch_merge_topk(const double* scores64, const int64_t* ids, int64_t shard_stride, const int64_t* row0_host,
                       int G, int64_t Q, int k, float* out_scores, int64_t* out_ids, double* out_scores64,
                       cudaStream_t st, const double* ubound = nullptr, int* flag_q = nullptr, int* n_flag = nullptr);
@@ -267,5 +294,7 @@ struct rbod_gallery {
   rbod::DevBuf seg_idx, seg_off, seg_out, seg_partials, seg_prefix, seg_arrive, seg_scratch, seg_member;
   rbod::DevBuf gather_idx, gather_out;
   rbod::DevBuf dist_q64, dist_thr, dist_ctl;   // K5: widened query batch, thresholds, {qsel, active, n_active, slot mask}
+  rbod::DevBuf mmr_scores, mmr_rows, mmr_keys;  // K8: the candidate search's answer [Q][L] (search_impl writes it directly)
+  rbod::DevBuf mmr_ctl, mmr_q64;                // K8: {diversity, threshold} per query; widened picks of wide rows
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };

@@ -227,6 +227,52 @@ class Gallery:
         stats = {f: getattr(st, f) for f, _ in st._fields_}
         return SearchResult(scores, rows, s64, stats)
 
+    # -- K8 ---------------------------------------------------------------------------------
+    def search_mmr(self, queries, limit: int, candidates: int, diversity, score_threshold=None, row_mask=None,
+                   mask_of_query=None, want_keys: bool = False) -> SearchResult:
+        """Maximal marginal relevance (rbod_search_mmr): per query, the exact top-``candidates`` c_0 .. c_{L-1} of an
+        ordinary search, then ``limit`` of them picked greedily.  With the collection's fp64 search key, sim = identity
+        (-sqrt(-key) for euclid), rel(c) = sim(key(query, c)) and lambda = 1 - diversity, the first pick is c_0 and every
+        later pick maximises lambda * rel(c) - diversity * max over picked s of sim(key(s, c)) (fp64, in that order),
+        exact ties to the smaller candidate rank.  Qdrant >= 1.15 documents the same kind of rule; this one has not been
+        checked against a live Qdrant or its source.
+
+        ``diversity``: a float in [0, 1] or one per query.  ``score_threshold``: None, a float or one per query (NaN =
+        none): only candidates whose search score is >= it (<= for euclid / manhattan distances) take part.
+        ``row_mask`` / ``mask_of_query``: as ``search``.  -> ``scores`` [Q, limit] float32 search scores and ``rows``
+        [Q, limit] int64 in SELECTION order (padded with -inf / +inf for distances, and -1), ``scores64`` the fp64 keys
+        when ``want_keys``."""
+        keep, p_q = self._in(queries, np.float32, "float32")
+        if keep.ndim == 1:
+            keep = keep.reshape(1, -1)
+        if keep.ndim != 2 or keep.shape[1] != self.dim:
+            raise ValueError(f"search_mmr: expected [Q, {self.dim}] queries, got {tuple(keep.shape)}")
+        Q = int(keep.shape[0])
+        div = np.ascontiguousarray(np.broadcast_to(np.asarray(diversity, dtype=np.float64), (Q,)))
+        thr = (None if score_threshold is None else
+               np.ascontiguousarray(np.broadcast_to(np.asarray(score_threshold, dtype=np.float32), (Q,))))
+        k_mask, p_mask = self._in(row_mask, np.uint32, "int32")
+        k_ids, p_ids = self._in(mask_of_query, np.int32, "int32")
+        n_masks = 0 if k_mask is None else 1
+        if k_ids is not None:
+            if tuple(k_ids.shape) != (Q,):
+                raise ValueError(f"search_mmr: mask_of_query must hold one mask id per query ({Q})")
+            n_masks = 0
+            if k_mask is not None:
+                words = (len(self) + 31) // 32
+                if k_mask.ndim != 2 or k_mask.shape[1] != words:
+                    raise ValueError(f"search_mmr: with mask_of_query, row_mask must be [M, {words}] words, "
+                                     f"got {tuple(k_mask.shape)}")
+                n_masks = int(k_mask.shape[0])
+        scores, p_s = self._alloc_like(keep, (Q, limit), np.float32, "float32")
+        rows, p_r = self._alloc_like(keep, (Q, limit), np.int64, "int64")
+        keys, p_k = (self._alloc_like(keep, (Q, limit), np.float64, "float64") if want_keys else (None, None))
+        st = N.SearchStats()
+        N.check(self._lib.rbod_search_mmr(self._h, p_q, Q, int(limit), int(candidates), div.ctypes.data,
+                                          None if thr is None else thr.ctypes.data, p_mask, n_masks, p_ids, p_s, p_r,
+                                          p_k, ctypes.byref(st), _current_stream()))
+        return SearchResult(scores, rows, keys, {f: getattr(st, f) for f, _ in st._fields_})
+
     # -- K6 ---------------------------------------------------------------------------------
     def recommend(self, examples, signs, offsets, k: int, row_mask=None, mask_of_request=None,
                   want_keys: bool = False) -> SearchResult:

@@ -669,6 +669,24 @@ class Collection:
         res = self.gallery.search(q, k, row_mask=self.filter_mask(flt))
         return res.scores, res.rows
 
+    def search_mmr(self, queries: np.ndarray, limit: int, candidates: int, diversity, score_thresholds=None,
+                   filters=None):
+        """Maximal marginal relevance (``Gallery.search_mmr``, kernel K8) of every query, in one device call: ``limit``
+        picks among the exact top-``candidates``, in selection order.  ``diversity`` / ``score_thresholds``: one value
+        or one per query (a threshold None = none); ``filters``: None or one filter (or None) per query.
+        -> (scores [Q, limit] float32, slots [Q, limit] int64)."""
+        self.flush()
+        q = np.ascontiguousarray(queries, dtype=np.float32).reshape(-1, self.dim)
+        thr = None
+        if score_thresholds is not None:
+            thr = np.asarray([np.nan if t is None else float(t)
+                              for t in np.broadcast_to(np.asarray(score_thresholds, dtype=object), (len(q),))],
+                             dtype=np.float32)
+        masks, ids = self._filter_masks(list(filters) if filters is not None else [None] * len(q))
+        res = self.gallery.search_mmr(q, int(limit), int(candidates), diversity, score_threshold=thr,
+                                      row_mask=masks, mask_of_query=None if masks is None else ids)
+        return np.asarray(res.scores), np.asarray(res.rows)
+
     def _filter_masks(self, filters):
         """One filter (or None) per request -> (row masks [M, words], or None when every filter is None; mask id per
         request, int32, -1 = no filter).  Equal filters compile to one mask; models are not hashable, their repr is
