@@ -15,12 +15,12 @@
 //      rows); a list that overflows `cap` tightens its threshold to the k-th best key it did record --
 //      still a lower bound of the true k-th key -- and only those queries are swept again;
 //   3. select: sort each list in shared memory, emit (distance, row) ascending by distance.
-// Every lane owns one gallery row and scores it against a batch of up to 32 queries staged in shared memory (32
-// independent DFMA chains per lane, no cross-lane reduction), so the gallery is read once per batch of 32 queries.
-#include "rbod_common.cuh"
-#include "rbod_internal.h"
-
-#include <algorithm>
+// The row loop is slot_sweep (rbod_slot_sweep.cuh), shared with K6 and K7: every lane owns one gallery row and scores
+// it against a pass of up to 32 queries staged in shared memory (32 independent DFMA chains per lane, no cross-lane
+// reduction), so the gallery is read once per 32 queries.  A query is a request of one slot and its end of a row,
+// KeyRow below, records the key itself; K6 and K7 fold a request's slots into one score instead.  The widening and
+// the selection below serve all three, and so does the host loop (rbod_api.cu: sweep).
+#include "rbod_slot_sweep.cuh"
 
 namespace rbod {
 
@@ -45,175 +45,27 @@ dist_widen_queries_kernel(const float* __restrict__ q, const int* __restrict__ q
   }
 }
 
-__device__ __forceinline__ void cp_async_4(void* smem_dst, const void* gsrc) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(smem_dst)), "l"(gsrc) : "memory");
-}
-__device__ __forceinline__ void cp_async_8(void* smem_dst, const void* gsrc) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(smem_dst)), "l"(gsrc) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_1() { asm volatile("cp.async.wait_group 1;" ::: "memory"); }
+// End of a row: a query is a request of one slot, whose score is its key.
+struct KeyRow {
+  static constexpr bool kSlotIsRequest = true;
+  double key = 0.0;
+  __device__ __forceinline__ void fold(int, double k) { key = k; }
+  __device__ __forceinline__ double score(int) const { return key; }
+  __device__ __forceinline__ void reset() {}
+};
 
-constexpr int K5_CH = 64;        // columns per staged chunk
-constexpr int K5_ROWS = 256;     // gallery rows per CTA step: 8 warps x 32 lanes, one row per lane
-
-// Rows r = row0, row0 + stride, ... < n_rows.  A CTA takes 256 of them at a time and every LANE owns one row, so a
-// row's distance to a query is a private fp64 accumulator: no reduction across lanes, NQ independent DFMA chains
-// per lane.  The work is staged through shared memory in chunks of 64 columns, double-buffered with cp.async: each
-// warp copies its 32 rows' chunk (coalesced, a row at a time, pitch odd so lane-strided reads are conflict-free),
-// the CTA copies the chunk of the NQ fp64 queries once for all 8 warps, and the inner loop is one broadcast
-// LDS.128 (two query elements) per four fp64 operations.  q64 is [32, dim], zero rows beyond the batch; `wpr` =
-// 4-byte words per chunk row (64 for fp32 rows, 32 for 16-bit rows), `pitch` = wpr + 1.
-template <int METRIC, int NQ>
+template <int METRIC, int NS>
 __global__ void __launch_bounds__(256, 1)
-dist_collect_kernel(const double* __restrict__ q64, const float* __restrict__ master32,
-                    const uint16_t* __restrict__ rows16, int kind16, int dim, int64_t ld32, int64_t ld16,
-                    int64_t n_rows, int64_t row0, int64_t stride, const uint32_t* __restrict__ row_mask,
-                    int64_t mask_words, const int* __restrict__ slot_mask, const double* __restrict__ thr, const uint32_t* __restrict__ thr_row, const int* __restrict__ active,
-                    const double* __restrict__ qnorm, int nf, int cap, double* __restrict__ coll_key,
-                    uint32_t* __restrict__ coll_idx, int* __restrict__ coll_cnt) {
-  extern __shared__ __align__(16) uint8_t k5_smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const bool f32rows = master32 != nullptr;
-  const int wpr = f32rows ? K5_CH : K5_CH / 2, pitch = wpr + 1;
-  double* qs = reinterpret_cast<double*>(k5_smem);                                   // [2][NQ][K5_CH]
-  uint32_t* xs = reinterpret_cast<uint32_t*>(k5_smem + (size_t)2 * NQ * K5_CH * 8);  // [2][8][32][pitch]
-  __shared__ double thr_s[32], qn_s[32];
-  __shared__ uint32_t thr_row_s[32];   // with thr_s a (key, row) pair bound: rows tying with the key count up to this row
-  __shared__ int mask_s[32];            // per-query masks: the mask slot f reads, -1 = none
-  if (threadIdx.x < 32) {
-    thr_s[threadIdx.x] = (threadIdx.x < nf && active[threadIdx.x]) ? thr[threadIdx.x] : INFINITY;
-    thr_row_s[threadIdx.x] = (threadIdx.x < nf && thr_row != nullptr) ? thr_row[threadIdx.x] : 0xffffffffu;
-    qn_s[threadIdx.x] = threadIdx.x < nf ? qnorm[threadIdx.x] : 0.0;
-    mask_s[threadIdx.x] = (threadIdx.x < nf && slot_mask != nullptr) ? slot_mask[threadIdx.x] : -1;
-  }
-  __syncthreads();
-  constexpr bool kInner = METRIC == RBOD_COSINE || METRIC == RBOD_DOT;   // keys built from q . g
-  double gg = 0.0;                                                        // |row|^2 of this lane's row (COSINE)
-
-  const int64_t n_visit = n_rows > row0 ? (n_rows - row0 + stride - 1) / stride : 0;   // rows of this pass
-  const int n_chunks = (dim + K5_CH - 1) / K5_CH;
-  const int64_t n_groups = (n_visit + K5_ROWS - 1) / K5_ROWS;
-  const int64_t my_groups = n_groups > blockIdx.x ? (n_groups - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-  const int64_t n_steps = my_groups * n_chunks;     // (group, chunk) pairs this CTA walks, in order
-
-  auto row_of = [&](int64_t g, int l) -> int64_t {  // gallery row of lane l of this warp in group g, or -1
-    const int64_t v = (blockIdx.x + g * gridDim.x) * K5_ROWS + warp * 32 + l;
-    if (v >= n_visit) return -1;
-    const int64_t r = row0 + v * stride;
-    // one mask for the whole batch: masked rows are not even loaded
-    if (row_mask != nullptr && slot_mask == nullptr && !((row_mask[r >> 5] >> (r & 31)) & 1u)) return -1;
-    return r;
-  };
-  auto issue = [&](int64_t step, int b) {
-    const int64_t g = step / n_chunks;
-    const int c0 = (int)(step - g * n_chunks) * K5_CH;
-    const int cw = min(K5_CH, dim - c0);
-    // this warp's 32 rows, one row per iteration, lanes across the chunk's words
-    uint32_t* xb = xs + ((size_t)b * 8 + warp) * 32 * pitch;
-    for (int j = 0; j < 32; ++j) {
-      const int64_t r = row_of(g, j);
-      if (r < 0) continue;
-      if (f32rows) {
-        const uint32_t* src = reinterpret_cast<const uint32_t*>(master32 + r * ld32 + c0);
-        for (int w = lane; w < cw; w += 32) cp_async_4(xb + j * pitch + w, src + w);
-      } else {
-        const uint32_t* src = reinterpret_cast<const uint32_t*>(rows16 + r * ld16 + c0);   // padded to 64 elements
-        cp_async_4(xb + j * pitch + lane, src + lane);
-      }
-    }
-    // the CTA's query chunk
-    double* qb = qs + (size_t)b * NQ * K5_CH;
-    for (int i = threadIdx.x; i < NQ * K5_CH; i += 256) {
-      const int f = i / K5_CH, c = i - f * K5_CH;
-      if (c < cw) cp_async_8(qb + i, q64 + (int64_t)f * dim + c0 + c);
-    }
-    cp_async_commit();
-  };
-
-  double acc[NQ];
-  if (n_steps > 0) issue(0, 0);
-  for (int64_t step = 0; step < n_steps; ++step) {
-    const int b = (int)(step & 1);
-    const int64_t g = step / n_chunks;
-    const int ci = (int)(step - g * n_chunks);
-    if (step + 1 < n_steps) issue(step + 1, b ^ 1); else cp_async_commit();
-    cp_async_wait_1();
-    __syncthreads();
-    if (ci == 0) {
-#pragma unroll
-      for (int f = 0; f < NQ; ++f) acc[f] = 0.0;
-      gg = 0.0;
-    }
-    const int cw = min(K5_CH, dim - ci * K5_CH);
-    const uint32_t* xr = xs + (((size_t)b * 8 + warp) * 32 + lane) * pitch;
-    const double* qb = qs + (size_t)b * NQ * K5_CH;
-    auto elem = [&](int c) -> double {
-      if (f32rows) return (double)__uint_as_float(xr[c]);
-      const uint32_t w = xr[c >> 1];
-      return (double)h16_to_f32((uint16_t)((c & 1) ? (w >> 16) : (w & 0xffffu)), kind16);
-    };
-    int c = 0;
-    for (; c + 1 < cw; c += 2) {
-      const double x0 = elem(c), x1 = elem(c + 1);
-      if (METRIC == RBOD_COSINE) gg = fma(x1, x1, fma(x0, x0, gg));
-#pragma unroll
-      for (int f = 0; f < NQ; ++f) {
-        const double2 qq = *reinterpret_cast<const double2*>(qb + f * K5_CH + c);
-        if (kInner) {
-          acc[f] = fma(qq.y, x1, fma(qq.x, x0, acc[f]));
-        } else {
-          const double d0 = qq.x - x0, d1 = qq.y - x1;
-          if (METRIC == RBOD_EUCLID) acc[f] = fma(d1, d1, fma(d0, d0, acc[f]));
-          else acc[f] += fabs(d0) + fabs(d1);
-        }
-      }
-    }
-    if (c < cw) {
-      const double x0 = elem(c);
-      if (METRIC == RBOD_COSINE) gg = fma(x0, x0, gg);
-#pragma unroll
-      for (int f = 0; f < NQ; ++f) {
-        if (kInner) {
-          acc[f] = fma(qb[f * K5_CH + c], x0, acc[f]);
-        } else {
-          const double d0 = qb[f * K5_CH + c] - x0;
-          if (METRIC == RBOD_EUCLID) acc[f] = fma(d0, d0, acc[f]);
-          else acc[f] += fabs(d0);
-        }
-      }
-    }
-    if (ci == n_chunks - 1) {
-      const int64_t r = row_of(g, lane);
-      if (r >= 0) {
-#pragma unroll
-        for (int f = 0; f < NQ; ++f) {
-          double key;
-          if (METRIC == RBOD_COSINE) {
-            const double den = qn_s[f] * sqrt(gg);
-            key = den > 0.0 ? acc[f] / den : 0.0;        // the formula of cosine_similarity, 33_…py:76-77
-          } else if (METRIC == RBOD_DOT) {
-            key = acc[f];
-          } else {
-            key = -acc[f];
-          }
-          // thr_s is +inf for slots beyond the batch and for finished queries; a list that overflowed was tightened to
-          // the k-th best (key, row) pair it had recorded, so a cluster of duplicates wider than the list resolves to
-          // its smallest row slots instead of overflowing for ever
-          // per-query masks (slot_mask != nullptr): a row slot f's mask excludes is never recorded for it
-          if ((key > thr_s[f] || (key == thr_s[f] && (uint32_t)r <= thr_row_s[f])) &&
-              (mask_s[f] < 0 || ((row_mask[(int64_t)mask_s[f] * mask_words + (r >> 5)] >> (r & 31)) & 1u))) {
-            const int slot = atomicAdd(coll_cnt + f, 1);
-            if (slot < cap) {
-              coll_key[(size_t)f * cap + slot] = key;
-              coll_idx[(size_t)f * cap + slot] = (uint32_t)r;
-            }
-          }
-        }
-      }
-    }
-    __syncthreads();   // everyone is done with buffer b before the copy of step + 2 lands in it
-  }
+key_collect_kernel(const double* __restrict__ q64, const float* __restrict__ master32,
+                   const uint16_t* __restrict__ rows16, int kind16, int dim, int64_t ld32, int64_t ld16,
+                   int64_t n_rows, int64_t row0, int64_t stride, const uint32_t* __restrict__ row_mask,
+                   int64_t mask_words, const int* __restrict__ slot_tab, const int* __restrict__ req_mask,
+                   const double* __restrict__ thr, const uint32_t* __restrict__ thr_row,
+                   const int* __restrict__ active, const double* __restrict__ qnorm, int n_slots, int n_req, int cap,
+                   double* __restrict__ coll_key, uint32_t* __restrict__ coll_idx, int* __restrict__ coll_cnt) {
+  slot_sweep<METRIC, NS, KeyRow>(q64, master32, rows16, kind16, dim, ld32, ld16, n_rows, row0, stride, row_mask,
+                                 mask_words, slot_tab, req_mask, thr, thr_row, active, qnorm, n_slots, n_req, cap,
+                                 coll_key, coll_idx, coll_cnt);
 }
 
 // Monotone map double -> uint64 (larger double <=> larger key).
@@ -307,40 +159,20 @@ int launch_dist_widen_queries(const float* q, const int* qsel, int nf, int dim, 
   return RBOD_OK;
 }
 
-int launch_dist_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
-                        int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride,
-                        const uint32_t* row_mask, int64_t mask_words, const int* slot_mask, const double* thr,
-                        const uint32_t* thr_row, const int* active, const double* qnorm, int nf, int cap,
-                        double* coll_key, uint32_t* coll_idx, int* coll_cnt, int num_sms, cudaStream_t st) {
-  if (nf <= 0 || n_rows <= 0) return RBOD_OK;
-  if (nf > 32) return set_error(RBOD_E_INVAL, "dist_collect: at most 32 queries per pass");
-  const int64_t rows_visited = (n_rows - row0 + stride - 1) / stride;
-  const int64_t groups = (rows_visited + K5_ROWS - 1) / K5_ROWS;
-  const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(groups, (int64_t)num_sms));
-  const int pitch = (master32 ? K5_CH : K5_CH / 2) + 1;
-#define RBOD_K5_GO(METRIC, NQ)                                                                                 \
-  do {                                                                                                         \
-    const size_t smem = (size_t)2 * NQ * K5_CH * 8 + (size_t)2 * 8 * 32 * pitch * 4;                           \
-    RBOD_CUDA(cudaFuncSetAttribute(dist_collect_kernel<METRIC, NQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                   (int)smem));                                                                \
-    dist_collect_kernel<METRIC, NQ><<<grid, 256, smem, st>>>(q64, master32, rows16, kind16, dim, ld32, ld16,    \
-                                                             n_rows, row0, stride, row_mask, mask_words,       \
-                                                             slot_mask, thr, thr_row, active,                  \
-                                                             qnorm, nf, cap, coll_key, coll_idx, coll_cnt);    \
-  } while (0)
-  // 8 accumulators per lane for batches of up to 8 queries (single-query searches of the scripts), 32 otherwise
-  if (metric == RBOD_EUCLID) {
-    if (nf <= 8) RBOD_K5_GO(RBOD_EUCLID, 8); else RBOD_K5_GO(RBOD_EUCLID, 32);
-  } else if (metric == RBOD_MANHATTAN) {
-    if (nf <= 8) RBOD_K5_GO(RBOD_MANHATTAN, 8); else RBOD_K5_GO(RBOD_MANHATTAN, 32);
-  } else if (metric == RBOD_DOT) {
-    if (nf <= 8) RBOD_K5_GO(RBOD_DOT, 8); else RBOD_K5_GO(RBOD_DOT, 32);
-  } else {
-    if (nf <= 8) RBOD_K5_GO(RBOD_COSINE, 8); else RBOD_K5_GO(RBOD_COSINE, 32);
-  }
-#undef RBOD_K5_GO
-  RBOD_CUDA(cudaGetLastError());
-  return RBOD_OK;
+int launch_key_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
+                       int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride,
+                       const uint32_t* row_mask, int64_t mask_words, const int* slot_tab, const int* req_mask,
+                       const double* thr, const uint32_t* thr_row, const int* active, const double* qnorm,
+                       int n_slots, int n_req, int cap, double* coll_key, uint32_t* coll_idx, int* coll_cnt,
+                       int num_sms, cudaStream_t st) {
+  static const SlotKernel kernels[4][2] = {
+      {key_collect_kernel<RBOD_COSINE, 8>, key_collect_kernel<RBOD_COSINE, 32>},
+      {key_collect_kernel<RBOD_DOT, 8>, key_collect_kernel<RBOD_DOT, 32>},
+      {key_collect_kernel<RBOD_EUCLID, 8>, key_collect_kernel<RBOD_EUCLID, 32>},
+      {key_collect_kernel<RBOD_MANHATTAN, 8>, key_collect_kernel<RBOD_MANHATTAN, 32>}};
+  return launch_slot_kernel(kernels, "key_collect", metric, q64, master32, rows16, kind16, dim, ld32, ld16, n_rows,
+                            row0, stride, row_mask, mask_words, slot_tab, req_mask, thr, thr_row, active, qnorm,
+                            n_slots, n_req, cap, coll_key, coll_idx, coll_cnt, num_sms, st);
 }
 
 int launch_dist_select(const double* coll_key, const uint32_t* coll_idx, int* coll_cnt, const int* qsel, int nf,

@@ -9,9 +9,9 @@
 //
 // K is larger-is-better for every metric, so the selection is K5's (key desc, row asc) with K as the key: the sample
 // pass, the threshold sweep, the tightening of an overflowing list and the final sort are K5's, through its launchers
-// (launch_dist_widen_queries widens the examples, launch_dist_select sorts the per-request lists).  Only the collecting
-// kernel differs: K5 records one key per slot, K6 folds a request's slots into one K before it records.  Its row loop is
-// slot_sweep (rbod_slot_sweep.cuh, shared with K7); the end of a row is RecoRow below.
+// (launch_dist_widen_queries widens the examples, launch_dist_select sorts the per-request lists) and its host loop.
+// Only the end of a row differs: K5 records one key per slot, K6 folds a request's slots into one K before it records.
+// The row loop is slot_sweep (rbod_slot_sweep.cuh, shared with K5 and K7); the end of a row is RecoRow below.
 #include "rbod_slot_sweep.cuh"
 
 namespace rbod {
@@ -21,6 +21,7 @@ namespace {
 // End of a row: a running bp / bn over the request's slots; SLOT_NEG marks a negative example.
 template <int METRIC>
 struct RecoRow {
+  static constexpr bool kSlotIsRequest = false;
   double bp = -INFINITY, bn = -INFINITY;
   __device__ __forceinline__ void fold(int tab, double key) {
     if (tab & SLOT_NEG) bn = fmax(bn, key); else bp = fmax(bp, key);

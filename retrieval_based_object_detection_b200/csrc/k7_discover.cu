@@ -7,9 +7,9 @@
 //   discovery (a target):  K = sum rank_pair + s(sim(key(t, g)))
 //   context (no target):   K = sum loss_pair, summed in pair order
 //
-// K is larger-is-better for every metric, so the selection, the sample pass, the sweep and the tightening are K6's
-// (rbod_api.cu: example_sweep); the row loop is slot_sweep (rbod_slot_sweep.cuh).  Only the end of a row differs:
-// DiscRow below.
+// K is larger-is-better for every metric, so the selection, the sample pass, the sweep and the tightening are K5's and
+// K6's (rbod_api.cu: sweep); the row loop is slot_sweep (rbod_slot_sweep.cuh).  Only the end of a row differs: DiscRow
+// below.
 #include "rbod_slot_sweep.cuh"
 
 namespace rbod {
@@ -22,6 +22,7 @@ __device__ __forceinline__ double disc_f(double y) { return y / (1.0 + fabs(y));
 // rank and loss; the request's last slot picks its score by SLOT_DISC.
 template <int METRIC>
 struct DiscRow {
+  static constexpr bool kSlotIsRequest = false;
   double t = 0.0, p = 0.0, loss = 0.0;
   int rank = 0;
   __device__ __forceinline__ void fold(int tab, double key) {

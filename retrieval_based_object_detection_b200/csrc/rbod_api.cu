@@ -729,8 +729,8 @@ struct K3Sample {
 };
 
 // Row masks of one search.  `dev`: [n_masks][words] bitmasks on the device, nullptr = no filter.  `of_query`: the mask
-// each query row of the K3 launch reads ([q_pad] on the device, -1 = none) and `of_query_host` the same ids by original
-// query index ([Q] on the host, read by the sweep's batch control); both nullptr = every query reads mask 0.
+// each query row of the K3 launch reads ([q_pad] on the device, -1 = none) and `of_query_host` the same ids by query (or
+// request) index ([Q] on the host, read by the sweep's batch control); both nullptr = every query reads mask 0.
 struct SearchMasks {
   const uint32_t* dev;
   int64_t words;
@@ -861,172 +861,191 @@ static int prepare_queries(rbod_gallery* g, const float* queries, int64_t Q, con
                              g->q_dq.as<float>(), g->q_qq.as<double>(), g->tau_shared.as<uint32_t>(), st);
 }
 
-// Exact fp64 sweep (kernel K5), 32 queries per pass over the gallery: answers the n queries of q_dev (device, [*, dim]
-// fp32) listed in the host array qsel -- queries 0..n-1 if it is null -- in their rows q * k of the outputs.  kth (host,
-// one per listed query, or null) is each query's provisional k-th key, -inf if it had fewer than k candidates: a
-// lower bound of the true k-th key that replaces the sample pass as the starting threshold.
-static int sweep_exact(rbod_gallery* g, const float* q_dev, int64_t n, const int* qsel, const double* kth, int k,
-                       const SearchMasks& M, float* d_scores, int64_t* d_rows, double* d_keys, int64_t* launches,
-                       int64_t* resweeps, cudaStream_t st) {
+// A call's answer, n entries each of fp32 scores, rows and fp64 keys (keys optional): the caller's arrays, and where
+// the kernels write them -- the caller's array when it is device memory, else the handle's out_* workspace.
+struct Answer {
+  float* scores;
+  int64_t* rows;
+  double* keys;
+  float* d_scores;
+  int64_t* d_rows;
+  double* d_keys;
+  size_t n;
+};
+
+static int stage_answer(rbod_gallery* g, float* scores, int64_t* rows, double* keys, size_t n, Answer* a) {
+  RBOD_TRY(g->out_scores.ensure(n * 4));
+  RBOD_TRY(g->out_rows.ensure(n * 8));
+  RBOD_TRY(g->out_scores64.ensure(n * 8));
+  *a = {scores, rows, keys, is_device_ptr(scores) ? scores : g->out_scores.as<float>(),
+        is_device_ptr(rows) ? rows : g->out_rows.as<int64_t>(),
+        (keys && is_device_ptr(keys)) ? keys : g->out_scores64.as<double>(), n};
+  return RBOD_OK;
+}
+
+// Queues the copy of a staged answer into the caller's arrays (where they are not the same).
+static int copy_out(const Answer& a, cudaStream_t st) {
+  RBOD_TRY(copy_out(a.scores, a.d_scores, a.n * 4, st));
+  RBOD_TRY(copy_out(a.rows, a.d_rows, a.n * 8, st));
+  return copy_out(a.keys, a.d_keys, a.n * 8, st);
+}
+
+// The answer of an empty gallery, written straight to the caller's arrays: every entry is "no result" -- row -1, key
+// -inf, score -inf, or +inf where `metric` ranks by distance (as dist_select_kernel pads a short list).
+static int answer_none(float* scores, int64_t* rows, double* keys, size_t n, int metric, cudaStream_t st) {
+  std::vector<float> hs(n, (metric == RBOD_EUCLID || metric == RBOD_MANHATTAN) ? INFINITY : -INFINITY);
+  std::vector<int64_t> hr(n, -1);
+  std::vector<double> hd(n, -INFINITY);
+  RBOD_CUDA(cudaMemcpyAsync(scores, hs.data(), n * 4, cudaMemcpyDefault, st));
+  RBOD_CUDA(cudaMemcpyAsync(rows, hr.data(), n * 8, cudaMemcpyDefault, st));
+  if (keys) RBOD_CUDA(cudaMemcpyAsync(keys, hd.data(), n * 8, cudaMemcpyDefault, st));
+  RBOD_CUDA(cudaStreamSynchronize(st));
+  return RBOD_OK;
+}
+
+// The per-item mask ids of a filtered call (n of them, in host or device memory), read to the host and checked before
+// anything is launched: each must be -1 (no mask) or one of the n_masks masks; `fmt` reports the first that is not,
+// from (who, its index, its value, n_masks).  `ids` stays empty without ids, and without masks (all ids are -1 then).
+static int read_mask_ids(const char* who, const char* fmt, rbod_gallery* g, const int32_t* src, int64_t n,
+                         int32_t n_masks, cudaStream_t st, std::vector<int>* ids) {
+  if (src == nullptr || n <= 0) return RBOD_OK;
+  ids->resize((size_t)n);
+  if (is_device_ptr(src)) {
+    if (!g) return set_error(RBOD_E_INVAL, "%s: NULL handle", who);
+    RBOD_CUDA(cudaSetDevice(g->device));
+    RBOD_CUDA(cudaMemcpyAsync(ids->data(), src, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+    RBOD_CUDA(cudaStreamSynchronize(st));
+  } else {
+    memcpy(ids->data(), src, (size_t)n * 4);
+  }
+  for (int64_t i = 0; i < n; ++i)
+    if ((*ids)[i] < -1 || (*ids)[i] >= n_masks) return set_error(RBOD_E_INVAL, fmt, who, (long long)i, (*ids)[i], n_masks);
+  if (n_masks == 0) ids->clear();
+  return RBOD_OK;
+}
+
+// Exact fp64 sweep (kernels K5 search, K6 recommend, K7 discover): requests are packed whole, in order, into passes of
+// at most 32 slots and 32 requests.  Request r is the examples off[r] .. off[r + 1] - 1 of ex_dev ([*, dim] fp32, on
+// the device) or, without offsets, the one example sel[r] (host; r when sel is null).  It answers into rows o * k of
+// a's device arrays, o = sel[r] (or r), its slots carry the flags of its examples (rbod_internal.h; none when flags is
+// null), and it reads the mask M.of_query_host[o] -- or mask 0 when M has masks but no ids, and then the rows mask 0
+// excludes are not even loaded.  Per pass a strided sample pass gives every request its starting threshold, unless kth
+// does (host, one per request, or null: a provisional k-th key, -inf if there were fewer than k candidates, a lower
+// bound of the true k-th key); then the gallery is swept, and the requests whose list overflowed are tightened and
+// swept again.  Nothing a request's answer depends on (its slots' accumulators, its threshold, its list, its mask) is
+// shared with another request of the pass, so the packing does not change any answer.  collect: the kernel's
+// launcher; metric: what the selection is given -- the gallery's for a search, which turns keys into distances, COSINE
+// for K6 / K7, which emits the score as it is and pads with -inf; who: the entry point named in errors, kth_of: what a
+// list overflows around in them ("key of a query", "score of a request").
+static int sweep(rbod_gallery* g, const char* who, const char* kth_of, CollectLauncher collect, int metric,
+                 const float* ex_dev, const int* flags, const int64_t* off, const int* sel, int64_t R, const double* kth,
+                 int k, const SearchMasks& M, const Answer& a, int64_t* launches, int64_t* resweeps, cudaStream_t st) {
   // lists hold 8192 rows and so does the sample: ~k * stride rows pass the threshold it yields (1M rows, k = 10:
   // ~1200), so one sweep is enough unless k * rows / 8192 exceeds a list (then a second sweep with the tightened
   // threshold finishes it)
   const int cap = 8192, sample_cap = 8192, batch = 32, max_iter = 12;
-  if (k > 1024)
-    return set_error(RBOD_E_UNSUPPORTED, "rbod_search: k=%d > 1024", k);
+  if (k > 1024) return set_error(RBOD_E_UNSUPPORTED, "%s: k=%d > 1024", who, k);
   RBOD_TRY(g->dist_q64.ensure((size_t)batch * g->dim * 8));
-  RBOD_TRY(g->dist_thr.ensure((size_t)2 * batch * 8 + (size_t)batch * 4));   // thresholds, query norms, row bounds
-  RBOD_TRY(g->dist_ctl.ensure((size_t)(3 * batch + 1) * 4));
-  RBOD_TRY(g->coll_score.ensure((size_t)batch * cap * 8));
-  RBOD_TRY(g->coll_idx.ensure((size_t)batch * cap * 4));
-  RBOD_TRY(g->coll_cnt.ensure((size_t)batch * 4));
-  int* d_qsel = g->dist_ctl.as<int>();
-  int* d_active = d_qsel + batch;
-  int* d_nactive = d_qsel + 2 * batch;
-  const bool per_query = M.dev != nullptr && M.of_query_host != nullptr;
-  const int* d_slot_mask = per_query ? d_qsel + 2 * batch + 1 : nullptr;   // the mask each slot of the batch reads
-  double* d_thr = g->dist_thr.as<double>();
-  double* d_qnorm = d_thr + batch;
-  uint32_t* d_thr_row = reinterpret_cast<uint32_t*>(d_qnorm + batch);
-  std::vector<double> h_thr(batch, -INFINITY);
-  std::vector<int> h_ctl(3 * batch + 1, -1);
-  const int64_t sample_stride = (g->rows + sample_cap - 1) / sample_cap;   // > 1 iff more than `sample_cap` rows
-  for (int64_t q0 = 0; q0 < n; q0 += batch) {
-    const int nf = (int)std::min<int64_t>(batch, n - q0);
-    for (int f = 0; f < batch; ++f) {
-      const int64_t i = q0 + std::min(f, nf - 1);
-      h_ctl[f] = qsel ? qsel[i] : (int)i;
-      h_ctl[batch + f] = f < nf ? 1 : 0;
-      if (per_query) h_ctl[2 * batch + 1 + f] = f < nf ? M.of_query_host[h_ctl[f]] : -1;
-      // kth was summed in another order than this sweep sums, so the very row that set it may come out an ulp lower
-      // here: seed a margin far above fp64 summation noise below it (-inf stays -inf)
-      if (kth) h_thr[f] = kth[i] - 1e-12 * std::max(1.0, std::fabs(kth[i]));
-    }
-    h_ctl[2 * batch] = 0;
-    RBOD_CUDA(cudaMemcpyAsync(d_qsel, h_ctl.data(), h_ctl.size() * 4, cudaMemcpyHostToDevice, st));
-    RBOD_CUDA(cudaMemcpyAsync(d_thr, h_thr.data(), (size_t)batch * 8, cudaMemcpyHostToDevice, st));
-    RBOD_CUDA(cudaMemsetAsync(d_thr_row, 0xff, (size_t)batch * 4, st));   // no row bound: every tie with the threshold counts
-    RBOD_CUDA(cudaMemsetAsync(g->coll_cnt.p, 0, (size_t)batch * 4, st));
-    if (nf < batch) RBOD_CUDA(cudaMemsetAsync(g->dist_q64.p, 0, (size_t)batch * g->dim * 8, st));   // zero rows pad the batch
-    RBOD_TRY(launch_dist_widen_queries(q_dev, d_qsel, nf, g->dim, g->dist_q64.as<double>(), d_qnorm, st));
-    ++*launches;
-    if (!kth && sample_stride > 1) {
-      RBOD_TRY(launch_dist_collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim,
-                                   g->dim, g->dp, g->rows, 0, sample_stride, M.dev, M.words, d_slot_mask, d_thr, d_thr_row,
-                                   d_active, d_qnorm, nf, cap,
-                                   g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
-                                   g->num_sms, st));
-      RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
-                                  d_qsel, nf, cap, k, 1, g->metric, d_thr, d_thr_row, d_active, d_nactive, d_scores, d_rows,
-                                  d_keys, st));
-      *launches += 2;
-    }
-    int iter = 0, left = nf;
-    for (; iter < max_iter && left > 0; ++iter) {
-      RBOD_CUDA(cudaMemsetAsync(d_nactive, 0, 4, st));
-      RBOD_TRY(launch_dist_collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim,
-                                   g->dim, g->dp, g->rows, 0, 1, M.dev, M.words, d_slot_mask, d_thr, d_thr_row, d_active,
-                                   d_qnorm, nf, cap,
-                                   g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
-                                   g->num_sms, st));
-      RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
-                                  d_qsel, nf, cap, k, 0, g->metric, d_thr, d_thr_row, d_active, d_nactive, d_scores, d_rows,
-                                  d_keys, st));
-      *launches += 2;
-      RBOD_CUDA(cudaMemcpyAsync(&left, d_nactive, 4, cudaMemcpyDeviceToHost, st));
-      RBOD_CUDA(cudaStreamSynchronize(st));
-      if (iter > 0) ++*resweeps;
-    }
-    if (left > 0)
-      return set_error(RBOD_E_OVERFLOW, "rbod_search: more than %d rows tie around the k-th key of a query", cap);
-  }
-  return RBOD_OK;
-}
-
-// Exact example-based search (kernels K6 recommend, K7 discover), the same loop as sweep_exact over requests instead of
-// queries: requests are packed whole, in order, into passes of at most 32 example slots and 32 requests.  Per pass a
-// strided sample pass gives every request its starting threshold, then the gallery is swept, and the requests whose
-// list overflowed are tightened and swept again.  Request r's answer goes to rows r * k of the outputs.  Nothing a
-// request's answer depends on (its slots' accumulators, its threshold, its list, its mask) is shared with another
-// request of the pass, so the packing does not change any answer.  ex_dev: [E, dim] fp32 examples on the device;
-// flags: [E] the examples' slot-table flags (rbod_internal.h), off / mask_of_req: host.  collect: the kernel's launcher,
-// who: the entry point named in errors.
-static int example_sweep(rbod_gallery* g, CollectLauncher collect, const char* who, const float* ex_dev,
-                         const int* flags, const int64_t* off, int64_t R, int k, const SearchMasks& M,
-                         const int* mask_of_req, float* d_scores, int64_t* d_rows, double* d_keys, int64_t* launches,
-                         int64_t* resweeps, cudaStream_t st) {
-  const int cap = 8192, sample_cap = 8192, batch = 32, max_iter = 12;
-  RBOD_TRY(g->dist_q64.ensure((size_t)batch * g->dim * 8));
-  RBOD_TRY(g->dist_thr.ensure((size_t)2 * batch * 8 + (size_t)batch * 4));   // thresholds, example norms, row bounds
+  RBOD_TRY(g->dist_thr.ensure((size_t)2 * batch * 8 + (size_t)batch * 4));   // thresholds, slot norms, row bounds
   RBOD_TRY(g->dist_ctl.ensure((size_t)(5 * batch + 1) * 4));
   RBOD_TRY(g->coll_score.ensure((size_t)batch * cap * 8));
   RBOD_TRY(g->coll_idx.ensure((size_t)batch * cap * 4));
   RBOD_TRY(g->coll_cnt.ensure((size_t)batch * 4));
   int* d_wsel = g->dist_ctl.as<int>();   // slot -> example (what the widening reads)
   int* d_slot = d_wsel + batch;           // slot table of the pass (rbod_internal.h)
-  int* d_req = d_wsel + 2 * batch;        // request of the pass -> request of the call (the output row)
+  int* d_out = d_wsel + 2 * batch;        // request of the pass -> its output row
   int* d_active = d_wsel + 3 * batch;
   int* d_rmask = d_wsel + 4 * batch;      // the mask each request of the pass reads, -1 = none
   int* d_nactive = d_wsel + 5 * batch;
+  const bool per_request = M.dev != nullptr && M.of_query_host != nullptr;
   double* d_thr = g->dist_thr.as<double>();
   double* d_qnorm = d_thr + batch;
   uint32_t* d_thr_row = reinterpret_cast<uint32_t*>(d_qnorm + batch);
-  const std::vector<double> h_thr(batch, -INFINITY);
+  std::vector<double> h_thr(batch, -INFINITY);
   std::vector<int> h_ctl(5 * batch + 1);
   const int64_t sample_stride = (g->rows + sample_cap - 1) / sample_cap;   // > 1 iff more than `sample_cap` rows
+  auto n_slots = [&](int64_t r) { return off ? (int)(off[r + 1] - off[r]) : 1; };
   for (int64_t r0 = 0; r0 < R;) {
     int nreq = 0, ns = 0;
-    while (r0 + nreq < R && nreq < batch && ns + (off[r0 + nreq + 1] - off[r0 + nreq]) <= batch) {
-      ns += (int)(off[r0 + nreq + 1] - off[r0 + nreq]);
-      ++nreq;
-    }
+    for (; r0 + nreq < R && nreq < batch && ns + n_slots(r0 + nreq) <= batch; ++nreq) ns += n_slots(r0 + nreq);
     std::fill(h_ctl.begin(), h_ctl.end(), 0);
-    for (int s = 0; s < batch; ++s) h_ctl[s] = (int)(off[r0] + std::min(s, ns - 1));
-    for (int q = 0; q < nreq; ++q) {
-      const int64_t e0 = off[r0 + q], e1 = off[r0 + q + 1];
-      for (int64_t e = e0; e < e1; ++e)
-        h_ctl[batch + (int)(e - off[r0])] = q | (e == e1 - 1 ? SLOT_LAST : 0) | flags[e];
-      h_ctl[2 * batch + q] = (int)(r0 + q);
+    for (int q = 0, s = 0; q < nreq; ++q) {
+      const int64_t r = r0 + q, o = sel ? sel[r] : r;
+      const int64_t e0 = off ? off[r] : o, e1 = off ? off[r + 1] : o + 1;
+      for (int64_t e = e0; e < e1; ++e, ++s) {
+        h_ctl[s] = (int)e;
+        h_ctl[batch + s] = q | (e == e1 - 1 ? SLOT_LAST : 0) | (flags ? flags[e] : 0);
+      }
+      h_ctl[2 * batch + q] = (int)o;
       h_ctl[3 * batch + q] = 1;
-      h_ctl[4 * batch + q] = (M.dev != nullptr && mask_of_req != nullptr) ? mask_of_req[r0 + q] : -1;
+      h_ctl[4 * batch + q] = per_request ? M.of_query_host[o] : -1;
+      // kth was summed in another order than this sweep sums, so the very row that set it may come out an ulp lower
+      // here: seed a margin far above fp64 summation noise below it (-inf stays -inf)
+      if (kth) h_thr[q] = kth[r] - 1e-12 * std::max(1.0, std::fabs(kth[r]));
     }
     RBOD_CUDA(cudaMemcpyAsync(d_wsel, h_ctl.data(), h_ctl.size() * 4, cudaMemcpyHostToDevice, st));
     RBOD_CUDA(cudaMemcpyAsync(d_thr, h_thr.data(), (size_t)batch * 8, cudaMemcpyHostToDevice, st));
-    RBOD_CUDA(cudaMemsetAsync(d_thr_row, 0xff, (size_t)batch * 4, st));
+    RBOD_CUDA(cudaMemsetAsync(d_thr_row, 0xff, (size_t)batch * 4, st));   // no row bound: every tie with the threshold counts
     RBOD_CUDA(cudaMemsetAsync(g->coll_cnt.p, 0, (size_t)batch * 4, st));
-    if (ns < batch) RBOD_CUDA(cudaMemsetAsync(g->dist_q64.p, 0, (size_t)batch * g->dim * 8, st));
+    if (ns < batch) RBOD_CUDA(cudaMemsetAsync(g->dist_q64.p, 0, (size_t)batch * g->dim * 8, st));   // zero rows pad the pass
     RBOD_TRY(launch_dist_widen_queries(ex_dev, d_wsel, ns, g->dim, g->dist_q64.as<double>(), d_qnorm, st));
     ++*launches;
-    // the K5 selection ranks by the key it is given; metric COSINE emits that key as the score and pads with -inf,
-    // which is what K (larger is better for every metric) needs
-    if (sample_stride > 1) {
+    // one collecting pass over the rows 0, stride, 2 stride, ... and the selection of its lists
+    auto collect_select = [&](int64_t stride, int sample) {
       RBOD_TRY(collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim, g->dim, g->dp,
-                       g->rows, 0, sample_stride, M.dev, M.words, d_slot, d_rmask, d_thr, d_thr_row, d_active, d_qnorm,
-                       ns, nreq, cap, g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
-                       g->num_sms, st));
-      RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
-                                  d_req, nreq, cap, k, 1, RBOD_COSINE, d_thr, d_thr_row, d_active, d_nactive, d_scores,
-                                  d_rows, d_keys, st));
+                       g->rows, 0, stride, M.dev, M.words, d_slot, per_request ? d_rmask : nullptr, d_thr, d_thr_row,
+                       d_active, d_qnorm, ns, nreq, cap, g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(),
+                       g->coll_cnt.as<int>(), g->num_sms, st));
+      RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(), d_out,
+                                  nreq, cap, k, sample, metric, d_thr, d_thr_row, d_active, d_nactive, a.d_scores,
+                                  a.d_rows, a.d_keys, st));
       *launches += 2;
-    }
+      return RBOD_OK;
+    };
+    if (!kth && sample_stride > 1) RBOD_TRY(collect_select(sample_stride, 1));
     int iter = 0, left = nreq;
     for (; iter < max_iter && left > 0; ++iter) {
       RBOD_CUDA(cudaMemsetAsync(d_nactive, 0, 4, st));
-      RBOD_TRY(collect(g->metric, g->dist_q64.as<double>(), g->master32, g->rows16, g->kind16, g->dim, g->dim, g->dp,
-                       g->rows, 0, 1, M.dev, M.words, d_slot, d_rmask, d_thr, d_thr_row, d_active, d_qnorm, ns, nreq,
-                       cap, g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(), g->num_sms,
-                       st));
-      RBOD_TRY(launch_dist_select(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
-                                  d_req, nreq, cap, k, 0, RBOD_COSINE, d_thr, d_thr_row, d_active, d_nactive, d_scores,
-                                  d_rows, d_keys, st));
-      *launches += 2;
+      RBOD_TRY(collect_select(1, 0));
       RBOD_CUDA(cudaMemcpyAsync(&left, d_nactive, 4, cudaMemcpyDeviceToHost, st));
       RBOD_CUDA(cudaStreamSynchronize(st));
       if (iter > 0) ++*resweeps;
     }
     if (left > 0)
-      return set_error(RBOD_E_OVERFLOW, "%s: more than %d rows tie around the k-th score of a request", who, cap);
+      return set_error(RBOD_E_OVERFLOW, "%s: more than %d rows tie around the k-th %s", who, cap, kth_of);
     r0 += nreq;
+  }
+  return RBOD_OK;
+}
+
+// The exact sweep's front end, past the entry point's argument checks: rbod_search / rbod_search_masks (what the
+// tensor-core pass does not cover), rbod_recommend and rbod_discover.  The answer of an empty gallery, or: the outputs
+// staged, the masks and the examples uploaded, the sweep, the copy-out and the stats.  ids: the checked host mask ids,
+// one per request, or null (every request reads mask 0, if there are masks).
+static int sweep_search(rbod_gallery* g, const char* who, const char* kth_of, CollectLauncher collect, int metric,
+                        const float* examples,
+                        int64_t n_examples, const int* flags, const int64_t* off, int64_t R, int k,
+                        const uint32_t* row_masks, int32_t n_masks, const int* ids, float* out_scores,
+                        int64_t* out_rows, double* out_keys, rbod_search_stats* stats, cudaStream_t st) {
+  Answer a;
+  RBOD_TRY(stage_answer(g, out_scores, out_rows, out_keys, (size_t)R * k, &a));
+  if (g->rows == 0) return answer_none(out_scores, out_rows, out_keys, a.n, metric, st);
+  SearchMasks M = {nullptr, (g->rows + 31) / 32, nullptr, ids};
+  const void* md = nullptr;
+  if (n_masks > 0) RBOD_TRY(to_device(row_masks, (size_t)n_masks * M.words * 4, g->mask_dev, st, &md));
+  M.dev = static_cast<const uint32_t*>(md);
+  const void* xd = nullptr;
+  RBOD_TRY(to_device(examples, (size_t)n_examples * g->dim * 4, g->q32, st, &xd));
+  int64_t launches = 0, resweeps = 0;
+  RBOD_TRY(sweep(g, who, kth_of, collect, metric, static_cast<const float*>(xd), flags, off, nullptr, R, nullptr, k, M,
+                 a, &launches, &resweeps, st));
+  RBOD_TRY(copy_out(a, st));
+  RBOD_CUDA(cudaStreamSynchronize(st));
+  if (stats) {
+    stats->queries = R;
+    stats->total_launches = launches;
+    stats->sweep_queries = R;        // every query or request is answered by the fp64 sweep
+    stats->fallback_queries = resweeps;
   }
   return RBOD_OK;
 }
@@ -1167,77 +1186,22 @@ static int search_impl(rbod_gallery* g, const float* queries, int64_t Q, int32_t
   if (g->rows >= 0xffffffffll) return set_error(RBOD_E_UNSUPPORTED, "rbod_search: more than 2^32-2 rows per shard");
   RBOD_CUDA(cudaSetDevice(g->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  std::vector<int> ids_h;
+  RBOD_TRY(read_mask_ids("rbod_search_masks", "%s: mask_of_query[%lld] = %d is outside [-1, %d)", g, mask_of_query, Q,
+                         n_masks, st, &ids_h));
+  const int* ids = ids_h.empty() ? nullptr : ids_h.data();
 
-  // Per-query mask ids are checked on the host before anything is launched; the sweep's batch control reads them there
-  // too.  Without masks every id is -1: a plain search.
-  std::vector<int> ids_host;
-  if (mask_of_query != nullptr) {
-    ids_host.resize((size_t)Q);
-    if (is_device_ptr(mask_of_query)) {
-      RBOD_CUDA(cudaMemcpyAsync(ids_host.data(), mask_of_query, (size_t)Q * 4, cudaMemcpyDeviceToHost, st));
-      RBOD_CUDA(cudaStreamSynchronize(st));
-    } else {
-      memcpy(ids_host.data(), mask_of_query, (size_t)Q * 4);
-    }
-    for (int64_t q = 0; q < Q; ++q)
-      if (ids_host[q] < -1 || ids_host[q] >= n_masks)
-        return set_error(RBOD_E_INVAL, "rbod_search_masks: mask_of_query[%lld] = %d is outside [-1, %d)", (long long)q,
-                         ids_host[q], n_masks);
-    if (n_masks == 0) ids_host.clear();
-  }
-  SearchMasks M = {nullptr, (g->rows + 31) / 32, nullptr, ids_host.empty() ? nullptr : ids_host.data()};
-
-  if (distance_metric) {
-    const size_t n_out = (size_t)Q * k;
-    RBOD_TRY(g->out_scores.ensure(n_out * 4));
-    RBOD_TRY(g->out_rows.ensure(n_out * 8));
-    RBOD_TRY(g->out_scores64.ensure(n_out * 8));
-    float* ds = is_device_ptr(out_scores) ? out_scores : g->out_scores.as<float>();
-    int64_t* dr = is_device_ptr(out_rows) ? out_rows : g->out_rows.as<int64_t>();
-    double* dk = (out_scores64 && is_device_ptr(out_scores64)) ? out_scores64 : g->out_scores64.as<double>();
-    if (g->rows == 0) {
-      std::vector<float> hs(n_out, (g->metric == RBOD_EUCLID || g->metric == RBOD_MANHATTAN) ? INFINITY : -INFINITY);
-      std::vector<int64_t> hr(n_out, -1);
-      std::vector<double> hd(n_out, -INFINITY);
-      RBOD_CUDA(cudaMemcpyAsync(out_scores, hs.data(), n_out * 4, cudaMemcpyDefault, st));
-      RBOD_CUDA(cudaMemcpyAsync(out_rows, hr.data(), n_out * 8, cudaMemcpyDefault, st));
-      if (out_scores64) RBOD_CUDA(cudaMemcpyAsync(out_scores64, hd.data(), n_out * 8, cudaMemcpyDefault, st));
-      RBOD_CUDA(cudaStreamSynchronize(st));
-      return RBOD_OK;
-    }
-    const void* md = nullptr;
-    if (n_masks > 0) RBOD_TRY(to_device(row_masks, (size_t)n_masks * M.words * 4, g->mask_dev, st, &md));
-    M.dev = static_cast<const uint32_t*>(md);
-    const void* qd = nullptr;
-    RBOD_TRY(to_device(queries, (size_t)Q * g->dim * 4, g->q32, st, &qd));
-    int64_t n_launch = 0, resweeps = 0;
-    RBOD_TRY(sweep_exact(g, static_cast<const float*>(qd), Q, nullptr, nullptr, k, M, ds, dr, dk, &n_launch, &resweeps,
-                         st));
-    RBOD_TRY(copy_out(out_scores, ds, n_out * 4, st));
-    RBOD_TRY(copy_out(out_rows, dr, n_out * 8, st));
-    if (out_scores64) RBOD_TRY(copy_out(out_scores64, dk, n_out * 8, st));
-    RBOD_CUDA(cudaStreamSynchronize(st));
-    if (stats) {
-      stats->queries = Q;
-      stats->total_launches = n_launch;
-      stats->sweep_queries = Q;        // every query is answered by the exact fp64 sweep
-      stats->fallback_queries = resweeps;
-    }
-    return RBOD_OK;
-  }
+  if (distance_metric)
+    return sweep_search(g, "rbod_search", "key of a query", launch_key_collect, g->metric, queries, Q, nullptr, nullptr,
+                        Q, k, row_masks, n_masks, ids, out_scores, out_rows, out_scores64, stats, st);
 
   const int smem_optin = k3_configure(g->device);
   if (smem_optin < 0) return smem_optin;
 
   RBOD_TRY(maybe_build_shadow(g, k, st));
 
-  const size_t nout = (size_t)Q * k;
-  RBOD_TRY(g->out_scores.ensure(nout * 4));
-  RBOD_TRY(g->out_rows.ensure(nout * 8));
-  RBOD_TRY(g->out_scores64.ensure(nout * 8));
-  float* d_scores = is_device_ptr(out_scores) ? out_scores : g->out_scores.as<float>();
-  int64_t* d_rows = is_device_ptr(out_rows) ? out_rows : g->out_rows.as<int64_t>();
-  double* d_scores64 = (out_scores64 && is_device_ptr(out_scores64)) ? out_scores64 : g->out_scores64.as<double>();
+  Answer a;
+  RBOD_TRY(stage_answer(g, out_scores, out_rows, out_scores64, (size_t)Q * k, &a));
 
   Trace tr;
   SearchPlan P;
@@ -1253,27 +1217,19 @@ static int search_impl(rbod_gallery* g, const float* queries, int64_t Q, int32_t
   int* d_flags = g->flags.as<int>();
   int64_t launches = 0;
 
-  if (g->rows == 0) {
-    // empty collection: every slot is "no result"
-    std::vector<float> hs(nout, g->metric == RBOD_EUCLID ? INFINITY : -INFINITY);
-    std::vector<int64_t> hr(nout, -1);
-    std::vector<double> hd(nout, -INFINITY);
-    RBOD_CUDA(cudaMemcpyAsync(out_scores, hs.data(), nout * 4, cudaMemcpyDefault, st));
-    RBOD_CUDA(cudaMemcpyAsync(out_rows, hr.data(), nout * 8, cudaMemcpyDefault, st));
-    if (out_scores64) RBOD_CUDA(cudaMemcpyAsync(out_scores64, hd.data(), nout * 8, cudaMemcpyDefault, st));
-    RBOD_CUDA(cudaStreamSynchronize(st));
-    return RBOD_OK;
-  }
+  if (g->rows == 0) return answer_none(out_scores, out_rows, out_scores64, a.n, g->metric, st);
 
+  SearchMasks M = {nullptr, (g->rows + 31) / 32, nullptr, ids};
   const void* mask_dev = nullptr;
   if (n_masks > 0) RBOD_TRY(to_device(row_masks, (size_t)n_masks * M.words * 4, g->mask_dev, st, &mask_dev));
   M.dev = static_cast<const uint32_t*>(mask_dev);
-  if (M.of_query_host != nullptr) {
+  std::vector<int> ids_pad;
+  if (ids != nullptr) {
     // the K3 launches read one id per query row of the padded tile: pad rows read no mask
-    ids_host.resize((size_t)P.q_pad, -1);
-    M.of_query_host = ids_host.data();
+    ids_pad.assign(ids, ids + Q);
+    ids_pad.resize((size_t)P.q_pad, -1);
     RBOD_TRY(g->mask_ids.ensure((size_t)P.q_pad * 4));
-    RBOD_CUDA(cudaMemcpyAsync(g->mask_ids.p, ids_host.data(), (size_t)P.q_pad * 4, cudaMemcpyHostToDevice, st));
+    RBOD_CUDA(cudaMemcpyAsync(g->mask_ids.p, ids_pad.data(), (size_t)P.q_pad * 4, cudaMemcpyHostToDevice, st));
     M.of_query = g->mask_ids.as<int>();
   }
 
@@ -1291,16 +1247,14 @@ static int search_impl(rbod_gallery* g, const float* queries, int64_t Q, int32_t
     const float* tau_init = nullptr;
     RBOD_TRY(launch_front(g, queries, Q, P, M, use_sample, sample_tiles, st, &q_dev, &tau_init, &launches, tr));
     FinishArgs F;
-    fill_finish(g, P, k, tau_init, q_dev, d_scores, d_rows, d_scores64, &F);
+    fill_finish(g, P, k, tau_init, q_dev, a.d_scores, a.d_rows, a.d_keys, &F);
     RBOD_TRY(launch_finish(F, Q, st));
     ++launches;
     tr.mark("finish_launch");
 
     // The answer and the certification flags travel together: in the common case (every query certified) this is
     // the only synchronisation of the call.
-    RBOD_TRY(copy_out(out_scores, d_scores, nout * 4, st));
-    RBOD_TRY(copy_out(out_rows, d_rows, nout * 8, st));
-    if (out_scores64) RBOD_TRY(copy_out(out_scores64, d_scores64, nout * 8, st));
+    RBOD_TRY(copy_out(a, st));
     RBOD_CUDA(cudaMemcpyAsync(hflags, d_flags, sizeof(hflags), cudaMemcpyDeviceToHost, st));
     tr.mark("copies");
     RBOD_CUDA(cudaStreamSynchronize(st));
@@ -1349,8 +1303,8 @@ static int search_impl(rbod_gallery* g, const float* queries, int64_t Q, int32_t
                                       g->dp, g->metric, g->flag_q.as<int>(), 0, n_flag, cap, g->coll_idx.as<uint32_t>(),
                                       g->coll_cnt.as<int>(), g->coll_score.as<double>(), st));
     RBOD_TRY(launch_select_collected(g->coll_score.as<double>(), g->coll_idx.as<uint32_t>(), g->coll_cnt.as<int>(),
-                                     g->flag_q.as<int>(), 0, n_flag, cap, k, g->metric, d_scores, d_rows, d_scores64,
-                                     st));
+                                     g->flag_q.as<int>(), 0, n_flag, cap, k, g->metric, a.d_scores, a.d_rows,
+                                     a.d_keys, st));
     launches += 4;
     ++k3_launches;
     RBOD_CUDA(cudaMemcpyAsync(cnt_h.data(), g->coll_cnt.p, (size_t)n_flag * 4, cudaMemcpyDeviceToHost, st));
@@ -1371,13 +1325,11 @@ static int search_impl(rbod_gallery* g, const float* queries, int64_t Q, int32_t
     }
     if (n_sweep > 0) {
       int64_t resweeps = 0;   // not reported: fallback_queries counts the uncertified queries here
-      RBOD_TRY(sweep_exact(g, q_dev, n_sweep, fq_h.data(), thr_h.data(), k, M, d_scores, d_rows, d_scores64, &launches,
-                           &resweeps, st));
+      RBOD_TRY(sweep(g, "rbod_search", "key of a query", launch_key_collect, g->metric, q_dev, nullptr, nullptr,
+                     fq_h.data(), n_sweep, thr_h.data(), k, M, a, &launches, &resweeps, st));
     }
     // the second pass rewrote the flagged queries' rows of the answer
-    RBOD_TRY(copy_out(out_scores, d_scores, nout * 4, st));
-    RBOD_TRY(copy_out(out_rows, d_rows, nout * 8, st));
-    if (out_scores64) RBOD_TRY(copy_out(out_scores64, d_scores64, nout * 8, st));
+    RBOD_TRY(copy_out(a, st));
     RBOD_CUDA(cudaStreamSynchronize(st));
   }
 
@@ -1430,23 +1382,9 @@ int rbod_search_mmr(rbod_gallery* g, const float* queries, int64_t Q, int32_t li
     if (!(diversity[q] >= 0.0 && diversity[q] <= 1.0))
       return set_error(RBOD_E_INVAL, "%s: query %lld: diversity %g is not in [0, 1]", who, (long long)q, diversity[q]);
   // mask ids are checked here, on the host, and handed to the search as a host array
-  std::vector<int32_t> ids;
-  if (mask_of_query && Q > 0) {
-    ids.resize((size_t)Q);
-    if (is_device_ptr(mask_of_query)) {
-      if (!g) return set_error(RBOD_E_INVAL, "%s: NULL handle", who);
-      RBOD_CUDA(cudaSetDevice(g->device));
-      RBOD_CUDA(cudaMemcpyAsync(ids.data(), mask_of_query, (size_t)Q * 4, cudaMemcpyDeviceToHost,
-                                static_cast<cudaStream_t>(stream)));
-      RBOD_CUDA(cudaStreamSynchronize(static_cast<cudaStream_t>(stream)));
-    } else {
-      memcpy(ids.data(), mask_of_query, (size_t)Q * 4);
-    }
-    for (int64_t q = 0; q < Q; ++q)
-      if (ids[q] < -1 || ids[q] >= n_masks)
-        return set_error(RBOD_E_INVAL, "%s: query %lld: mask_of_query = %d is outside [-1, %d)", who, (long long)q,
-                         ids[q], n_masks);
-  }
+  std::vector<int> ids;
+  RBOD_TRY(read_mask_ids(who, "%s: query %lld: mask_of_query = %d is outside [-1, %d)", g, mask_of_query, Q, n_masks,
+                         static_cast<cudaStream_t>(stream), &ids));
   if (candidates > MMR_MAX_CANDIDATES)
     return set_error(RBOD_E_UNSUPPORTED, "%s: candidates = %d > %d", who, candidates, MMR_MAX_CANDIDATES);
   if (!g) return set_error(RBOD_E_INVAL, "%s: NULL handle", who);
@@ -1454,18 +1392,9 @@ int rbod_search_mmr(rbod_gallery* g, const float* queries, int64_t Q, int32_t li
   if (Q == 0) return RBOD_OK;
   RBOD_CUDA(cudaSetDevice(g->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const bool dist = g->metric == RBOD_EUCLID || g->metric == RBOD_MANHATTAN;
-  const size_t n_out = (size_t)Q * limit;
   if (g->rows == 0) {
-    std::vector<float> hs(n_out, dist ? INFINITY : -INFINITY);
-    std::vector<int64_t> hr(n_out, -1);
-    std::vector<double> hd(n_out, -INFINITY);
-    RBOD_CUDA(cudaMemcpyAsync(out_scores, hs.data(), n_out * 4, cudaMemcpyDefault, st));
-    RBOD_CUDA(cudaMemcpyAsync(out_rows, hr.data(), n_out * 8, cudaMemcpyDefault, st));
-    if (out_keys) RBOD_CUDA(cudaMemcpyAsync(out_keys, hd.data(), n_out * 8, cudaMemcpyDefault, st));
-    RBOD_CUDA(cudaStreamSynchronize(st));
     if (stats) stats->queries = Q;
-    return RBOD_OK;
+    return answer_none(out_scores, out_rows, out_keys, (size_t)Q * limit, g->metric, st);
   }
 
   // 1. the candidates: an ordinary search with k = candidates, written straight into the K8 workspaces
@@ -1484,9 +1413,8 @@ int rbod_search_mmr(rbod_gallery* g, const float* queries, int64_t Q, int32_t li
   RBOD_CUDA(cudaMemcpyAsync(g->mmr_ctl.p, ctl_d.data(), (size_t)Q * 8, cudaMemcpyHostToDevice, st));
   if (score_threshold)
     RBOD_CUDA(cudaMemcpyAsync(g->mmr_ctl.as<double>() + Q, ctl_t.data(), (size_t)Q * 4, cudaMemcpyHostToDevice, st));
-  RBOD_TRY(g->out_scores.ensure(n_out * 4));
-  RBOD_TRY(g->out_rows.ensure(n_out * 8));
-  RBOD_TRY(g->out_scores64.ensure(n_out * 8));
+  Answer a;
+  RBOD_TRY(stage_answer(g, out_scores, out_rows, out_keys, (size_t)Q * limit, &a));
   MmrArgs A;
   A.Q = Q;
   A.L = candidates;
@@ -1507,15 +1435,13 @@ int rbod_search_mmr(rbod_gallery* g, const float* queries, int64_t Q, int32_t li
     RBOD_TRY(g->mmr_q64.ensure((size_t)mmr_grid(Q, g->dim, g->num_sms) * g->dim * 8));
     A.q64_scratch = g->mmr_q64.as<double>();
   }
-  A.out_scores = is_device_ptr(out_scores) ? out_scores : g->out_scores.as<float>();
-  A.out_rows = is_device_ptr(out_rows) ? out_rows : g->out_rows.as<int64_t>();
-  A.out_keys = (out_keys && is_device_ptr(out_keys)) ? out_keys : g->out_scores64.as<double>();
+  A.out_scores = a.d_scores;
+  A.out_rows = a.d_rows;
+  A.out_keys = a.d_keys;
   RBOD_TRY(launch_mmr_select(g->metric, A, g->num_sms, st));
 
   // 3. copy-out
-  RBOD_TRY(copy_out(out_scores, A.out_scores, n_out * 4, st));
-  RBOD_TRY(copy_out(out_rows, A.out_rows, n_out * 8, st));
-  if (out_keys) RBOD_TRY(copy_out(out_keys, A.out_keys, n_out * 8, st));
+  RBOD_TRY(copy_out(a, st));
   RBOD_CUDA(cudaStreamSynchronize(st));
   if (stats) stats->total_launches += 1;
   return RBOD_OK;
@@ -1549,79 +1475,33 @@ static int check_example_args(const char* who, const char* what, const float* ex
 }
 
 // The rest of rbod_recommend / rbod_discover once the requests themselves are checked: the host mask ids, k, the
-// handle, then example_sweep with `collect` over the examples whose slot-table flags are `flags` [n_examples].
+// handle, then the sweep's front end with `collect` over the examples whose slot-table flags are `flags` [n_examples].
 static int example_search(const char* who, CollectLauncher collect, rbod_gallery* g, const float* examples,
                           int64_t n_examples, const int* flags, const int64_t* request_offsets, int64_t R, int32_t k,
                           const uint32_t* row_masks, int32_t n_masks, const int32_t* mask_of_request,
                           float* out_scores, int64_t* out_rows, double* out_keys, rbod_search_stats* stats,
                           void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const char* bad_id = "%s: mask_of_request[%lld] = %d is outside [-1, %d)";
+  // ids in host memory are checked before the handle is; ids in device memory are read once the device is set, and
+  // only when there are masks to read
   const bool ids_dev = is_device_ptr(mask_of_request);
-  if (mask_of_request && !ids_dev)
-    for (int64_t r = 0; r < R; ++r)
-      if (mask_of_request[r] < -1 || mask_of_request[r] >= n_masks)
-        return set_error(RBOD_E_INVAL, "%s: mask_of_request[%lld] = %d is outside [-1, %d)", who, (long long)r,
-                         mask_of_request[r], n_masks);
+  std::vector<int> ids;
+  if (!ids_dev) RBOD_TRY(read_mask_ids(who, bad_id, g, mask_of_request, R, n_masks, st, &ids));
   if (k > 1024) return set_error(RBOD_E_UNSUPPORTED, "%s: k=%d > 1024", who, k);
   if (!g) return set_error(RBOD_E_INVAL, "%s: NULL handle", who);
-  if (stats) memset(stats, 0, sizeof(*stats));
+  if (stats) {
+    memset(stats, 0, sizeof(*stats));
+    stats->queries = R;   // what an empty gallery reports too
+  }
   if (R == 0) return RBOD_OK;
   if (g->rows >= 0xffffffffll) return set_error(RBOD_E_UNSUPPORTED, "%s: more than 2^32-2 rows per shard", who);
   RBOD_CUDA(cudaSetDevice(g->device));
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-
-  // one mask id per request: -1 without masks, mask 0 for every request when mask_of_request is NULL
-  std::vector<int> ids(n_masks > 0 ? (size_t)R : 0, 0);
-  if (n_masks > 0 && mask_of_request) {
-    if (ids_dev) {
-      RBOD_CUDA(cudaMemcpyAsync(ids.data(), mask_of_request, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
-      RBOD_CUDA(cudaStreamSynchronize(st));
-      for (int64_t r = 0; r < R; ++r)
-        if (ids[r] < -1 || ids[r] >= n_masks)
-          return set_error(RBOD_E_INVAL, "%s: mask_of_request[%lld] = %d is outside [-1, %d)", who, (long long)r,
-                           ids[r], n_masks);
-    } else {
-      memcpy(ids.data(), mask_of_request, (size_t)R * 4);
-    }
-  }
-  SearchMasks M = {nullptr, (g->rows + 31) / 32, nullptr, nullptr};
-
-  const size_t n_out = (size_t)R * k;
-  RBOD_TRY(g->out_scores.ensure(n_out * 4));
-  RBOD_TRY(g->out_rows.ensure(n_out * 8));
-  RBOD_TRY(g->out_scores64.ensure(n_out * 8));
-  if (g->rows == 0) {
-    std::vector<float> hs(n_out, -INFINITY);
-    std::vector<int64_t> hr(n_out, -1);
-    std::vector<double> hd(n_out, -INFINITY);
-    RBOD_CUDA(cudaMemcpyAsync(out_scores, hs.data(), n_out * 4, cudaMemcpyDefault, st));
-    RBOD_CUDA(cudaMemcpyAsync(out_rows, hr.data(), n_out * 8, cudaMemcpyDefault, st));
-    if (out_keys) RBOD_CUDA(cudaMemcpyAsync(out_keys, hd.data(), n_out * 8, cudaMemcpyDefault, st));
-    RBOD_CUDA(cudaStreamSynchronize(st));
-    if (stats) stats->queries = R;
-    return RBOD_OK;
-  }
-  float* ds = is_device_ptr(out_scores) ? out_scores : g->out_scores.as<float>();
-  int64_t* dr = is_device_ptr(out_rows) ? out_rows : g->out_rows.as<int64_t>();
-  double* dk = (out_keys && is_device_ptr(out_keys)) ? out_keys : g->out_scores64.as<double>();
-  const void* md = nullptr;
-  if (n_masks > 0) RBOD_TRY(to_device(row_masks, (size_t)n_masks * M.words * 4, g->mask_dev, st, &md));
-  M.dev = static_cast<const uint32_t*>(md);
-  const void* xd = nullptr;
-  RBOD_TRY(to_device(examples, (size_t)n_examples * g->dim * 4, g->q32, st, &xd));
-  int64_t n_launch = 0, resweeps = 0;
-  RBOD_TRY(example_sweep(g, collect, who, static_cast<const float*>(xd), flags, request_offsets, R, k, M,
-                         ids.empty() ? nullptr : ids.data(), ds, dr, dk, &n_launch, &resweeps, st));
-  RBOD_TRY(copy_out(out_scores, ds, n_out * 4, st));
-  RBOD_TRY(copy_out(out_rows, dr, n_out * 8, st));
-  if (out_keys) RBOD_TRY(copy_out(out_keys, dk, n_out * 8, st));
-  RBOD_CUDA(cudaStreamSynchronize(st));
-  if (stats) {
-    stats->queries = R;
-    stats->sweep_queries = R;          // every request is answered by the fp64 sweep
-    stats->total_launches = n_launch;
-    stats->fallback_queries = resweeps;
-  }
-  return RBOD_OK;
+  if (ids_dev && n_masks > 0) RBOD_TRY(read_mask_ids(who, bad_id, g, mask_of_request, R, n_masks, st, &ids));
+  // K is larger-is-better: the selection takes it as a COSINE key, emitted as it is and padded with -inf
+  return sweep_search(g, who, "score of a request", collect, RBOD_COSINE, examples, n_examples, flags, request_offsets,
+                      R, k, row_masks, n_masks, ids.empty() ? nullptr : ids.data(), out_scores, out_rows, out_keys, stats,
+                      st);
 }
 
 int rbod_recommend(rbod_gallery* g, const float* examples, int64_t n_examples, const int8_t* example_sign,

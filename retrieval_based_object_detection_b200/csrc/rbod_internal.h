@@ -177,21 +177,15 @@ int launch_rescore_collected(const float* q, const double* q_qq, const float* ma
 int launch_select_collected(const double* coll_score, const uint32_t* coll_idx, const int* coll_cnt,
                             const int* flag_q, int f0, int nf, int cap, int k, int metric, float* out_scores,
                             int64_t* out_rows, double* out_scores64, cudaStream_t st);
-// K5: exact fp64 sweep (every metric)
+// K5 / K6 / K7: the exact fp64 sweep (rbod_slot_sweep.cuh), one collecting kernel per end of a row, with K5's widening
+// and selection.  Slot table of a pass: request of the pass | SLOT_LAST (the request's last slot) | the slot's flags:
+// SLOT_NEG (a negative example, K6; a pair's negative, K7), SLOT_TARGET (K7's target) and SLOT_DISC (K7, on every slot
+// of a request with a target: the request is scored as a discovery, not a context search).  A K5 query has no flags.
 int launch_dist_widen_queries(const float* q, const int* qsel, int nf, int dim, double* q64, double* qnorm,
                               cudaStream_t st);
-int launch_dist_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
-                        int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride,
-                        const uint32_t* row_mask, int64_t mask_words, const int* slot_mask, const double* thr,
-                        const uint32_t* thr_row, const int* active, const double* qnorm, int nf, int cap,
-                        double* coll_key, uint32_t* coll_idx, int* coll_cnt, int num_sms, cudaStream_t st);
 int launch_dist_select(const double* coll_key, const uint32_t* coll_idx, int* coll_cnt, const int* qsel, int nf,
                        int cap, int k, int sample, int metric, double* thr, uint32_t* thr_row, int* active,
                        int* n_active, float* out_scores, int64_t* out_rows, double* out_keys, cudaStream_t st);
-// K6 / K7: exact example sweeps (rbod_slot_sweep.cuh; selection through K5's widen / select launchers).  Slot table of
-// a pass: request of the pass | SLOT_LAST (the request's last slot) | the example's flags: SLOT_NEG (a negative
-// example, K6; a pair's negative, K7), SLOT_TARGET (K7's target) and SLOT_DISC (K7, on every slot of a request with a
-// target: the request is scored as a discovery, not a context search).
 constexpr int SLOT_REQ = 31, SLOT_LAST = 32, SLOT_NEG = 64, SLOT_TARGET = 128, SLOT_DISC = 256;
 using CollectLauncher = int (*)(int metric, const double* q64, const float* master32, const uint16_t* rows16,
                                 int kind16, int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0,
@@ -199,6 +193,12 @@ using CollectLauncher = int (*)(int metric, const double* q64, const float* mast
                                 const int* req_mask, const double* thr, const uint32_t* thr_row, const int* active,
                                 const double* qnorm, int n_slots, int n_req, int cap, double* coll_key,
                                 uint32_t* coll_idx, int* coll_cnt, int num_sms, cudaStream_t st);
+int launch_key_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
+                       int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride,
+                       const uint32_t* row_mask, int64_t mask_words, const int* slot_tab, const int* req_mask,
+                       const double* thr, const uint32_t* thr_row, const int* active, const double* qnorm,
+                       int n_slots, int n_req, int cap, double* coll_key, uint32_t* coll_idx, int* coll_cnt,
+                       int num_sms, cudaStream_t st);
 int launch_reco_collect(int metric, const double* q64, const float* master32, const uint16_t* rows16, int kind16,
                         int dim, int64_t ld32, int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride,
                         const uint32_t* row_mask, int64_t mask_words, const int* slot_tab, const int* req_mask,
@@ -293,7 +293,7 @@ struct rbod_gallery {
   } pending;
   rbod::DevBuf seg_idx, seg_off, seg_out, seg_partials, seg_prefix, seg_arrive, seg_scratch, seg_member;
   rbod::DevBuf gather_idx, gather_out;
-  rbod::DevBuf dist_q64, dist_thr, dist_ctl;   // K5: widened query batch, thresholds, {qsel, active, n_active, slot mask}
+  rbod::DevBuf dist_q64, dist_thr, dist_ctl;   // K5-K7 sweep: widened slots of a pass, thresholds, the pass's control
   rbod::DevBuf mmr_scores, mmr_rows, mmr_keys;  // K8: the candidate search's answer [Q][L] (search_impl writes it directly)
   rbod::DevBuf mmr_ctl, mmr_q64;                // K8: {diversity, threshold} per query; widened picks of wide rows
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;

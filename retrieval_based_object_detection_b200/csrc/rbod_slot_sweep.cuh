@@ -1,15 +1,17 @@
-// The exact fp64 example sweep shared by K6 (recommend) and K7 (discover): the row loop of K5's collecting kernel
-// (k5_distance_topk.cu) over a pass of up to 32 example vectors ("slots") of up to 32 whole requests, with the end of a
-// row left to a policy.  Every lane owns one gallery row and NS private fp64 accumulators (one per slot, no cross-lane
-// reduction); 64-column chunks of the rows and of the fp64 examples are double-buffered in shared memory with cp.async.
-// At the end of a row the lane scans the slots in (unrolled) order: the policy folds each slot's key into its running
-// values, and at a request's last slot forms the request's score, which is recorded as (score, row) in the request's
-// list when it beats the request's (threshold, row) bound and the request's mask allows the row.
+// The row loop of the exact fp64 sweep, shared by K5 (search), K6 (recommend) and K7 (discover), which differ only in
+// the end of a row, a policy: a pass of up to 32 vectors ("slots": queries or examples) of up to 32 whole requests.
+// Every lane owns one gallery row and NS private fp64 accumulators (one per slot, no cross-lane reduction); 64-column
+// chunks of the rows and of the fp64 slots are double-buffered in shared memory with cp.async.  At the end of a row
+// the lane scans the slots in (unrolled) order: the policy folds each slot's key into its running values, and at a
+// request's last slot forms the request's score, which is recorded as (score, row) in the request's list when it beats
+// the request's (threshold, row) bound and the request's mask allows the row.  A K5 query is a request of one slot.
 //
 // slot_tab[s] = request of the pass | SLOT_LAST (s is its request's last slot) | the policy's flags (rbod_internal.h);
-// req_mask[r] = the mask request r reads (-1 = none); thr / thr_row / active are per request, as K5's are per query.
+// req_mask[r] = the mask request r reads (-1 = none), or nullptr: every request reads mask 0 of row_mask (if any), and
+// the rows it excludes are not even loaded; thr / thr_row / active are per request.
 //
 // A policy End is default-constructed at the start of each row with its running values reset, and provides
+//   static constexpr bool kSlotIsRequest   true: slot f is request f of the pass (and its last slot), no table is read
 //   void fold(int tab, double key)    the key of the slot whose table entry is tab
 //   double score(int tab)             at the request's last slot (tab is that slot's entry)
 //   void reset()                      after the score is recorded, before the next request's first slot
@@ -68,7 +70,7 @@ __device__ __forceinline__ void slot_sweep(const double* __restrict__ q64, const
     const int t = threadIdx.x;
     thr_s[t] = (t < n_req && active[t]) ? thr[t] : INFINITY;   // +inf: beyond the pass, or the request is finished
     thr_row_s[t] = t < n_req ? thr_row[t] : 0xffffffffu;
-    rmask_s[t] = t < n_req ? req_mask[t] : -1;
+    rmask_s[t] = (t < n_req && req_mask != nullptr) ? req_mask[t] : -1;
     qn_s[t] = t < n_slots ? qnorm[t] : 0.0;
     slot_s[t] = t < n_slots ? slot_tab[t] : 0;                  // slots beyond the pass end no request
   }
@@ -82,18 +84,25 @@ __device__ __forceinline__ void slot_sweep(const double* __restrict__ q64, const
   const int64_t my_groups = n_groups > blockIdx.x ? (n_groups - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
   const int64_t n_steps = my_groups * n_chunks;
 
+  auto visit = [&](int64_t g, int l) -> int64_t { return (blockIdx.x + g * gridDim.x) * SLOT_ROWS + warp * 32 + l; };
+  // the gallery row lane l of this warp reads in group g, or -1: beyond the pass, or excluded by the one mask of the
+  // whole pass (req_mask == nullptr) -- such rows are not even loaded
   auto row_of = [&](int64_t g, int l) -> int64_t {
-    const int64_t v = (blockIdx.x + g * gridDim.x) * SLOT_ROWS + warp * 32 + l;
-    return v < n_visit ? row0 + v * stride : -1;
+    const int64_t v = visit(g, l);
+    if (v >= n_visit) return -1;
+    const int64_t r = row0 + v * stride;
+    if (row_mask != nullptr && req_mask == nullptr && !((row_mask[r >> 5] >> (r & 31)) & 1u)) return -1;
+    return r;
   };
   auto issue = [&](int64_t step, int b) {
     const int64_t g = step / n_chunks;
     const int c0 = (int)(step - g * n_chunks) * SLOT_CH;
     const int cw = min(SLOT_CH, dim - c0);
     uint32_t* xb = xs + ((size_t)b * 8 + warp) * 32 * pitch;
+    const unsigned live = __ballot_sync(0xffffffffu, row_of(g, lane) >= 0);   // one test per lane, not one per row
     for (int j = 0; j < 32; ++j) {
-      const int64_t r = row_of(g, j);
-      if (r < 0) continue;
+      if (!((live >> j) & 1u)) continue;
+      const int64_t r = row0 + visit(g, j) * stride;
       if (f32rows) {
         const uint32_t* src = reinterpret_cast<const uint32_t*>(master32 + r * ld32 + c0);
         for (int w = lane; w < cw; w += 32) cp_async_4(xb + j * pitch + w, src + w);
@@ -178,7 +187,8 @@ __device__ __forceinline__ void slot_sweep(const double* __restrict__ q64, const
           } else {
             key = -acc[f];
           }
-          const int tab = slot_s[f];
+          // a policy whose every slot is its own request (slot f = request f) reads no slot table: q = f at compile time
+          const int tab = End::kSlotIsRequest ? (f | SLOT_LAST) : slot_s[f];
           end.fold(tab, key);
           if (tab & SLOT_LAST) {
             const int q = tab & SLOT_REQ;
@@ -205,7 +215,7 @@ using SlotKernel = void (*)(const double*, const float*, const uint16_t*, int, i
                             const int*, const double*, int, int, int, double*, uint32_t*, int*);
 
 // Launches kernels[metric][NS == 32] (a kernel whose body is slot_sweep<metric, NS>) over the gallery rows row0,
-// row0 + stride, ...: 8 accumulators per lane for passes of up to 8 example slots (a request or two), 32 otherwise.
+// row0 + stride, ...: 8 accumulators per lane for passes of up to 8 slots, 32 otherwise.
 inline int launch_slot_kernel(const SlotKernel (&kernels)[4][2], const char* who, int metric, const double* q64,
                               const float* master32, const uint16_t* rows16, int kind16, int dim, int64_t ld32,
                               int64_t ld16, int64_t n_rows, int64_t row0, int64_t stride, const uint32_t* row_mask,
